@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- tracking hot path throughput on B200 (contract: see the task prompt / DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
+
+--steps K is the number of timed steps of value, with_status_err, e2e and e2e_rgb_frames.  --dump-outputs DIR writes what the
+last timed step of value returned (see dump_outputs) as .npy files; the inputs are generated from fixed seeds, so two builds
+run with the same arguments can be compared file for file.
 
 Workload = BASELINE.json configs[1]: 24 MP (6000x4000) synthetic frames, 20 000 Shi-Tomasi points, winSize 31,
 maxLevel 4, criteria (EPS|COUNT, 30, 0.01), forward-backward check < 1 px.
@@ -29,7 +33,6 @@ import argparse
 import gc
 import hashlib
 import json
-import math
 import os
 import sys
 import threading
@@ -39,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only: the benchmark writes nothing into it
 
 H, W, NPTS = 4000, 6000, 20000
 LK = dict(winSize=(31, 31), maxLevel=4, criteria=(3, 30, 0.01))
@@ -54,7 +58,8 @@ CONFIG = {
     "step": "cvtColor(new) + pyramid/Scharr(new) + LK fwd + LK bwd + FB check vs the previous frame (s1:311,323,326,329-333)",
     "sharding": "independent frame-pair streams per rank, no data-path collective",
 }
-MIN_TIMED_MS = 500.0           # the timed region is never shorter than this, whatever --steps says (inner repeats)
+SPIN_CYCLES = int(3e7)         # ~15 ms spin ahead of a timed region: the host enqueues its steps before the GPU starts on them
+DUMP_SAMPLE = 1 << 18          # --dump-outputs: pixels per pyramid plane (fixed seeded positions); all files 13 MB <= 64 MB
 SEQ_FRAMES = 8 * 46 + 1        # sharded_sequence: 369 frames = 184 groups of track_len 2 (23 per rank at N = 8)
 SEQ_T = 2
 
@@ -148,7 +153,6 @@ def cpu_step_fn(threads=None):
         desc = "cv2 %s (the OpenCV the reference calls), %d threads" % (cv2.__version__, cores)
     except Exception:                               # noqa: BLE001
         from oracle import oracle as m
-        m.build()
         kind, cores = "port", 1
         desc = "oracle/ibt_oracle.c scalar port, 1 thread"
 
@@ -245,6 +249,24 @@ def timed_steps(pipe, frames, pts, first, n, iter_total=None, probes=None):
     for k in range(n):
         i = first + k
         pipe.step(i, frames[pingpong(i + 1)], pts[pingpong(i)], iter_total, None if probes is None else probes[k])
+
+
+def dump_outputs(out_dir, p1, fb_dist, pyr):
+    """--dump-outputs: what the last timed step returned to its caller, as float32 .npy files in out_dir: p1 (NPTS, 2) tracked
+    positions and fb_dist (NPTS,) forward-backward distances of every point, and of the new frame's pyramid (what
+    SequenceTracker.prepare returns) DUMP_SAMPLE pixels per level at positions drawn from SEED: level<l> (gray) and
+    scharr<l> (dx, dy)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"p1": p1, "fb_dist": fb_dist}
+    rng = np.random.default_rng(SEED)
+    for l, (img, der) in enumerate(zip(pyr.levels, pyr.derivs)):
+        n = img.numel()
+        idx = torch.from_numpy(np.sort(rng.choice(n, min(n, DUMP_SAMPLE), replace=False))).to(img.device)
+        arrays["level%d" % l] = img.reshape(-1)[idx]
+        arrays["scharr%d" % l] = der.reshape(-1, 2)[idx]
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def run_from_files(trk, pipe, pts, host_frames, steps, cv, dev, ndec=None):
@@ -553,6 +575,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sequence", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true", help="issue every step on one stream (no overlap between steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -575,9 +598,8 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
 
-    from iceberg_tracking_code_b200 import build
-    build.build()
     from iceberg_tracking_code_b200 import _native
+    _native.lib()                                   # libibt.so as build() left it; raises when it was not built
     numa_node = _native.bind_to_gpu_numa_node(local_rank) if os.environ.get("IBT_NO_NUMA_BIND") is None else None
     from iceberg_tracking_code_b200 import cv
     from iceberg_tracking_code_b200.tracking import SequenceTracker
@@ -623,23 +645,18 @@ def main():
         pipe_.prime(frames[pingpong(first)])
         torch.cuda.synchronize()
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
+        torch.cuda._sleep(SPIN_CYCLES)
         e0.record(main_stream)
+        for s in pipe_.streams:
+            s.wait_event(e0)
         timed_steps(pipe_, frames, pts, first, n, iter_total)
         pipe_.join(main_stream)
         e1.record(main_stream)
         return e0, e1
 
-    # ---- warm-up + pilot (sizes the inner repeats so that the timed region lasts >= MIN_TIMED_MS) -------------------------
-    e0, e1 = run_region(pipe, warmup)
+    # ---- warm-up ----------------------------------------------------------------------------------------------------------
+    run_region(pipe, warmup)
     torch.cuda.synchronize()
-    e0, e1 = run_region(pipe, min(steps, 20))
-    torch.cuda.synchronize()
-    pilot_ms = e0.elapsed_time(e1) / min(steps, 20)
-    repeats = max(1, int(math.ceil(MIN_TIMED_MS / max(1e-3, pilot_ms * steps))))
-    if dist is not None:
-        rp = torch.tensor([repeats], dtype=torch.int64, device=dev)
-        dist.all_reduce(rp, op=dist.ReduceOp.MAX)
-        repeats = int(rp.item())
 
     # ---- timed region: device-resident inputs ---------------------------------------------------------------------
     sampler = ClockSampler(local_rank)
@@ -649,7 +666,7 @@ def main():
     trk.iter_total.zero_()
     gc.collect(); gc.disable()
     sampler.start()
-    e0, e1 = run_region(pipe, steps * repeats, 0, trk.iter_total)
+    e0, e1 = run_region(pipe, steps, 0, trk.iter_total)
     sampler.sample_now()                       # the GPU is still working through the queued steps
     torch.cuda.synchronize()
     gc.enable()
@@ -657,15 +674,17 @@ def main():
         dist.barrier()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1)
-    nsteps = steps * repeats
     iters = int(trk.iter_total.item())
-    alive_frac = float((pipe.fbd[(nsteps - 1) & 1] < 1).float().mean().item())
+    last = steps - 1                            # PairPipeline.step(last) wrote p1 / fbd[last & 1] and pyramid slot last % 3
+    alive_frac = float((pipe.fbd[last & 1] < 1).float().mean().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pipe.p1[last & 1], pipe.fbd[last & 1], pipe.pyr[last % 3])
 
     # ---- the same loop returning what cv2 returns: status + err of both passes (OpenCV's level-0 residual stage) ----------
     pipe_se = PairPipeline(trk, dev, frames[0], want_status_err=True)
     if args.no_pipeline:
         pipe_se.streams[1] = pipe_se.streams[0]
-    n_se = max(20, min(nsteps, 200))
+    n_se = steps
     run_region(pipe_se, 6); torch.cuda.synchronize()
     e0, e1 = run_region(pipe_se, n_se)
     torch.cuda.synchronize()
@@ -719,7 +738,7 @@ def main():
         d2h_done[(first + n - 1) & 1].synchronize()
         acc += float(h_fbd[(first + n - 1) & 1][0])
         return acc
-    n_e2e = max(steps, int(math.ceil(MIN_TIMED_MS / 1.3)))
+    n_e2e = steps
     e2e_loop(max(3, warmup // 2) * 2, 0)
     torch.cuda.synchronize()
     if dist is not None:
@@ -740,7 +759,7 @@ def main():
     try:
         if dist is not None:
             dist.barrier()
-        from_files = run_from_files(trk, pipe, pts, host_frames, min(max(steps, 60), 200), cv, dev)
+        from_files = run_from_files(trk, pipe, pts, host_frames, steps, cv, dev)
     except ImportError as e:                        # Pillow missing on the box: the section is skipped, not faked
         from_files = {"skipped": repr(e)}
     if dist is not None and "ms_per_step" in from_files:
@@ -794,25 +813,25 @@ def main():
     prep_bytes = 4 * n0 + sum(npx) + sum(npx[1:]) + 4 * sum(npx)
     k1_bytes = n0 + 4 * n0 + npx[1]                # level 0 alone: read level 0 once, write (dx,dy) int16, write level 1
     achieved = prep_bytes / (prep_ms * 1e-3) / 1e9
-    value = world * NPTS * nsteps / (ms * 1e-3)
+    value = world * NPTS * steps / (ms * 1e-3)
     out = {
         "metric": METRIC, "value": value, "unit": "points/s",
-        "n_gpus": world, "steps": steps, "warmup": warmup, "ms_per_step": ms / nsteps, "higher_is_better": True,
+        "n_gpus": world, "steps": steps, "warmup": warmup, "ms_per_step": ms / steps, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "u8/int32 fixed point + f32 2x2 solve", "data": "synthetic",
         "config": CONFIG,
-        "inner_repeats": repeats, "timed_steps": nsteps, "timed_region_ms": ms,
+        "timed_steps": steps, "timed_region_ms": ms,
         "numa_node_rank0": numa_node,
         "pipelining": "none (one stream)" if args.no_pipeline else "consecutive (independent) frame pairs overlap on two CUDA streams, three pyramid slots",
-        "frame_pairs_per_s": world * nsteps / (ms * 1e-3),
+        "frame_pairs_per_s": world * steps / (ms * 1e-3),
         "feature_pair_iterations_per_s": iters / (ms * 1e-3),
-        "iterations_per_point_pair": iters / (world * NPTS * nsteps),
+        "iterations_per_point_pair": iters / (world * NPTS * steps),
         "fb_valid_fraction_last_step": alive_frac,
         "with_status_err": {"ms_per_step": ms_se, "value": world * NPTS / (ms_se * 1e-3), "unit": "points/s", "steps": n_se,
                             "note": "same step with st/err buffers of both passes passed (what cv2 returns, s1:323,326): "
                                     "adds OpenCV's level-0 bounds test and residual"},
         "gftt_ms": float(np.median(gftt_ms)),
         "gftt_async_ms": float(np.median(gftt_async_ms[1:])),
-        "gpu_launches": own_launches_per_step * nsteps,
+        "gpu_launches": own_launches_per_step * steps,
         "clocks": clocks,
         "e2e_rgb_frames": {"value": world * NPTS * n_e2e / (e2e_ms * 1e-3), "unit": "points/s", "h2d_bytes_per_step": h2d,
                            "d2h_bytes_per_step": d2h, "ms_per_step": e2e_ms / n_e2e, "steps": n_e2e,
