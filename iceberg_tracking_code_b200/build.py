@@ -12,7 +12,7 @@ import sys
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(_HERE, "libibt.so")
-SOURCES = ["core.cu", "gray.cu", "pyramid.cu", "gftt.cu", "lk.cu", "tracks.cu", "utm.cu", "mask.cu", "jpeg.cu", "grid.cu"]
+SOURCES = ["core.cu", "gray.cu", "pyramid.cu", "gftt.cu", "lk.cu", "tracks.cu", "utm.cu", "mask.cu", "jpeg.cu", "grid.cu", "scan.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(_HERE, "..", "include", "ibt.h")]
 
 NVCC_FLAGS = [

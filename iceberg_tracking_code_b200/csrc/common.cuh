@@ -131,10 +131,38 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
-// gftt.cu: stable LSD radix sort of 64-bit keys on a byte range (also used by grid.cu)
-size_t radix_sort_scratch_words(uint32_t n);
-unsigned long long *radix_sort_u64_bytes(unsigned long long *keys0, unsigned long long *keys1, uint32_t n, int first_byte,
-                                         int last_byte, uint32_t *scratch, cudaStream_t st);
+// ---- CTA-wide exclusive scan of one value per thread (blockDim.x <= 1024, multiple of 32) -------------------------------
+__device__ __forceinline__ uint32_t cta_exclusive_scan(uint32_t v, uint32_t *total)
+{
+    __shared__ uint32_t warp_sums[32];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    uint32_t inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += t;
+    }
+    __syncthreads();                                       // warp_sums may still be read by a previous call
+    if (lane == 31) warp_sums[w] = inc;
+    __syncthreads();
+    uint32_t ws = lane < nw ? warp_sums[lane] : 0u;
+    uint32_t wi = ws;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t t = __shfl_up_sync(0xffffffffu, wi, o);
+        if (lane >= o) wi += t;
+    }
+    const uint32_t wbase = __shfl_sync(0xffffffffu, wi - ws, w);
+    if (total) *total = __shfl_sync(0xffffffffu, wi, nw - 1);
+    return wbase + inc - v;
+}
+
+// scan.cu: device-wide exclusive scan of `rows` rows of n uint32 each, `stride` elements apart (1 <= rows <= 65535).
+// in == out is allowed.  total (device, optional) receives the total of each row.  partial: scan_partial_words(n, rows)
+// words.  Launch errors are left for the caller's check_launch.
+size_t scan_partial_words(int n, int rows);
+void launch_scan(const uint32_t *in, uint32_t *out, uint32_t *partial, int n, int rows, int64_t stride, uint32_t *total,
+                 cudaStream_t st);
 
 constexpr int kNumSMs = 148;             // B200: 2 dies x 74 SMs
 

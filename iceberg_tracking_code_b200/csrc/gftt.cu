@@ -524,167 +524,11 @@ static int launch_eig_nms(const uint8_t *gray, int H, int W, int64_t pitch, int 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Radix sort (ascending, 64-bit keys, stable LSD, 8-bit digits).
-constexpr int RS_WARPS = 8, RS_STEPS = 16, RS_TILE = RS_WARPS * RS_STEPS * 32;   // 4096 keys per block
-
-__global__ void __launch_bounds__(256)
-rs_count_kernel(const unsigned long long *__restrict__ keys, uint32_t n, int shift, uint32_t nblocks,
-                uint32_t *__restrict__ blockhist /*[256][nblocks]*/)
-{
-    __shared__ uint32_t sh[256];
-    sh[threadIdx.x] = 0;
-    __syncthreads();
-    const uint32_t base = blockIdx.x * RS_TILE;
-    for (uint32_t i = threadIdx.x; i < RS_TILE; i += 256) {
-        const uint32_t g = base + i;
-        if (g < n) atomicAdd(&sh[(uint32_t)((keys[g] >> shift) & 0xff)], 1u);
-    }
-    __syncthreads();
-    blockhist[threadIdx.x * nblocks + blockIdx.x] = sh[threadIdx.x];
-}
-
-// exclusive scan of uint32 in place.  Block b scans its SCAN_TILE elements; with `block_sums` the block total goes there
-// (phase 1 of the hierarchical scan), with `block_offs` the scanned totals are added back (phase 3).
-constexpr int SCAN_EPT = 8, SCAN_TILE = 1024 * SCAN_EPT;
-
-__global__ void __launch_bounds__(1024)
-scan_tile_kernel(uint32_t *__restrict__ data, uint32_t len, uint32_t *__restrict__ block_sums, uint32_t *__restrict__ total_out)
-{
-    __shared__ uint32_t warp_tot[32];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const uint32_t i0 = blockIdx.x * SCAN_TILE + threadIdx.x * SCAN_EPT;
-    uint32_t v[SCAN_EPT], sum = 0;
-#pragma unroll
-    for (int e = 0; e < SCAN_EPT; e++) { v[e] = (i0 + e < len) ? data[i0 + e] : 0; sum += v[e]; }
-    uint32_t inc = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t tmp = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += tmp;
-    }
-    if (lane == 31) warp_tot[wid] = inc;
-    __syncthreads();
-    if (wid == 0) {
-        uint32_t w = warp_tot[lane];
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t tmp = __shfl_up_sync(0xffffffffu, w, o);
-            if (lane >= o) w += tmp;
-        }
-        warp_tot[lane] = w;              // inclusive over warps
-    }
-    __syncthreads();
-    uint32_t run = (wid ? warp_tot[wid - 1] : 0) + inc - sum;
-#pragma unroll
-    for (int e = 0; e < SCAN_EPT; e++) { if (i0 + e < len) data[i0 + e] = run; run += v[e]; }
-    if (threadIdx.x == 1023) {
-        if (block_sums) block_sums[blockIdx.x] = run;
-        if (total_out) *total_out = run;
-    }
-}
-
-__global__ void __launch_bounds__(1024)
-scan_add_kernel(uint32_t *__restrict__ data, uint32_t len, const uint32_t *__restrict__ block_offs, uint32_t nblocks,
-                uint32_t *__restrict__ total_out)
-{
-    const uint32_t off = block_offs[blockIdx.x];
-    const uint32_t i0 = blockIdx.x * SCAN_TILE + threadIdx.x * SCAN_EPT;
-#pragma unroll
-    for (int e = 0; e < SCAN_EPT; e++) if (i0 + e < len) data[i0 + e] += off;
-    // grand total = offset of the last block + its own sum, which phase 1 left in block_offs[nblocks] (see scan_u32)
-    if (total_out && blockIdx.x == 0 && threadIdx.x == 0) *total_out = block_offs[nblocks];
-}
-
-// exclusive scan of data[0..len) in place; *total_out (device, optional) receives the grand total.
-// scratch: (len / SCAN_TILE + 2) uint32.  len up to SCAN_TILE^2 (67 M).
-static void scan_u32(uint32_t *data, uint32_t len, uint32_t *total_out, uint32_t *scratch, cudaStream_t st)
-{
-    const uint32_t nb = (len + SCAN_TILE - 1) / SCAN_TILE;
-    if (nb <= 1) {
-        scan_tile_kernel<<<1, 1024, 0, st>>>(data, len, nullptr, total_out);
-        return;
-    }
-    scan_tile_kernel<<<nb, 1024, 0, st>>>(data, len, scratch, nullptr);
-    // scan the nb block sums; the total lands in scratch[nb]
-    scan_tile_kernel<<<1, 1024, 0, st>>>(scratch, nb, nullptr, scratch + nb);
-    scan_add_kernel<<<nb, 1024, 0, st>>>(data, len, scratch, nb, total_out);
-}
-
-__global__ void __launch_bounds__(256)
-rs_scatter_kernel(const unsigned long long *__restrict__ src, unsigned long long *__restrict__ dst, uint32_t n,
-                  int shift, uint32_t nblocks, const uint32_t *__restrict__ blockoff /*[256][nblocks] scanned*/)
-{
-    __shared__ uint32_t wcount[RS_WARPS][256];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (int i = threadIdx.x; i < RS_WARPS * 256; i += 256) (&wcount[0][0])[i] = 0;
-    __syncthreads();
-    const uint32_t wbase = blockIdx.x * RS_TILE + wid * (RS_STEPS * 32);
-    unsigned long long k[RS_STEPS];
-    uint32_t rank[RS_STEPS];
-#pragma unroll
-    for (int s = 0; s < RS_STEPS; s++) {
-        const uint32_t g = wbase + s * 32 + lane;
-        const bool valid = g < n;
-        k[s] = valid ? src[g] : 0ull;
-        const uint32_t d = (uint32_t)((k[s] >> shift) & 0xff);
-        const uint32_t vmask = __ballot_sync(0xffffffffu, valid);
-        uint32_t peers = __match_any_sync(0xffffffffu, valid ? d : 0x100u + lane) & vmask;
-        if (!valid) peers = 0;
-        const uint32_t before = __popc(peers & ((1u << lane) - 1));
-        uint32_t prev = 0;
-        if (valid) prev = wcount[wid][d];          // all peers read the same value before the leader updates
-        __syncwarp();
-        if (valid && before == 0) wcount[wid][d] = prev + __popc(peers);
-        __syncwarp();
-        rank[s] = prev + before;                  // rank within this warp's chunk for digit d
-    }
-    __syncthreads();
-    // exclusive prefix over warps per digit, plus the global offset of (digit, block)
-    {
-        const int d = threadIdx.x;
-        uint32_t run = blockoff[d * nblocks + blockIdx.x];
-#pragma unroll
-        for (int w = 0; w < RS_WARPS; w++) { const uint32_t c = wcount[w][d]; wcount[w][d] = run; run += c; }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int s = 0; s < RS_STEPS; s++) {
-        const uint32_t g = wbase + s * 32 + lane;
-        if (g < n) {
-            const uint32_t d = (uint32_t)((k[s] >> shift) & 0xff);
-            dst[wcount[wid][d] + rank[s]] = k[s];
-        }
-    }
-}
-
-// Stable LSD radix sort of n 64-bit keys on bytes [first_byte, last_byte] (shared with grid.cu).  keys0 holds the input,
-// keys1 is the ping-pong buffer; returns the buffer that holds the result.  scratch: radix_sort_scratch_words(n) uint32.
-size_t radix_sort_scratch_words(uint32_t n)
-{
-    const size_t nblocks = ((size_t)n + RS_TILE - 1) / RS_TILE;
-    return 256 * nblocks + (256 * nblocks) / SCAN_TILE + 4;
-}
-unsigned long long *radix_sort_u64_bytes(unsigned long long *keys0, unsigned long long *keys1, uint32_t n, int first_byte,
-                                         int last_byte, uint32_t *scratch, cudaStream_t st)
-{
-    if (n <= 1) return keys0;
-    const uint32_t nblocks = (n + RS_TILE - 1) / RS_TILE;
-    uint32_t *blockhist = scratch, *scan_scratch = scratch + 256 * (size_t)nblocks;
-    unsigned long long *src = keys0, *dst = keys1;
-    for (int p = first_byte; p <= last_byte; p++) {
-        rs_count_kernel<<<nblocks, 256, 0, st>>>(src, n, 8 * p, nblocks, blockhist);
-        scan_u32(blockhist, 256u * nblocks, nullptr, scan_scratch, st);
-        rs_scatter_kernel<<<nblocks, 256, 0, st>>>(src, dst, n, 8 * p, nblocks, blockhist);
-        unsigned long long *t = src; src = dst; dst = t;
-    }
-    return src;
-}
-
-// ---------------------------------------------------------------------------------------------
 // K2b: the whole selection in ONE persistent launch.  sorted[r] = ~key of rank r (rank 0 = strongest).
 constexpr int SEL_THREADS = 256;
 constexpr int SEL_CTAS_PER_SM = 2;                   // 2 x 256 threads x 128 registers fill an SM: the grid is kNumSMs * 2, all resident
-constexpr int SEL_STEPS = 4, SEL_TILE = RS_WARPS * SEL_STEPS * 32, SEL_TILE_SHIFT = 10;   // 1024 keys per sort tile: ~80 tiles for 81 k keys
+constexpr int SEL_WARPS = SEL_THREADS / 32;
+constexpr int SEL_STEPS = 4, SEL_TILE = SEL_WARPS * SEL_STEPS * 32, SEL_TILE_SHIFT = 10;   // 1024 keys per sort tile: ~80 tiles for 81 k keys
 constexpr uint32_t CELL_END = 0xffffffffu;
 
 struct SelArgs {
@@ -810,7 +654,7 @@ __global__ void __launch_bounds__(SEL_THREADS, SEL_CTAS_PER_SM)
 gftt_select_kernel(const __grid_constant__ SelArgs a)
 {
     __shared__ uint32_t sh[4096];
-    __shared__ uint32_t wcount[RS_WARPS][256];
+    __shared__ uint32_t wcount[SEL_WARPS][256];
     __shared__ uint32_t wtot[9];
     __shared__ uint32_t s_misc[8];
     GfttCounters *cnt = a.cnt;
@@ -956,7 +800,7 @@ gftt_select_kernel(const __grid_constant__ SelArgs a)
                     block_scan_excl(sh, 256, wtot);
                     const uint32_t digit_base = sh[tid];
                     __syncthreads();
-                    for (int i = tid; i < RS_WARPS * 256; i += SEL_THREADS) (&wcount[0][0])[i] = 0;
+                    for (int i = tid; i < SEL_WARPS * 256; i += SEL_THREADS) (&wcount[0][0])[i] = 0;
                     __syncthreads();
                     const uint32_t wbase = tile * SEL_TILE + wid * (SEL_STEPS * 32);
                     unsigned long long k[SEL_STEPS];
@@ -986,7 +830,7 @@ gftt_select_kernel(const __grid_constant__ SelArgs a)
                     {
                         uint32_t run = digit_base + before;        // thread d: exclusive prefix over warps + global offset of (digit, tile)
 #pragma unroll
-                        for (int w = 0; w < RS_WARPS; w++) { const uint32_t c = wcount[w][tid]; wcount[w][tid] = run; run += c; }
+                        for (int w = 0; w < SEL_WARPS; w++) { const uint32_t c = wcount[w][tid]; wcount[w][tid] = run; run += c; }
                     }
                     __syncthreads();
 #pragma unroll

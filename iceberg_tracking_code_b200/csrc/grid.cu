@@ -151,6 +151,95 @@ grid_reduce_kernel(const double *__restrict__ u, const double *__restrict__ v, c
     sum_v[c] = 0.0 + np_pairwise_sum(v, keys, lo, n);
 }
 
+// radix sort (ascending, 64-bit keys, stable LSD, 8-bit digits)
+constexpr int RS_WARPS = 8, RS_STEPS = 16, RS_TILE = RS_WARPS * RS_STEPS * 32;   // 4096 keys per block
+
+__global__ void __launch_bounds__(256)
+rs_count_kernel(const unsigned long long *__restrict__ keys, uint32_t n, int shift, uint32_t nblocks,
+                uint32_t *__restrict__ blockhist /*[256][nblocks]*/)
+{
+    __shared__ uint32_t sh[256];
+    sh[threadIdx.x] = 0;
+    __syncthreads();
+    const uint32_t base = blockIdx.x * RS_TILE;
+    for (uint32_t i = threadIdx.x; i < RS_TILE; i += 256) {
+        const uint32_t g = base + i;
+        if (g < n) atomicAdd(&sh[(uint32_t)((keys[g] >> shift) & 0xff)], 1u);
+    }
+    __syncthreads();
+    blockhist[threadIdx.x * nblocks + blockIdx.x] = sh[threadIdx.x];
+}
+
+__global__ void __launch_bounds__(256)
+rs_scatter_kernel(const unsigned long long *__restrict__ src, unsigned long long *__restrict__ dst, uint32_t n,
+                  int shift, uint32_t nblocks, const uint32_t *__restrict__ blockoff /*[256][nblocks] scanned*/)
+{
+    __shared__ uint32_t wcount[RS_WARPS][256];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    for (int i = threadIdx.x; i < RS_WARPS * 256; i += 256) (&wcount[0][0])[i] = 0;
+    __syncthreads();
+    const uint32_t wbase = blockIdx.x * RS_TILE + wid * (RS_STEPS * 32);
+    unsigned long long k[RS_STEPS];
+    uint32_t rank[RS_STEPS];
+#pragma unroll
+    for (int s = 0; s < RS_STEPS; s++) {
+        const uint32_t g = wbase + s * 32 + lane;
+        const bool valid = g < n;
+        k[s] = valid ? src[g] : 0ull;
+        const uint32_t d = (uint32_t)((k[s] >> shift) & 0xff);
+        const uint32_t vmask = __ballot_sync(0xffffffffu, valid);
+        uint32_t peers = __match_any_sync(0xffffffffu, valid ? d : 0x100u + lane) & vmask;
+        if (!valid) peers = 0;
+        const uint32_t before = __popc(peers & ((1u << lane) - 1));
+        uint32_t prev = 0;
+        if (valid) prev = wcount[wid][d];          // all peers read the same value before the leader updates
+        __syncwarp();
+        if (valid && before == 0) wcount[wid][d] = prev + __popc(peers);
+        __syncwarp();
+        rank[s] = prev + before;                  // rank within this warp's chunk for digit d
+    }
+    __syncthreads();
+    // exclusive prefix over warps per digit, plus the global offset of (digit, block)
+    {
+        const int d = threadIdx.x;
+        uint32_t run = blockoff[d * nblocks + blockIdx.x];
+#pragma unroll
+        for (int w = 0; w < RS_WARPS; w++) { const uint32_t c = wcount[w][d]; wcount[w][d] = run; run += c; }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int s = 0; s < RS_STEPS; s++) {
+        const uint32_t g = wbase + s * 32 + lane;
+        if (g < n) {
+            const uint32_t d = (uint32_t)((k[s] >> shift) & 0xff);
+            dst[wcount[wid][d] + rank[s]] = k[s];
+        }
+    }
+}
+
+// Stable LSD radix sort of n 64-bit keys on bytes [first_byte, last_byte].  keys0 holds the input, keys1 is the ping-pong
+// buffer; returns the buffer that holds the result.  scratch: radix_sort_scratch_words(n) uint32, n <= 2^30.
+static size_t radix_sort_scratch_words(uint32_t n)
+{
+    const size_t nblocks = ((size_t)n + RS_TILE - 1) / RS_TILE;
+    return 256 * nblocks + scan_partial_words((int)(256 * nblocks), 1);
+}
+static unsigned long long *radix_sort_u64_bytes(unsigned long long *keys0, unsigned long long *keys1, uint32_t n, int first_byte,
+                                                int last_byte, uint32_t *scratch, cudaStream_t st)
+{
+    if (n <= 1) return keys0;
+    const uint32_t nblocks = (n + RS_TILE - 1) / RS_TILE;
+    uint32_t *blockhist = scratch, *partial = scratch + 256 * (size_t)nblocks;
+    unsigned long long *src = keys0, *dst = keys1;
+    for (int p = first_byte; p <= last_byte; p++) {
+        rs_count_kernel<<<nblocks, 256, 0, st>>>(src, n, 8 * p, nblocks, blockhist);
+        launch_scan(blockhist, blockhist, partial, (int)(256 * nblocks), 1, 0, nullptr, st);
+        rs_scatter_kernel<<<nblocks, 256, 0, st>>>(src, dst, n, 8 * p, nblocks, blockhist);
+        unsigned long long *t = src; src = dst; dst = t;
+    }
+    return src;
+}
+
 struct GridLayout { size_t off_keys0, off_keys1, off_scratch, off_start, off_end, total; };
 static void grid_layout(int64_t n, int ncell, GridLayout &L)
 {

@@ -23,6 +23,7 @@
 #include "common.cuh"
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include <atomic>
 
 namespace ibt {
@@ -61,85 +62,6 @@ struct JpgGeom {
 __constant__ uint8_t c_zigzag[64] = {0,  1,  8,  16, 9,  2,  3,  10, 17, 24, 32, 25, 18, 11, 4,  5,  12, 19, 26, 33, 40, 48,
                                      41, 34, 27, 20, 13, 6,  7,  14, 21, 28, 35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23,
                                      30, 37, 44, 51, 58, 59, 52, 45, 38, 31, 39, 46, 53, 60, 61, 54, 47, 55, 62, 63};
-
-// ---- CTA-wide exclusive scan of one value per thread (blockDim.x <= 1024, multiple of 32) -------------------------------
-__device__ __forceinline__ uint32_t cta_exclusive_scan(uint32_t v, uint32_t *total)
-{
-    __shared__ uint32_t warp_sums[32];
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    uint32_t inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += t;
-    }
-    __syncthreads();                                       // warp_sums may still be read by a previous call
-    if (lane == 31) warp_sums[w] = inc;
-    __syncthreads();
-    uint32_t ws = lane < nw ? warp_sums[lane] : 0u;
-    uint32_t wi = ws;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t t = __shfl_up_sync(0xffffffffu, wi, o);
-        if (lane >= o) wi += t;
-    }
-    const uint32_t wbase = __shfl_sync(0xffffffffu, wi - ws, w);
-    if (total) *total = __shfl_sync(0xffffffffu, wi, nw - 1);
-    return wbase + inc - v;
-}
-
-// ---- generic exclusive scan of `n` u32 values per row (gridDim.y rows, `stride` elements apart), tiles of 1024 --------------
-__global__ void __launch_bounds__(256) jpg_scan_reduce(const uint32_t *__restrict__ in, uint32_t *__restrict__ partial, int n,
-                                                       int64_t stride, int ptiles)
-{
-    const uint32_t *row = in + blockIdx.y * stride;
-    const int base = blockIdx.x * 1024 + threadIdx.x * 4;
-    uint32_t s = 0;
-#pragma unroll
-    for (int j = 0; j < 4; j++)
-        if (base + j < n) s += row[base + j];
-    uint32_t tot;
-    cta_exclusive_scan(s, &tot);
-    if (threadIdx.x == 0) partial[blockIdx.y * ptiles + blockIdx.x] = tot;
-}
-__global__ void __launch_bounds__(1024) jpg_scan_partials(uint32_t *__restrict__ partial, int ntiles, int ptiles)
-{
-    uint32_t *row = partial + blockIdx.x * ptiles;
-    uint32_t carry = 0;
-    for (int b = 0; b < ntiles; b += 1024) {
-        const int i = b + threadIdx.x;
-        const uint32_t v = i < ntiles ? row[i] : 0u;
-        uint32_t tot;
-        const uint32_t ex = cta_exclusive_scan(v, &tot);
-        if (i < ntiles) row[i] = carry + ex;
-        carry += tot;
-    }
-}
-__global__ void __launch_bounds__(256) jpg_scan_apply(const uint32_t *__restrict__ in, const uint32_t *__restrict__ partial,
-                                                      uint32_t *__restrict__ out, int n, int64_t stride, int ptiles)
-{
-    const uint32_t *row = in + blockIdx.y * stride;
-    uint32_t *orow = out + blockIdx.y * stride;
-    const int base = blockIdx.x * 1024 + threadIdx.x * 4;
-    uint32_t v[4], s = 0;
-#pragma unroll
-    for (int j = 0; j < 4; j++) { v[j] = base + j < n ? row[base + j] : 0u; s += v[j]; }
-    uint32_t ex = cta_exclusive_scan(s, nullptr) + partial[blockIdx.y * ptiles + blockIdx.x];
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-        if (base + j < n) orow[base + j] = ex;
-        ex += v[j];
-    }
-}
-static int launch_scan(const uint32_t *in, uint32_t *out, uint32_t *partial, int n, int rows, int64_t stride, cudaStream_t st)
-{
-    if (n <= 0) return IBT_OK;
-    const int ntiles = (n + 1023) / 1024;
-    jpg_scan_reduce<<<dim3(ntiles, rows), 256, 0, st>>>(in, partial, n, stride, ntiles);
-    jpg_scan_partials<<<rows, 1024, 0, st>>>(partial, ntiles, ntiles);
-    jpg_scan_apply<<<dim3(ntiles, rows), 256, 0, st>>>(in, partial, out, n, stride, ntiles);
-    return check_launch("jpeg scan");
-}
 
 // ---- destuff ------------------------------------------------------------------------------------------------
 // byte j of the segment is dropped iff it is the 0x00 that follows a 0xFF, or belongs to an RSTn marker (FF D0..D7);
@@ -898,8 +820,8 @@ static void jpeg_layout(const ibt_jpeg_info_t *I, JpgLayout &L)
     L.off_nblk = take((size_t)L.nsub * JPG_Q * 4);
     L.off_base = take((size_t)L.nsub * JPG_Q * 4);
     L.off_qstart = take((size_t)L.nsub * JPG_Q * 8);
-    const size_t np1 = (size_t)(L.nsub * JPG_Q + 1023) / 1024 + 1, np2 = 3 * ((size_t)(L.nmcu + 1023) / 1024 + 1), np3 = (size_t)(L.nchunks + 1023) / 1024 + 1;
-    L.off_partial = take((np1 > np2 ? (np1 > np3 ? np1 : np3) : (np2 > np3 ? np2 : np3)) * 4);
+    L.off_partial = take(std::max({scan_partial_words(L.nchunks, 1), scan_partial_words(L.nsub * JPG_Q, 1),
+                                   scan_partial_words(L.nmcu, 3)}) * 4);
     L.coef_bytes = (size_t)L.nblocks * 64 * 2;
     L.off_coef = take(L.coef_bytes);
     L.off_dcs = take((size_t)3 * L.nmcu * 4);
@@ -1129,8 +1051,7 @@ static int jpeg_decode_impl(const uint8_t *d_file, const ibt_jpeg_info_t *I, voi
     IBT_CUDA_TRY(cudaMemsetAsync(sbytes, 0, L.stream_bytes, st));
     IBT_CUDA_TRY(cudaMemsetAsync(coef, 0, L.coef_bytes, st));
     jpg_destuff_count<<<L.nchunks, 256, 0, st>>>(scan, I->scan_bytes, counts);
-    rc = launch_scan(counts, offsets, partial, L.nchunks, 1, 0, st);
-    if (rc) return rc;
+    launch_scan(counts, offsets, partial, L.nchunks, 1, 0, nullptr, st);
     uint32_t *rst = L.rst_bytes ? reinterpret_cast<uint32_t *>(ws + L.off_rst) : nullptr;
     if (rst) IBT_CUDA_TRY(cudaMemsetAsync(rst, 0, L.rst_bytes, st));
     jpg_destuff_write<<<L.nchunks, 256, 0, st>>>(scan, I->scan_bytes, offsets, sbytes, meta, rst);
@@ -1176,14 +1097,12 @@ static int jpeg_decode_impl(const uint8_t *d_file, const ibt_jpeg_info_t *I, voi
     }
 
     // 3. output block of every subsequence, coefficient pass
-    rc = launch_scan(nblk, base, partial, L.nsub * JPG_Q, 1, 0, st);
-    if (rc) return rc;
+    launch_scan(nblk, base, partial, L.nsub * JPG_Q, 1, 0, nullptr, st);
     jpg_huff_write<<<(L.nsub * JPG_Q + 127) / 128, 128, 0, st>>>(words, meta, dT, qstart, base, coef, L.nsub, (uint32_t)L.nblocks, rst, L.sbits);
 
     // 4. DC prediction: prefix sums over MCUs per component
     jpg_dc_sums<<<(L.nmcu + 255) / 256, 256, 0, st>>>(coef, L.G, dcs, L.nmcu);
-    rc = launch_scan(dcs, dcpre, partial, L.nmcu, I->ncomp, L.nmcu, st);
-    if (rc) return rc;
+    launch_scan(dcs, dcpre, partial, L.nmcu, I->ncomp, L.nmcu, nullptr, st);
 
     // 5. inverse DCT into the component planes, 6. upsampling + colour conversion (+ gray)
     jpg_idct<<<(L.nblocks + 127) / 128, 128, 0, st>>>(coef, dcpre, L.G, L.nmcu, L.nblocks);

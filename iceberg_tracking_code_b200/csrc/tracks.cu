@@ -16,46 +16,6 @@ alive_count_kernel(const uint8_t *__restrict__ alive, int n, int32_t *__restrict
     if (threadIdx.x == 0) block_counts[blockIdx.x] = c;
 }
 
-// exclusive scan of block_counts[0..nb) in place by one CTA; total -> *total_out
-__global__ void __launch_bounds__(1024)
-block_scan_kernel(int32_t *__restrict__ block_counts, int nb, int32_t *__restrict__ total_out)
-{
-    __shared__ int32_t warp_tot[32];
-    __shared__ int32_t carry_s;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (int base = 0; base < nb; base += 1024) {
-        const int i = base + threadIdx.x;
-        const int32_t v = i < nb ? block_counts[i] : 0;
-        int32_t inc = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int32_t t = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= o) inc += t;
-        }
-        if (lane == 31) warp_tot[wid] = inc;
-        __syncthreads();
-        if (wid == 0) {
-            int32_t w = warp_tot[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int32_t t = __shfl_up_sync(0xffffffffu, w, o);
-                if (lane >= o) w += t;
-            }
-            warp_tot[lane] = w;
-        }
-        __syncthreads();
-        const int32_t woff = wid ? warp_tot[wid - 1] : 0;
-        const int32_t c = carry_s;
-        if (i < nb) block_counts[i] = c + woff + inc - v;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry_s = c + woff + inc;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) *total_out = carry_s;
-}
-
 __global__ void __launch_bounds__(CB)
 tracks_scatter_kernel(const float2 *__restrict__ tracks_tm, const float *__restrict__ quality_tm,
                       const uint8_t *__restrict__ alive, int n, int T, const int32_t *__restrict__ block_off,
@@ -88,9 +48,12 @@ static int tracks_compact_enqueue(const float *tracks_tm, const float *quality_t
     if (!tracks_tm || !quality_tm || !alive || !scratch || !out_tracks || !out_quality ||
         reinterpret_cast<uintptr_t>(tracks_tm) % 8 != 0 || reinterpret_cast<uintptr_t>(out_tracks) % 8 != 0)
         return IBT_E_INVALID;
+    // scratch: (N + 1) words, block counts -> block offsets in [0, nb), survivor count at [N].  The scan's partial sums, when
+    // it needs any (ceil(nb / 1024) words), fit in [nb, N): N > 256 * (nb - 1).
     const int nb = (N + CB - 1) / CB;
+    uint32_t *counts = reinterpret_cast<uint32_t *>(scratch);
     alive_count_kernel<<<nb, CB, 0, st>>>(alive, N, scratch);
-    block_scan_kernel<<<1, 1024, 0, st>>>(scratch, nb, scratch + N);
+    launch_scan(counts, counts, counts + nb, nb, 1, 0, counts + N, st);
     tracks_scatter_kernel<<<nb, CB, 0, st>>>(reinterpret_cast<const float2 *>(tracks_tm), quality_tm, alive, N, T, scratch,
                                              reinterpret_cast<float2 *>(out_tracks), out_quality);
     return check_launch("ibt_tracks_compact");

@@ -224,6 +224,27 @@ def test_tracks_compact_and_empty_group(ibt):
     assert trk.harvest()[0].shape == (0,)
 
 
+@pytest.mark.parametrize("n", [1, 262144, 262145, 300000, 2097152, 2097153])
+def test_tracks_compact_across_scan_tiles(ibt, n):
+    """Compaction of n tracks: its ceil(n / 256) block counts take one 1024-element step of the one-CTA scan up to
+    n = 262 144, several steps up to n = 2 097 152 (8 192 counts), and the multi-tile scan (partial sums inside the
+    scratch) above."""
+    from iceberg_tracking_code_b200.tracking import SequenceTracker
+    rng = np.random.default_rng(n)
+    T = 3
+    tm = rng.standard_normal((T + 1, n, 2)).astype(np.float32)
+    qm = rng.random((T, n), dtype=np.float32)
+    alive = rng.random(n) < 0.7
+    alive[-1] = True
+    trk = SequenceTracker()
+    trk.n, trk.T, trk.steps = n, T, T
+    trk._tracks, trk._quality = torch.from_numpy(tm).cuda(), torch.from_numpy(qm).cuda()
+    trk._alive = torch.from_numpy(alive.astype(np.uint8)).cuda()
+    want_t, want_q = tm[:, alive].transpose(1, 0, 2), qm[:, alive].T
+    for tracks, quality in (trk.harvest(), trk.finalize(trk.harvest_async())):
+        assert np.array_equal(tracks, want_t) and np.array_equal(quality, want_q)
+
+
 def test_config2_full_size_properties(ibt, oracle):
     """BASELINE config 2 at full size (6000x4000, 20k points, win 31, L4): determinism, known synthetic shift,
     FB round trip, and a sampled comparison with the oracle (the oracle is too slow for all 20k)."""
