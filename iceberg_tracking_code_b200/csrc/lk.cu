@@ -19,12 +19,15 @@
 //      template entries.  The mismatch vector is  b = sum(Jw*Ix) - C1  (sum(Jw*Iy) - C2): identical, as an exact
 //      integer, to OpenCV's sum((Jw - Iw)*Ix), and it halves the template.  Template entries outside the window are
 //      zero, so the iteration loop carries no masks.
+// Multi-channel frames (cv2 takes 3- and 4-channel images) run the same solver with every window sum taken over the channel
+// planes as well, on the runtime-window kernel without tensor maps.
 // All sums are exact integers (int32 per lane, REDUX across the warp, int64 totals) rounded to float once; OpenCV
 // accumulates in float SIMD lanes, which differs in the last bits only.  Float arithmetic that OpenCV does unfused is
 // compiled with -fmad=false.
 #include "common.cuh"
 #include <stdlib.h>
 #include <string.h>
+#include <type_traits>
 #include <mutex>
 #include <vector>
 
@@ -69,6 +72,15 @@ struct LKPyr {
 // tensor maps of both pyramids: [pyramid][level]; boxes = I window, J search patch, Scharr window
 struct LKMaps {
     CUtensorMap imgI[2][IBT_MAX_LEVELS], imgJ[2][IBT_MAX_LEVELS], der[2][IBT_MAX_LEVELS];
+};
+// Multi-channel frames (ibt_lk_multichannel): cn single-channel pyramids per frame, one per channel plane (built by the
+// single-channel kernels).  OpenCV sums every window quantity (structure tensor, mismatch vector, residual) over the window
+// pixels AND the channels; the min-eigenvalue test and the Newton update are unchanged, err is divided by 32 * winW * cn * winH.
+// These pyramids carry no tensor maps, so they are staged by cp.async and the gather.
+constexpr int LK_MC_MAX = 4;
+struct LKMcPyr {
+    LKPyr I[LK_MC_MAX], J[LK_MC_MAX];
+    int cn;
 };
 
 struct LKArgs {
@@ -522,16 +534,28 @@ __device__ __noinline__ long long window_err(const LKArgs &a, const uint8_t *jpa
     return S;
 }
 
-// One pyramidal pass for one point.  On entry (ox, oy) holds the initial flow if use_init.
-// On exit (ox, oy) = nextPts[k], status/err as cv2 (err = 0 where status == 0).
-template <int WW, int WH>
-__device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const LKArgs &a, float ptx, float pty,
+// Channel c's copy of p, `stride` bytes per channel after channel 0's.  Channel c owns the slab bytes [c, c + 1) * warp_smem,
+// and its pyramid levels lie in PI[c], PJ[c].
+template <typename T>
+__device__ __forceinline__ T *lk_chan(T *p, int c, int stride)
+{
+    using B = std::conditional_t<std::is_const<T>::value, const unsigned char, unsigned char>;
+    return reinterpret_cast<T *>(reinterpret_cast<B *>(p) + (size_t)c * stride);
+}
+
+// One pyramidal pass for one point over cn channel planes (PI[c], PJ[c]: the pyramids of channel c); every window sum runs
+// over the pixels and the channels.  CN is the channel count, or 0 for a runtime cn: CN = 1 folds the channel loops away.
+// On entry (ox, oy) holds the initial flow if use_init.  On exit (ox, oy) = nextPts[k], status/err as cv2 (err = 0 where
+// status == 0).
+template <int WW, int WH, int CN>
+__device__ __forceinline__ void lk_point(const LKPyr *PI, const LKPyr *PJ, int cn_rt, const LKArgs &a, float ptx, float pty,
                                          bool use_init, bool want_status, bool want_err, float &ox, float &oy, int &status,
                                          float &err, int &iters, unsigned char *slab, int rowbase, int cq, bool lane_on,
                                          int lane, const CUtensorMap *mapI, const CUtensorMap *mapJ, const CUtensorMap *mapD,
                                          uint64_t *bars, unsigned &phases)
 {
     const float FLT_SCALE = 1.f / (1 << 20);
+    const int cn = CN ? CN : cn_rt;
     const int winW = WW ? WW : a.winW, winH = WH ? WH : a.winH;
     const int IPITCH = WW ? lk_ipitch(WW) : a.ipitch, JPITCH = WW ? lk_jpitch(WW) : a.jpitch;
     const int DPITCH = WW ? lk_dpitch(WW) : a.dpitch;
@@ -541,11 +565,14 @@ __device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const
     uint32_t *dpatch = reinterpret_cast<uint32_t *>(slab);
     uint8_t *ipatch = slab + a.off_ipatch;
     uint8_t *jpatch = slab + a.off_jpatch;
+    auto ch = [&](auto *p, int c) { return lk_chan(p, c, a.warp_smem); };                      // of a slab buffer
+    auto chl = [](const LKLevel &l, int c) -> const LKLevel & { return *lk_chan(&l, c, (int)sizeof(LKPyr)); };  // of a level
     status = 1; err = 0.f;
-    const int L = PI.nlevels;
+    const int L = PI[0].nlevels;
     for (int level = L - 1; level >= 0; --level) {
-        const LKLevel &LI = PI.lv[level];
-        const LKLevel &LJ = PJ.lv[level];
+        // channel 0 decides geometry and staging: every channel has the same sizes, and multi-channel pyramids have no tensor maps
+        const LKLevel &LI = PI[0].lv[level];
+        const LKLevel &LJ = PJ[0].lv[level];
         const int rows = LI.rows, cols = LI.cols;
         const float sc = __int_as_float((127 - level) << 23);       // 2^-level
         float ppx = __fmul_rn(ptx, sc), ppy = __fmul_rn(pty, sc);
@@ -598,10 +625,13 @@ __device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const
                 tma_load_2d(jpatch, &mapJ[level], px0, py0, &bars[1]);
             }
         }
-        if (!i_tma) stage_bytes(LI, ipxa, ipy, winH + 1, IPITCH, lane, ipatch);
-        if (!d_tma) stage_deriv<WW, WH>(LI, a, ipx, ipy, dpatch, lane);
+        for (int c = 0; c < cn; c++) {
+            if (!i_tma) stage_bytes(chl(LI, c), ipxa, ipy, winH + 1, IPITCH, lane, ch(ipatch, c));
+            if (!d_tma) stage_deriv<WW, WH>(chl(LI, c), a, ipx, ipy, ch(dpatch, c), lane);
+        }
         cp_async_commit();
-        if (j_ok && !j_tma) stage_bytes(LJ, px0, py0, JROWS, JPITCH, lane, jpatch);
+        if (j_ok && !j_tma)
+            for (int c = 0; c < cn; c++) stage_bytes(chl(LJ, c), px0, py0, JROWS, JPITCH, lane, ch(jpatch, c));
         cp_async_commit();
         cp_async_wait<1>();
         if (i_tma || d_tma) { mbar_wait(&bars[0], phases & 1u); phases ^= 1u; }
@@ -615,8 +645,15 @@ __device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const
 
         // ---- template window: (Ix, Iy) per pixel; structure tensor; C1 = sum Iw*Ix, C2 = sum Iw*Iy -------------------------
         long long sA11, sA12, sA22, sC1, sC2;
+        // channel 0 sets the sums and the other channels add theirs (a loop from channel 0 costs the 35 x 35 kernel spills)
         build_template<WW, WH>(a, ipatch + (ipx - ipxa), dpatch + doff, tmpl, wtop, wbot, iw00, iw01, iw10, iw11, lane,
                                sA11, sA12, sA22, sC1, sC2);
+        for (int c = 1; c < cn; c++) {
+            long long t11, t12, t22, tc1, tc2;
+            build_template<WW, WH>(a, ch(ipatch, c) + (ipx - ipxa), ch(dpatch, c) + doff, ch(tmpl, c), wtop, wbot, iw00, iw01, iw10, iw11, lane,
+                                   t11, t12, t22, tc1, tc2);
+            sA11 += t11; sA12 += t12; sA22 += t22; sC1 += tc1; sC2 += tc2;
+        }
         cp_async_wait<0>();
         if (j_tma) { mbar_wait(&bars[1], (phases >> 1) & 1u); phases ^= 2u; }
         __syncwarp();
@@ -643,12 +680,16 @@ __device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const
             }
             if (!staged || (unsigned)(inx - vx0) > 2u * LK_MARGIN || (unsigned)(iny - py0) > 2u * LK_MARGIN) {
                 vx0 = inx - LK_MARGIN; px0 = vx0 & ~3; py0 = iny - LK_MARGIN;
-                restage_sync(LJ, px0, py0, JROWS, JPITCH, jpatch, lane);
+                for (int c = 0; c < cn; c++) restage_sync(chl(LJ, c), px0, py0, JROWS, JPITCH, ch(jpatch, c), lane);
                 staged = true;
             }
             bilinear_weights(__fsub_rn(nx, (float)inx), __fsub_rn(ny, (float)iny), wtop, wbot, iw00, iw01, iw10, iw11);
-            long long sb1, sb2;
-            newton_sums<WW, WH>(a, jpatch, inx - px0, iny - py0, wtop, wbot, tmpl, rowbase, cq, lane_on, sb1, sb2);
+            long long sb1 = 0, sb2 = 0;
+            for (int c = 0; c < cn; c++) {
+                long long t1, t2;
+                newton_sums<WW, WH>(a, ch(jpatch, c), inx - px0, iny - py0, wtop, wbot, ch(tmpl, c), rowbase, cq, lane_on, t1, t2);
+                sb1 += t1; sb2 += t2;
+            }
             ++iters;
             const float b1 = __fmul_rn(__ll2float_rn(sb1 - sC1), FLT_SCALE);
             const float b2 = __fmul_rn(__ll2float_rn(sb2 - sC2), FLT_SCALE);
@@ -672,12 +713,14 @@ __device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const
             if (!want_err) continue;
             if (!staged || (unsigned)(iqx - vx0) > 2u * LK_MARGIN || (unsigned)(iqy - py0) > 2u * LK_MARGIN) {
                 vx0 = iqx - LK_MARGIN; px0 = vx0 & ~3; py0 = iqy - LK_MARGIN;
-                restage_sync(LJ, px0, py0, JROWS, JPITCH, jpatch, lane);
+                for (int c = 0; c < cn; c++) restage_sync(chl(LJ, c), px0, py0, JROWS, JPITCH, ch(jpatch, c), lane);
             }
             bilinear_weights(__fsub_rn(qx, (float)iqx), __fsub_rn(qy, (float)iqy), wtop, wbot, iw00, iw01, iw10, iw11);
-            const long long s = window_err<WW, WH>(a, jpatch, iqx - px0, iqy - py0, wtop, wbot, ipatch, ipx - ipxa, iwtop, iwbot,
-                                                   rowbase, cq, lane_on);
-            err = __fdiv_rn(__ll2float_rn(s), (float)(32 * winW * winH));
+            long long s = 0;
+            for (int c = 0; c < cn; c++)
+                s += window_err<WW, WH>(a, ch(jpatch, c), iqx - px0, iqy - py0, wtop, wbot, ch(ipatch, c), ipx - ipxa, iwtop, iwbot,
+                                        rowbase, cq, lane_on);
+            err = __fdiv_rn(__ll2float_rn(s), (float)(32 * winW * cn * winH));
         }
         __syncwarp();
     }
@@ -685,9 +728,15 @@ __device__ __forceinline__ void lk_point(const LKPyr &PI, const LKPyr &PJ, const
     if (!status && !(a.flags & IBT_LK_GET_MIN_EIGENVALS)) err = 0.f;
 }
 
-template <int WW, int WH>
-__global__ void __launch_bounds__(256, 3)
-lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKMaps maps)
+// The kernel's second parameter: gray frames (CN = 1) bring the tensor maps of a.pyr, multi-channel frames (CN = 0, any cn)
+// their channel pyramids (a.pyr unused).
+template <int CN> using LKFrames = std::conditional_t<CN == 1, LKMaps, LKMcPyr>;
+
+// Gray frames: 3 CTAs of 8 warps per SM (80 registers).  Multi-channel frames: no minimum (0), which keeps the runtime-cn
+// solver out of local memory (128 registers: 16 warps per SM).
+template <int WW, int WH, int CN>
+__global__ void __launch_bounds__(256, CN == 1 ? 3 : 0)
+lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKFrames<CN> fr)
 {
     extern __shared__ __align__(128) unsigned char lk_smem[];
     __shared__ __align__(8) uint64_t lk_bars[8][2];        // per warp: [0] I window + Scharr planes, [1] J patch
@@ -698,7 +747,9 @@ lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKMaps maps)
     }
     __syncwarp();
     unsigned phases = 0u;                                  // bit b = parity to wait for on lk_bars[wib][b]
-    unsigned char *slab = lk_smem + (size_t)wib * a.warp_smem;
+    int cn = 1;
+    if constexpr (CN != 1) cn = fr.cn;
+    unsigned char *slab = lk_smem + (size_t)wib * a.warp_smem * cn;     // cn channel slabs per warp
     // Newton mapping of this lane: row group and column quad (lanes beyond the last group idle on group 0's rows)
     const int NL = WW ? lk_nl(WW) : a.nl, NG = (WW && WH) ? lk_ng(WW, WH) : a.ng, RG = (WW && WH) ? lk_rg(WW, WH) : a.rg;
     const int grp = lane / NL;
@@ -722,9 +773,12 @@ lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKMaps maps)
         if (use_init) { ox = a.p1[2 * k]; oy = a.p1[2 * k + 1]; }
         const bool want_status = pass == 0 ? a.st1 != nullptr : a.st0 != nullptr;
         const bool want_err = pass == 0 ? a.err1 != nullptr : a.err0 != nullptr;
-        lk_point<WW, WH>(a.pyr[pass], a.pyr[pass ^ 1], a, ptx, pty, use_init, want_status, want_err, ox, oy, status, err, iters,
-                         slab, rowbase, cq, lane_on, lane, maps.imgI[pass], maps.imgJ[pass ^ 1], maps.der[pass], lk_bars[wib],
-                         phases);
+        const LKPyr *PI = a.pyr + pass, *PJ = a.pyr + (pass ^ 1);
+        const CUtensorMap *mapI = nullptr, *mapJ = nullptr, *mapD = nullptr;
+        if constexpr (CN == 1) { mapI = fr.imgI[pass]; mapJ = fr.imgJ[pass ^ 1]; mapD = fr.der[pass]; }
+        else { PI = fr.I; PJ = fr.J; }
+        lk_point<WW, WH, CN>(PI, PJ, cn, a, ptx, pty, use_init, want_status, want_err, ox, oy, status, err, iters,
+                             slab, rowbase, cq, lane_on, lane, mapI, mapJ, mapD, lk_bars[wib], phases);
         if (pass == 0) it_f = iters; else it_b = iters;
         if (lane == 0) {
             if (pass == 0) {
@@ -753,193 +807,6 @@ lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKMaps maps)
   }
     // the last warp to leave re-arms the work queue for the next launch on this stream (no memset node per launch)
     if (lane == 0) {
-        __threadfence();
-        if (atomicAdd(a.work_counter + 1, 1u) == a.total_warps - 1u) {
-            a.work_counter[0] = 0u; a.work_counter[1] = 0u;
-            __threadfence();
-        }
-    }
-}
-
-// ---- multi-channel images ------------------------------------------------------------------------------------------
-// cv2.calcOpticalFlowPyrLK also takes 3- (or 4-) channel 8-bit images (SURVEY 8b); the reference never does -- it converts
-// to gray first (s1:311) -- so this is the plain form of the solver, not the tuned one: no tensor maps, the generic
-// (runtime window) helpers, one pass.  OpenCV builds the pyramid and the Scharr planes per channel and sums every window
-// quantity (structure tensor, mismatch vector, residual) over the window pixels AND the channels; min-eigenvalue test and
-// Newton update are unchanged, err is divided by 32 * winW * cn * winH.  Channel planes arrive as cn single-channel
-// pyramids (the kernels that build them are the single-channel ones); channel c owns the c-th slab of a.warp_smem bytes.
-constexpr int LK_MC_MAX = 4;
-struct LKMcPyr {
-    LKPyr I[LK_MC_MAX], J[LK_MC_MAX];
-    int cn;
-};
-
-__device__ __noinline__ void lk_point_mc(const LKMcPyr &mc, const LKArgs &a, float ptx, float pty, bool use_init, bool want_status,
-                                         bool want_err, float &ox, float &oy, int &status, float &err, int &iters,
-                                         unsigned char *slab, int rowbase, int cq, bool lane_on, int lane)
-{
-    const float FLT_SCALE = 1.f / (1 << 20);
-    const int cn = mc.cn;
-    const int winW = a.winW, winH = a.winH;
-    const int IPITCH = a.ipitch, JPITCH = a.jpitch;
-    const int JROWS = winH + 1 + 2 * LK_MARGIN;
-    const float halfx = (winW - 1) * 0.5f, halfy = (winH - 1) * 0.5f;
-    status = 1; err = 0.f;
-    const int L = mc.I[0].nlevels;
-    for (int level = L - 1; level >= 0; --level) {
-        const int rows = mc.I[0].lv[level].rows, cols = mc.I[0].lv[level].cols;
-        const float sc = __int_as_float((127 - level) << 23);       // 2^-level
-        float ppx = __fmul_rn(ptx, sc), ppy = __fmul_rn(pty, sc);
-        float nx, ny;
-        if (level == L - 1) {
-            if (use_init) { nx = __fmul_rn(ox, sc); ny = __fmul_rn(oy, sc); }
-            else { nx = ppx; ny = ppy; }
-        } else { nx = __fmul_rn(ox, 2.f); ny = __fmul_rn(oy, 2.f); }
-        ox = nx; oy = ny;
-        ppx = __fsub_rn(ppx, halfx); ppy = __fsub_rn(ppy, halfy);
-        const int ipx = cv_floor(ppx), ipy = cv_floor(ppy);
-        if (window_oob(ipx, ipy, winW, winH, rows, cols)) {
-            if (level == 0) { status = 0; err = 0.f; }
-            continue;
-        }
-        nx = __fsub_rn(nx, halfx); ny = __fsub_rn(ny, halfy);
-        const int ipxa = ipx & ~3;
-        int px0 = 0, py0 = 0, vx0 = 0;
-        bool staged = false;
-        const int jnx = cv_floor(nx), jny = cv_floor(ny);
-        const bool j_ok = !window_oob(jnx, jny, winW, winH, rows, cols);
-        if (j_ok) { vx0 = jnx - LK_MARGIN; px0 = vx0 & ~3; py0 = jny - LK_MARGIN; staged = true; }
-        __syncwarp();
-        for (int c = 0; c < cn; c++) {
-            unsigned char *sl = slab + (size_t)c * a.warp_smem;
-            stage_bytes(mc.I[c].lv[level], ipxa, ipy, winH + 1, IPITCH, lane, sl + a.off_ipatch);
-            stage_deriv<0, 0>(mc.I[c].lv[level], a, ipx, ipy, reinterpret_cast<uint32_t *>(sl), lane);
-        }
-        cp_async_commit();
-        if (j_ok)
-            for (int c = 0; c < cn; c++)
-                stage_bytes(mc.J[c].lv[level], px0, py0, JROWS, JPITCH, lane, slab + (size_t)c * a.warp_smem + a.off_jpatch);
-        cp_async_commit();
-        cp_async_wait<1>();
-        __syncwarp();
-
-        uint32_t wtop, wbot;
-        int iw00, iw01, iw10, iw11;
-        bilinear_weights(__fsub_rn(ppx, (float)ipx), __fsub_rn(ppy, (float)ipy), wtop, wbot, iw00, iw01, iw10, iw11);
-        const uint32_t iwtop = wtop, iwbot = wbot;
-        long long sA11 = 0, sA12 = 0, sA22 = 0, sC1 = 0, sC2 = 0;
-        for (int c = 0; c < cn; c++) {
-            unsigned char *sl = slab + (size_t)c * a.warp_smem;
-            long long t11, t12, t22, tc1, tc2;
-            build_template<0, 0>(a, sl + a.off_ipatch + (ipx - ipxa), reinterpret_cast<uint32_t *>(sl), reinterpret_cast<uint32_t *>(sl),
-                                 wtop, wbot, iw00, iw01, iw10, iw11, lane, t11, t12, t22, tc1, tc2);
-            sA11 += t11; sA12 += t12; sA22 += t22; sC1 += tc1; sC2 += tc2;
-        }
-        cp_async_wait<0>();
-        __syncwarp();
-        const float A11 = __fmul_rn(__ll2float_rn(sA11), FLT_SCALE);
-        const float A12 = __fmul_rn(__ll2float_rn(sA12), FLT_SCALE);
-        const float A22 = __fmul_rn(__ll2float_rn(sA22), FLT_SCALE);
-        float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
-        const float dA = __fsub_rn(A11, A22);
-        const float disc = __fadd_rn(__fmul_rn(dA, dA), __fmul_rn(__fmul_rn(4.f, A12), A12));
-        const float minEig = __fdiv_rn(__fsub_rn(__fadd_rn(A22, A11), __fsqrt_rn(disc)), (float)(2 * winW * winH));
-        if (a.flags & IBT_LK_GET_MIN_EIGENVALS) err = minEig;
-        if (minEig < a.minEigThr || D < 1.1920929e-07f) {
-            if (level == 0) status = 0;
-            continue;
-        }
-        D = __fdiv_rn(1.f, D);
-        float pdx = 0.f, pdy = 0.f;
-        for (int j = 0; j < a.maxCount; j++) {
-            const int inx = cv_floor(nx), iny = cv_floor(ny);
-            if (window_oob(inx, iny, winW, winH, rows, cols)) {
-                if (level == 0) status = 0;
-                break;
-            }
-            if (!staged || (unsigned)(inx - vx0) > 2u * LK_MARGIN || (unsigned)(iny - py0) > 2u * LK_MARGIN) {
-                vx0 = inx - LK_MARGIN; px0 = vx0 & ~3; py0 = iny - LK_MARGIN;
-                for (int c = 0; c < cn; c++)
-                    restage_sync(mc.J[c].lv[level], px0, py0, JROWS, JPITCH, slab + (size_t)c * a.warp_smem + a.off_jpatch, lane);
-                staged = true;
-            }
-            bilinear_weights(__fsub_rn(nx, (float)inx), __fsub_rn(ny, (float)iny), wtop, wbot, iw00, iw01, iw10, iw11);
-            long long sb1 = 0, sb2 = 0;
-            for (int c = 0; c < cn; c++) {
-                const unsigned char *sl = slab + (size_t)c * a.warp_smem;
-                long long t1, t2;
-                newton_sums<0, 0>(a, sl + a.off_jpatch, inx - px0, iny - py0, wtop, wbot, reinterpret_cast<const uint32_t *>(sl),
-                                  rowbase, cq, lane_on, t1, t2);
-                sb1 += t1; sb2 += t2;
-            }
-            ++iters;
-            const float b1 = __fmul_rn(__ll2float_rn(sb1 - sC1), FLT_SCALE);
-            const float b2 = __fmul_rn(__ll2float_rn(sb2 - sC2), FLT_SCALE);
-            const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
-            const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D);
-            nx = __fadd_rn(nx, dx); ny = __fadd_rn(ny, dy);
-            ox = __fadd_rn(nx, halfx); oy = __fadd_rn(ny, halfy);
-            if (__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)) <= a.eps2) break;
-            if (j > 0 && fabsf(__fadd_rn(dx, pdx)) < 0.01f && fabsf(__fadd_rn(dy, pdy)) < 0.01f) {
-                ox = __fsub_rn(ox, __fmul_rn(dx, 0.5f)); oy = __fsub_rn(oy, __fmul_rn(dy, 0.5f));
-                break;
-            }
-            pdx = dx; pdy = dy;
-        }
-        if (status && level == 0 && !(a.flags & IBT_LK_GET_MIN_EIGENVALS) && (want_status || want_err)) {
-            const float qx = __fsub_rn(ox, halfx), qy = __fsub_rn(oy, halfy);
-            const int iqx = cv_floor(qx), iqy = cv_floor(qy);
-            if (window_oob(iqx, iqy, winW, winH, rows, cols)) { status = 0; err = 0.f; continue; }
-            if (!want_err) continue;
-            if (!staged || (unsigned)(iqx - vx0) > 2u * LK_MARGIN || (unsigned)(iqy - py0) > 2u * LK_MARGIN) {
-                vx0 = iqx - LK_MARGIN; px0 = vx0 & ~3; py0 = iqy - LK_MARGIN;
-                for (int c = 0; c < cn; c++)
-                    restage_sync(mc.J[c].lv[level], px0, py0, JROWS, JPITCH, slab + (size_t)c * a.warp_smem + a.off_jpatch, lane);
-            }
-            bilinear_weights(__fsub_rn(qx, (float)iqx), __fsub_rn(qy, (float)iqy), wtop, wbot, iw00, iw01, iw10, iw11);
-            long long s = 0;
-            for (int c = 0; c < cn; c++) {
-                const unsigned char *sl = slab + (size_t)c * a.warp_smem;
-                s += window_err<0, 0>(a, sl + a.off_jpatch, iqx - px0, iqy - py0, wtop, wbot, sl + a.off_ipatch, ipx - ipxa, iwtop, iwbot,
-                                      rowbase, cq, lane_on);
-            }
-            err = __fdiv_rn(__ll2float_rn(s), (float)(32 * winW * cn * winH));
-        }
-        __syncwarp();
-    }
-    cp_async_wait<0>();
-    if (!status && !(a.flags & IBT_LK_GET_MIN_EIGENVALS)) err = 0.f;
-}
-
-__global__ void __launch_bounds__(256)
-lk_mc_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKMcPyr mc)
-{
-    extern __shared__ __align__(128) unsigned char lk_smem[];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    unsigned char *slab = lk_smem + (size_t)wib * a.warp_smem * mc.cn;
-    const int grp = lane / a.nl;
-    const bool lane_on = grp < a.ng;
-    const int rowbase = lane_on ? grp * a.rg : 0, cq = lane_on ? lane - grp * a.nl : 0;
-    for (;;) {
-        int k = 0;
-        if (lane == 0) k = (int)atomicAdd(a.work_counter, 1u);
-        k = __shfl_sync(0xffffffffu, k, 0);
-        if (k >= a.n) break;
-        float ox = 0.f, oy = 0.f, err;
-        int status, iters = 0;
-        const bool use_init = (a.flags & IBT_LK_USE_INITIAL_FLOW) != 0;
-        if (use_init) { ox = a.p1[2 * k]; oy = a.p1[2 * k + 1]; }
-        lk_point_mc(mc, a, a.p0[2 * k], a.p0[2 * k + 1], use_init, a.st1 != nullptr, a.err1 != nullptr, ox, oy, status, err, iters,
-                    slab, rowbase, cq, lane_on, lane);
-        if (lane == 0) {
-            a.p1[2 * k] = ox; a.p1[2 * k + 1] = oy;
-            if (a.st1) a.st1[k] = (uint8_t)status;
-            if (a.err1) a.err1[k] = err;
-            if (a.iters) a.iters[k] = iters;
-        }
-        __syncwarp();
-    }
-    if (lane == 0) {                                       // the last warp to leave re-arms the work queue (see lk_kernel)
         __threadfence();
         if (atomicAdd(a.work_counter + 1, 1u) == a.total_warps - 1u) {
             a.work_counter[0] = 0u; a.work_counter[1] = 0u;
@@ -992,19 +859,30 @@ static int lk_queue_for(int dev, cudaStream_t st, unsigned int **out)
     return IBT_OK;
 }
 
-static int launch_lk(LKArgs &a, const ibt_pyramid_t *A, const ibt_pyramid_t *B, int winW, int winH, int max_count,
-                     double epsilon, double min_eig, cudaStream_t st)
+// The one launcher of every LK entry point.  A and B are host arrays of cn pyramids, one per channel plane.  planes == false
+// (ibt_lk, ibt_lk_fb; cn == 1): gray frames in a.pyr, with tensor maps, on the window-specialised kernels.  planes == true
+// (ibt_lk_multichannel): the channel pyramids travel as LKMcPyr to the runtime-cn kernel.
+static int launch_lk(LKArgs &a, const ibt_pyramid_t *const *A, const ibt_pyramid_t *const *B, int cn, bool planes, int winW,
+                     int winH, int max_count, double epsilon, double min_eig, cudaStream_t st)
 {
-    if (a.n < 0 || winW < 3 || winH < 3 || winW > IBT_MAX_WIN || winH > IBT_MAX_WIN) return IBT_E_INVALID;
+    if (a.n < 0 || winW < 3 || winH < 3 || winW > IBT_MAX_WIN || winH > IBT_MAX_WIN || cn < 1 || cn > LK_MC_MAX || !A || !B)
+        return IBT_E_INVALID;
     if (a.n == 0) return IBT_OK;
     if (!a.p0 || !a.p1) return IBT_E_INVALID;
-    int rc = fill_pyr(A, a.pyr[0], true);
-    if (rc) return rc;
-    rc = fill_pyr(B, a.pyr[1], a.fb != 0);
-    if (rc) return rc;
-    if (A->nlevels != B->nlevels) return IBT_E_INVALID;
-    for (int l = 0; l < A->nlevels; l++)
-        if (A->rows[l] != B->rows[l] || A->cols[l] != B->cols[l]) return IBT_E_INVALID;
+    static thread_local LKMcPyr mc;
+    LKPyr *PI = planes ? mc.I : &a.pyr[0], *PJ = planes ? mc.J : &a.pyr[1];
+    mc.cn = cn;
+    for (int c = 0; c < cn; c++) {
+        int rc = fill_pyr(A[c], PI[c], true);
+        if (rc) return rc;
+        rc = fill_pyr(B[c], PJ[c], a.fb != 0);
+        if (rc) return rc;
+        if (A[c]->nlevels != A[0]->nlevels || B[c]->nlevels != A[0]->nlevels) return IBT_E_INVALID;
+        for (int l = 0; l < A[0]->nlevels; l++)
+            if (A[c]->rows[l] != A[0]->rows[l] || A[c]->cols[l] != A[0]->cols[l] || B[c]->rows[l] != A[0]->rows[l] ||
+                B[c]->cols[l] != A[0]->cols[l])
+                return IBT_E_INVALID;
+    }
     a.winW = winW; a.winH = winH;
     a.nl = lk_nl(winW); a.ng = lk_ng(winW, winH); a.rg = lk_rg(winW, winH);
     a.trows = lk_trows(winW, winH); a.tcols = lk_tcols(winW);
@@ -1024,20 +902,19 @@ static int launch_lk(LKArgs &a, const ibt_pyramid_t *A, const ibt_pyramid_t *B, 
     a.off_ipatch = (int)off; off += (size_t)(winH + 1) * a.ipitch; off = (off + 127) & ~(size_t)127;
     // Newton lanes of the last row group read (never use) J rows down to trows + 2 * MARGIN
     a.off_jpatch = (int)off; off += (size_t)(a.trows + 1 + 2 * LK_MARGIN) * a.jpitch;
-    a.warp_smem = (int)((off + 127) & ~(size_t)127);
+    a.warp_smem = (int)((off + 127) & ~(size_t)127);      // one slab per channel
     // tensor maps (boxes: I window ipitch x (winH+1), J patch jpitch x jrows, Scharr window dpitch words x (winH+1))
     static thread_local LKMaps maps;
     static const bool no_tma = getenv("IBT_NO_TMA") != nullptr;
-    static const int tma_mask = getenv("IBT_LK_TMA") ? atoi(getenv("IBT_LK_TMA")) : 3;      // 1: intensity patches, 2: Scharr
-    for (int pi = 0; pi < 2 && !no_tma; pi++) {
-        const ibt_pyramid_t *P = pi ? B : A;
+    for (int pi = 0; pi < 2 && !planes && !no_tma; pi++) {
+        const ibt_pyramid_t *P = pi ? B[0] : A[0];
         for (int l = 0; l < P->nlevels; l++) {
             LKLevel &lv = a.pyr[pi].lv[l];
-            lv.tma_img = (tma_mask & 1) && make_map_2d(&maps.imgI[pi][l], CU_TENSOR_MAP_DATA_TYPE_UINT8, P->img[l], P->cols[l], P->rows[l],
+            lv.tma_img = make_map_2d(&maps.imgI[pi][l], CU_TENSOR_MAP_DATA_TYPE_UINT8, P->img[l], P->cols[l], P->rows[l],
                                      P->img_pitch[l], a.ipitch, winH + 1) &&
                          make_map_2d(&maps.imgJ[pi][l], CU_TENSOR_MAP_DATA_TYPE_UINT8, P->img[l], P->cols[l], P->rows[l],
                                      P->img_pitch[l], a.jpitch, a.jrows);
-            lv.tma_der = (tma_mask & 2) && P->deriv[l] != nullptr &&
+            lv.tma_der = P->deriv[l] != nullptr &&
                          make_map_2d(&maps.der[pi][l], CU_TENSOR_MAP_DATA_TYPE_UINT32, P->deriv[l], P->cols[l], P->rows[l],
                                      P->deriv_pitch[l], a.dpitch, winH + 1);
         }
@@ -1047,37 +924,30 @@ static int launch_lk(LKArgs &a, const ibt_pyramid_t *A, const ibt_pyramid_t *B, 
     if (epsilon > 10) epsilon = 10;
     a.eps2 = (float)(epsilon * epsilon);
     a.minEigThr = (float)min_eig;
-    // warps per CTA: the choice that keeps the most warps resident in 227 KB of shared memory per SM (at most 24: the
-    // kernel is compiled for 3 CTAs of 8 warps per SM, 85 registers per thread)
+    // warps per CTA: the choice that keeps the most warps resident in 227 KB of shared memory per SM, at most as many as the
+    // registers allow (gray kernels: compiled for 3 CTAs of 8 warps per SM, 80 registers; runtime-cn kernel: 128 registers)
+    const size_t per_warp = (size_t)a.warp_smem * cn;
+    const int max_warps = planes ? 16 : 24;
     int wpc = 1, best = 0, best_ctas = 1;
     for (int w = 1; w <= 8; w++) {
-        const size_t per_cta = (size_t)a.warp_smem * w + 1024;
+        const size_t per_cta = per_warp * w + 1024;
         if (per_cta > 200 * 1024) break;
         int ctas = (int)((227 * 1024) / per_cta);
         if (ctas > 32) ctas = 32;
-        if (ctas * w > 24) ctas = 24 / w;
+        if (ctas * w > max_warps) ctas = max_warps / w;
         const int warps = ctas * w;
         if (warps >= best) { best = warps; wpc = w; best_ctas = ctas; }
     }
     if (best == 0) return IBT_E_INVALID;
-    if (const char *e = getenv("IBT_LK_WPC")) {             // tuning knob (warps per CTA); the default is the choice above
-        const int w = atoi(e);
-        if (w >= 1 && w <= 8 && (size_t)a.warp_smem * w + 1024 <= 200 * 1024) {
-            wpc = w;
-            best_ctas = (int)((227 * 1024) / ((size_t)a.warp_smem * w + 1024));
-            if (best_ctas > 32) best_ctas = 32;
-            if (const char *c = getenv("IBT_LK_CTAS")) { const int v = atoi(c); if (v >= 1 && v < best_ctas) best_ctas = v; }
-        }
-    }
     {
         std::lock_guard<std::mutex> lock(lk_mu);
         if (lk_max_ctas_per_sm > 0 && best_ctas > lk_max_ctas_per_sm) best_ctas = lk_max_ctas_per_sm;
     }
-    const size_t smem = (size_t)a.warp_smem * wpc;
-    void (*kern)(const LKArgs, const LKMaps) = lk_kernel<0, 0>;      // generic window; the sizes the configs use are specialised
-    if (winW == 21 && winH == 21) kern = lk_kernel<21, 21>;
-    else if (winW == 31 && winH == 31) kern = lk_kernel<31, 31>;
-    else if (winW == 35 && winH == 35) kern = lk_kernel<35, 35>;
+    const size_t smem = per_warp * wpc;
+    void (*kern)(const LKArgs, const LKMaps) = lk_kernel<0, 0, 1>;      // generic window; the sizes the configs use are specialised
+    if (winW == 21 && winH == 21) kern = lk_kernel<21, 21, 1>;
+    else if (winW == 31 && winH == 31) kern = lk_kernel<31, 31, 1>;
+    else if (winW == 35 && winH == 35) kern = lk_kernel<35, 35, 1>;
     int dev_id = 0;
     IBT_CUDA_TRY(cudaGetDevice(&dev_id));
     if (dev_id < 0 || dev_id >= 64) return IBT_E_INVALID;
@@ -1085,92 +955,24 @@ static int launch_lk(LKArgs &a, const ibt_pyramid_t *A, const ibt_pyramid_t *B, 
         std::lock_guard<std::mutex> lock(lk_mu);
         if (!lk_attr_set[dev_id]) {
             const int lim = 200 * 1024;
-            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
-            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<21, 21>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
-            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<31, 31>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
-            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<35, 35>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<0, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<21, 21, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<31, 31, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<35, 35, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_kernel<0, 0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
             lk_attr_set[dev_id] = true;
         }
-        rc = lk_queue_for(dev_id, st, &a.work_counter);
+        const int rc = lk_queue_for(dev_id, st, &a.work_counter);
         if (rc) return rc;
     }
     int blocks = kNumSMs * best_ctas;                   // persistent: one wave, warps pull points until none are left
     const int need = (a.n + wpc - 1) / wpc;
     if (blocks > need) blocks = need;
     a.total_warps = (unsigned)(blocks * wpc);
-    kern<<<blocks, wpc * 32, smem, st>>>(a, maps);          // the tensor maps travel as a __grid_constant__ parameter
-    return check_launch("ibt_lk");
-}
-
-// cv2.calcOpticalFlowPyrLK on multi-channel images: cn single-channel pyramids per image (channel planes)
-static int launch_lk_mc(LKArgs &a, const ibt_pyramid_t *const *A, const ibt_pyramid_t *const *B, int cn, int winW, int winH,
-                        int max_count, double epsilon, double min_eig, cudaStream_t st)
-{
-    if (a.n < 0 || winW < 3 || winH < 3 || winW > IBT_MAX_WIN || winH > IBT_MAX_WIN || cn < 1 || cn > LK_MC_MAX || !A || !B)
-        return IBT_E_INVALID;
-    if (a.n == 0) return IBT_OK;
-    if (!a.p0 || !a.p1) return IBT_E_INVALID;
-    static thread_local LKMcPyr mc;
-    mc.cn = cn;
-    for (int c = 0; c < cn; c++) {
-        int rc = fill_pyr(A[c], mc.I[c], true);
-        if (rc) return rc;
-        rc = fill_pyr(B[c], mc.J[c], false);
-        if (rc) return rc;
-        if (A[c]->nlevels != A[0]->nlevels || B[c]->nlevels != A[0]->nlevels) return IBT_E_INVALID;
-        for (int l = 0; l < A[0]->nlevels; l++)
-            if (A[c]->rows[l] != A[0]->rows[l] || A[c]->cols[l] != A[0]->cols[l] || B[c]->rows[l] != A[0]->rows[l] ||
-                B[c]->cols[l] != A[0]->cols[l])
-                return IBT_E_INVALID;
-    }
-    a.winW = winW; a.winH = winH;
-    a.nl = lk_nl(winW); a.ng = lk_ng(winW, winH); a.rg = lk_rg(winW, winH);
-    a.trows = lk_trows(winW, winH); a.tcols = lk_tcols(winW);
-    a.nstrips = lk_nstrips(winW);
-    a.strip_cols = lk_strip_cols(winW);
-    a.dpitch = lk_dpitch(winW);
-    a.ipitch = lk_ipitch(winW);
-    a.jpitch = lk_jpitch(winW);
-    a.jrows = winH + 1 + 2 * LK_MARGIN;
-    size_t off = (size_t)a.trows * a.tcols * 4;                  // per-channel slab: the layout of launch_lk
-    const size_t dbytes = (size_t)(winH + 1) * a.dpitch * 4;
-    if (off < dbytes) off = dbytes;
-    off = (off + 127) & ~(size_t)127;
-    a.off_ipatch = (int)off; off += (size_t)(winH + 1) * a.ipitch; off = (off + 127) & ~(size_t)127;
-    a.off_jpatch = (int)off; off += (size_t)(a.trows + 1 + 2 * LK_MARGIN) * a.jpitch;
-    a.warp_smem = (int)((off + 127) & ~(size_t)127);
-    a.maxCount = max_count < 0 ? 0 : (max_count > 100 ? 100 : max_count);
-    if (epsilon < 0) epsilon = 0;
-    if (epsilon > 10) epsilon = 10;
-    a.eps2 = (float)(epsilon * epsilon);
-    a.minEigThr = (float)min_eig;
-    const size_t per_warp = (size_t)a.warp_smem * cn;
-    int wpc = (int)((200 * 1024) / per_warp);
-    if (wpc < 1) return IBT_E_INVALID;
-    if (wpc > 8) wpc = 8;
-    const size_t smem = per_warp * wpc;
-    int ctas = (int)((227 * 1024) / (smem + 1024));
-    if (ctas < 1) ctas = 1;
-    if (ctas * wpc > 16) ctas = 16 / wpc > 0 ? 16 / wpc : 1;
-    int dev_id = 0;
-    IBT_CUDA_TRY(cudaGetDevice(&dev_id));
-    if (dev_id < 0 || dev_id >= 64) return IBT_E_INVALID;
-    {
-        std::lock_guard<std::mutex> lock(lk_mu);
-        static bool mc_attr_set[64] = {false};
-        if (!mc_attr_set[dev_id]) {
-            IBT_CUDA_TRY(cudaFuncSetAttribute(lk_mc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            mc_attr_set[dev_id] = true;
-        }
-        const int rc = lk_queue_for(dev_id, st, &a.work_counter);
-        if (rc) return rc;
-    }
-    int blocks = kNumSMs * ctas;
-    const int need = (a.n + wpc - 1) / wpc;
-    if (blocks > need) blocks = need;
-    a.total_warps = (unsigned)(blocks * wpc);
-    lk_mc_kernel<<<blocks, wpc * 32, smem, st>>>(a, mc);
-    return check_launch("ibt_lk_multichannel");
+    // the tensor maps or the channel pyramids travel as a __grid_constant__ parameter
+    if (planes) lk_kernel<0, 0, 0><<<blocks, wpc * 32, smem, st>>>(a, mc);
+    else kern<<<blocks, wpc * 32, smem, st>>>(a, maps);
+    return check_launch(planes ? "ibt_lk_multichannel" : "ibt_lk");
 }
 
 } // namespace ibt
@@ -1191,7 +993,8 @@ IBT_API int ibt_lk(const ibt_pyramid_t *pyrI, const ibt_pyramid_t *pyrJ, const f
     memset(&a, 0, sizeof(a));
     a.p0 = pts; a.n = N; a.flags = flags; a.fb = 0;
     a.p1 = next_pts; a.st1 = status; a.err1 = err; a.iters = iters;
-    return ibt::launch_lk(a, pyrI, pyrJ, winW, winH, max_count, epsilon, min_eig_threshold, static_cast<cudaStream_t>(stream));
+    return ibt::launch_lk(a, &pyrI, &pyrJ, 1, false, winW, winH, max_count, epsilon, min_eig_threshold,
+                          static_cast<cudaStream_t>(stream));
 }
 
 IBT_API int ibt_lk_fb(const ibt_pyramid_t *prev, const ibt_pyramid_t *next, const float *p0, int N, int winW, int winH,
@@ -1204,7 +1007,8 @@ IBT_API int ibt_lk_fb(const ibt_pyramid_t *prev, const ibt_pyramid_t *next, cons
     a.p0 = p0; a.n = N; a.flags = 0; a.fb = 1; a.fb_thresh = fb_threshold;
     a.p1 = p1; a.st1 = st1; a.err1 = err1; a.p0r = p0r; a.st0 = st0; a.err0 = err0;
     a.fbdist = fbdist; a.alive = alive; a.iters = iters; a.iter_total = iter_total;
-    return ibt::launch_lk(a, prev, next, winW, winH, max_count, epsilon, min_eig_threshold, static_cast<cudaStream_t>(stream));
+    return ibt::launch_lk(a, &prev, &next, 1, false, winW, winH, max_count, epsilon, min_eig_threshold,
+                          static_cast<cudaStream_t>(stream));
 }
 
 IBT_API int ibt_lk_multichannel(const ibt_pyramid_t *const *pyrI, const ibt_pyramid_t *const *pyrJ, int cn, const float *pts,
@@ -1215,5 +1019,6 @@ IBT_API int ibt_lk_multichannel(const ibt_pyramid_t *const *pyrI, const ibt_pyra
     memset(&a, 0, sizeof(a));
     a.p0 = pts; a.n = N; a.flags = flags; a.fb = 0;
     a.p1 = next_pts; a.st1 = status; a.err1 = err; a.iters = iters;
-    return ibt::launch_lk_mc(a, pyrI, pyrJ, cn, winW, winH, max_count, epsilon, min_eig_threshold, static_cast<cudaStream_t>(stream));
+    return ibt::launch_lk(a, pyrI, pyrJ, cn, true, winW, winH, max_count, epsilon, min_eig_threshold,
+                          static_cast<cudaStream_t>(stream));
 }

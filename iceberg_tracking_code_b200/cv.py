@@ -259,38 +259,6 @@ def _channels(img):
     return int(img.shape[2])
 
 
-def _lk_multichannel(prevImg, nextImg, cn, pts, shp, nextPts, w, maxLevel, cnt, eps, flags, minEigThreshold, return_iters, as_np):
-    """calcOpticalFlowPyrLK on (H,W,C) u8 images, C = 2..4 (cv2 takes 3-channel frames; the reference converts to gray first,
-    s1:311): one single-channel pyramid per channel plane, window sums taken over pixels and channels (ibt_lk_multichannel)."""
-    if cn > 4:
-        raise error("calcOpticalFlowPyrLK: at most 4 channels")
-    a = _to_dev(prevImg, np.uint8, "calcOpticalFlowPyrLK prevImg")
-    b = _to_dev(nextImg, np.uint8, "calcOpticalFlowPyrLK nextImg")
-    if tuple(a.shape) != tuple(b.shape):
-        raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
-    pI = [FramePyramid(a[..., c].contiguous(), w, maxLevel, True) for c in range(cn)]
-    pJ = [FramePyramid(b[..., c].contiguous(), w, maxLevel, False) for c in range(cn)]
-    n = pts.shape[0]
-    if flags & OPTFLOW_USE_INITIAL_FLOW:
-        if nextPts is None:
-            raise error("calcOpticalFlowPyrLK: OPTFLOW_USE_INITIAL_FLOW needs nextPts")
-        nxt = _to_dev(nextPts, np.float32, "calcOpticalFlowPyrLK nextPts").reshape(-1, 2).clone()
-        if nxt.shape[0] != n:
-            raise error("calcOpticalFlowPyrLK: nextPts and prevPts differ in length")
-    else:
-        nxt = torch.empty((n, 2), dtype=torch.float32, device=pts.device)
-    st = torch.empty((n,), dtype=torch.uint8, device=pts.device)
-    err = torch.empty((n,), dtype=torch.float32, device=pts.device)
-    iters = torch.empty((n,), dtype=torch.int32, device=pts.device) if return_iters else None
-    PP = C.POINTER(N.ibt_pyramid_t)
-    arrI = (PP * cn)(*[C.pointer(p.c) for p in pI])
-    arrJ = (PP * cn)(*[C.pointer(p.c) for p in pJ])
-    N.check(N.lib().ibt_lk_multichannel(arrI, arrJ, cn, _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps, float(minEigThreshold),
-                                        flags, _ptr(st), _ptr(err), _ptr(iters), _stream()), "ibt_lk_multichannel")
-    res = (_out(nxt.reshape(shp), as_np), _out(st.reshape(n, 1), as_np), _out(err.reshape(n, 1), as_np))
-    return res + ((_out(iters, as_np),) if return_iters else ())
-
-
 def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, err=None, winSize=(21, 21), maxLevel=3,
                          criteria=(TERM_CRITERIA_COUNT | TERM_CRITERIA_EPS, 30, 0.01), flags=0, minEigThreshold=1e-4,
                          *, return_iters=False):
@@ -320,15 +288,24 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
     cn = _channels(prevImg)
     if cn != _channels(nextImg):
         raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in the number of channels")
-    if cn > 1:
-        return _lk_multichannel(prevImg, nextImg, cn, pts, shp, nextPts, w, maxLevel, cnt, eps, int(flags), minEigThreshold,
-                                return_iters, as_np)
-    pI = _as_pyramid(prevImg, w, maxLevel, True, "calcOpticalFlowPyrLK prevImg")
-    pJ = _as_pyramid(nextImg, w, maxLevel, False, "calcOpticalFlowPyrLK nextImg")
-    if pI.sizes[0] != pJ.sizes[0]:
-        raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
-    if pI.maxLevel != pJ.maxLevel:
-        raise error("calcOpticalFlowPyrLK: pyramids differ in depth")
+    if cn == 1:
+        pI = _as_pyramid(prevImg, w, maxLevel, True, "calcOpticalFlowPyrLK prevImg")
+        pJ = _as_pyramid(nextImg, w, maxLevel, False, "calcOpticalFlowPyrLK nextImg")
+        if pI.sizes[0] != pJ.sizes[0]:
+            raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
+        if pI.maxLevel != pJ.maxLevel:
+            raise error("calcOpticalFlowPyrLK: pyramids differ in depth")
+    else:
+        # (H,W,C) u8 frames, C = 2..4 (cv2 takes 3-channel frames; the reference converts to gray first, s1:311): one
+        # single-channel pyramid per channel plane, window sums taken over pixels and channels
+        if cn > 4:
+            raise error("calcOpticalFlowPyrLK: at most 4 channels")
+        a = _to_dev(prevImg, np.uint8, "calcOpticalFlowPyrLK prevImg")
+        b = _to_dev(nextImg, np.uint8, "calcOpticalFlowPyrLK nextImg")
+        if tuple(a.shape) != tuple(b.shape):
+            raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
+        pI = [FramePyramid(a[..., c].contiguous(), w, maxLevel, True) for c in range(cn)]
+        pJ = [FramePyramid(b[..., c].contiguous(), w, maxLevel, False) for c in range(cn)]
     flags = int(flags)
     if flags & OPTFLOW_USE_INITIAL_FLOW:
         if nextPts is None:
@@ -341,8 +318,15 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
     st = torch.empty((n,), dtype=torch.uint8, device=pts.device)
     err = torch.empty((n,), dtype=torch.float32, device=pts.device)
     iters = torch.empty((n,), dtype=torch.int32, device=pts.device) if return_iters else None
-    N.check(N.lib().ibt_lk(C.byref(pI.c), C.byref(pJ.c), _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps,
-                           float(minEigThreshold), flags, _ptr(st), _ptr(err), _ptr(iters), _stream()), "ibt_lk")
+    if cn == 1:
+        N.check(N.lib().ibt_lk(C.byref(pI.c), C.byref(pJ.c), _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps,
+                               float(minEigThreshold), flags, _ptr(st), _ptr(err), _ptr(iters), _stream()), "ibt_lk")
+    else:
+        PP = C.POINTER(N.ibt_pyramid_t)
+        arrI = (PP * cn)(*[C.pointer(p.c) for p in pI])
+        arrJ = (PP * cn)(*[C.pointer(p.c) for p in pJ])
+        N.check(N.lib().ibt_lk_multichannel(arrI, arrJ, cn, _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps, float(minEigThreshold),
+                                            flags, _ptr(st), _ptr(err), _ptr(iters), _stream()), "ibt_lk_multichannel")
     res = (_out(nxt.reshape(shp), as_np), _out(st.reshape(n, 1), as_np), _out(err.reshape(n, 1), as_np))
     return res + ((_out(iters, as_np),) if return_iters else ())
 

@@ -249,3 +249,44 @@ def test_multichannel_lk_golden(ibt, golden):
     """calcOpticalFlowPyrLK on 3- / 4-channel frames through the C-ABI (ibt_lk_multichannel) vs cv2's recorded answers"""
     import multichannel_cases as MC
     MC.check_multichannel_golden(ibt, golden("kat_multichannel.npz"))
+
+
+@pytest.mark.parametrize("win", [(21, 21), (9, 15)])
+def test_lk_multichannel_one_plane_equals_gray(ibt, win):
+    """ibt_lk_multichannel with one channel plane runs the runtime-cn kernel (cp.async staging); ibt_lk runs the gray kernel
+    (window-specialised at 21 x 21, TMA staging).  Both are the one solver body: on the same pyramids p1, status, err and
+    iters agree bit for bit, for points inside, near and beyond the border, with and without the two flags."""
+    import ctypes as C
+    from iceberg_tracking_code_b200 import _native as N, synthetic as syn
+    h, w = 1080, 1920
+    base = syn.base_texture(h, w, 7)
+    pa = ibt.FramePyramid(syn.frame_gray(base, 0).cuda(), win, 3, True)
+    pb = ibt.FramePyramid(syn.frame_gray(base, 1).cuda(), win, 3, False)
+    rng = np.random.default_rng(7)
+    inside = rng.uniform([40, 40], [w - 40, h - 40], (3000, 2))
+    near = np.concatenate([rng.uniform([-2, 0], [12, h], (300, 2)), rng.uniform([0, h - 12], [w, h + 2], (300, 2))])
+    beyond = np.concatenate([rng.uniform([-60, 0], [-15, h], (100, 2)), rng.uniform([0, h + 15], [w, h + 60], (100, 2))])
+    pts = torch.from_numpy(np.concatenate([inside, near, beyond]).astype(np.float32)).cuda()
+    guess = pts + torch.from_numpy(rng.normal(0, 1.5, tuple(pts.shape)).astype(np.float32)).cuda()
+    n = pts.shape[0]
+    one = C.POINTER(N.ibt_pyramid_t) * 1
+    for flags in (0, ibt.OPTFLOW_USE_INITIAL_FLOW, ibt.OPTFLOW_LK_GET_MIN_EIGENVALS,
+                  ibt.OPTFLOW_USE_INITIAL_FLOW | ibt.OPTFLOW_LK_GET_MIN_EIGENVALS):
+        res = []
+        for mc in (False, True):
+            p1 = guess.clone()
+            st = torch.empty(n, dtype=torch.uint8, device="cuda")
+            err = torch.empty(n, dtype=torch.float32, device="cuda")
+            it = torch.empty(n, dtype=torch.int32, device="cuda")
+            tail = (ibt._ptr(pts), ibt._ptr(p1), n, win[0], win[1], 30, 0.01, 1e-4, flags, ibt._ptr(st), ibt._ptr(err),
+                    ibt._ptr(it), ibt._stream())
+            if mc:
+                rc = N.lib().ibt_lk_multichannel(one(C.pointer(pa.c)), one(C.pointer(pb.c)), 1, *tail)
+            else:
+                rc = N.lib().ibt_lk(C.byref(pa.c), C.byref(pb.c), *tail)
+            assert rc == N.IBT_OK
+            res.append([t.cpu().numpy() for t in (p1, st, err, it)])
+        for name, g, m in zip(("p1", "status", "err", "iters"), *res):
+            assert np.array_equal(g, m), (win, flags, name, int((g != m).sum()))
+        st = res[0][1]
+        assert 0 < st.sum() < n, (win, flags)        # both outcomes occur: the border cases are exercised
