@@ -853,7 +853,9 @@ static int lk_queue_for(int dev, cudaStream_t st, unsigned int **out)
         if (q.dev == dev && q.stream == st) { *out = q.words; return IBT_OK; }
     unsigned int *w = nullptr;
     IBT_CUDA_TRY(cudaMalloc(&w, 2 * sizeof(unsigned int)));
-    IBT_CUDA_TRY(cudaMemset(w, 0, 2 * sizeof(unsigned int)));      // synchronous: visible to every stream afterwards
+    // zeroed on the queue's own stream: a plain cudaMemset goes to the legacy default stream, which a non-blocking stream does
+    // not wait for -- the zeroing could land in the middle of the first launches and leave the queue un-armed
+    IBT_CUDA_TRY(cudaMemsetAsync(w, 0, 2 * sizeof(unsigned int), st));
     lk_queues.push_back({dev, st, w});
     *out = w;
     return IBT_OK;

@@ -141,7 +141,9 @@ size_t ibt_gftt_workspace_bytes(int H, int W);
  * truncated to maxCorners (<= 0: unlimited).  useHarrisDetector / k: cv2's arguments of the same name (the reference leaves
  * them at False / 0.04, s1:240-243): non-zero ranks the Harris response instead of lambda_min.  out_count: HOST int*.
  * SYNCHRONISES `stream` (the corner count decides the shapes the caller allocates next, like cv2's return value).
- * Returns IBT_E_CAPACITY (and the full count) if cap was too small. */
+ * Returns IBT_E_CAPACITY (and the full count) if cap was too small.  It also returns IBT_E_CAPACITY when the raw 3x3 maxima
+ * above the threshold exceed the workspace's candidate capacity, H*W/4 + 4096: isolated maxima never do, only plateaus of
+ * exactly equal responses (e.g. blockSize 31 on a periodic 0/255 checkerboard). */
 int ibt_gftt(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch,
              int H, int W, int maxCorners, double qualityLevel, double minDistance, int blockSize,
              int useHarrisDetector, double k,
