@@ -23,6 +23,8 @@
 //                        all such candidates are REJECTED; rounds repeat until none is undecided) -> ordered compaction
 //                        -> (x, y) float32 of the first maxCorners, count left in device memory.
 //   ibt_min_eigen_f32    (cornerMinEigenVal test hook) keeps the map-writing eig_kernel.
+//   cv2's other Sobel apertures (gradientSize / ksize = -1, 1, 5, 7) take eig_nms_ap_kernel / eig_ap_kernel in place of K2a /
+//   eig_kernel (table and int64 bound at eig_ap_kernel); K2b is the same.
 #include "common.cuh"
 #include <atomic>
 #include <float.h>
@@ -140,6 +142,138 @@ static int launch_eig(const uint8_t *gray, int H, int W, int64_t pitch, int bs, 
 }
 
 // ---------------------------------------------------------------------------------------------
+// The other Sobel apertures of cv2's cornerEigenValsVecs (ksize / gradientSize = -1 (Scharr), 1, 5, 7).  dx correlates the
+// derivative taps d along x and the smoothing taps s along y, dy the transpose; every aperture is written as KT = 3, 5 or 7
+// taps (ksize 1: s = 0 1 0), so the Sobel radius is KT / 2.  OpenCV scales the derivatives by 1 / (sden * blockSize * 255):
+//     g    d                   s                   sden   max |sx| on u8
+//     1    -1 0 1              (0) 1 (0)             1      255
+//     3    -1 0 1              1 2 1                 4      1 020        (eig_kernel / eig_nms_kernel above)
+//    -1    -1 0 1              3 10 3                8      4 080
+//     5    -1 -2 0 2 1         1 4 6 4 1            16      12 240
+//     7    -1 -4 -5 0 5 4 1    1 6 15 20 15 6 1     64      163 200
+// Aperture 3's exact int32 sums do not carry over: a blockSize-31 window sum of sx^2 reaches 1.6e10 (Scharr), 1.4e11 (5) and
+// 2.6e13 (7) (6.2e7 for 1).  These kernels sum the products in int64; every sum stays below 2^53, so the conversion to double
+// before the scaling is exact as well.
+__host__ __device__ constexpr int ap_taps(int g) { return g == 5 ? 5 : g == 7 ? 7 : 3; }
+__host__ __device__ constexpr int ap_d(int g, int j)
+{
+    return g == 5 ? (j == 0 ? -1 : j == 1 ? -2 : j == 2 ? 0 : j == 3 ? 2 : 1)
+         : g == 7 ? (j == 0 ? -1 : j == 1 ? -4 : j == 2 ? -5 : j == 3 ? 0 : j == 4 ? 5 : j == 5 ? 4 : 1)
+         : j - 1;
+}
+__host__ __device__ constexpr int ap_s(int g, int j)
+{
+    return g == 5 ? (j == 0 || j == 4 ? 1 : j == 2 ? 6 : 4)
+         : g == 7 ? (j == 0 || j == 6 ? 1 : j == 1 || j == 5 ? 6 : j == 2 || j == 4 ? 15 : 20)
+         : g == 1 ? (j == 1 ? 1 : 0)
+         : g == -1 ? (j == 1 ? 10 : 3)
+         : (j == 1 ? 2 : 1);
+}
+static bool ap_supported(int g) { return g == -1 || g == 1 || g == 3 || g == 5 || g == 7; }
+static float ap_scale(int g, int bs)                  // OpenCV's Sobel / Scharr scale of cornerEigenValsVecs, rounded to float
+{
+    const double sden = g == -1 ? 8.0 : (double)(1 << (g - 1));
+    return (float)(1.0 / (sden * bs * 255.0));
+}
+
+// eig_kernel for the apertures above: each thread gathers the KT x KT bytes of its support pixel; products, ring and sums in int64
+template <int G>
+__global__ void __launch_bounds__(EW)
+eig_ap_kernel(const uint8_t *__restrict__ img, int H, int W, int64_t pitch, int bs, double s2, int harris, float harris_k,
+              float *__restrict__ eig, int64_t eig_pitch_f)
+{
+    constexpr int KT = ap_taps(G), R = KT / 2;
+    extern __shared__ long long eap_smem[];
+    long long *prod = eap_smem;                      // [2][3][EW]   products of the current support row (double-buffered)
+    long long *ring = eap_smem + 2 * 3 * EW;         // [bs][3][EW]  horizontal window sums of the last bs support rows
+    const int t = threadIdx.x;
+    const int nout = EW - bs + 1;
+    const int a0 = -(bs / 2);
+    const int X0 = blockIdx.x * nout, Y0 = blockIdx.y * ERS;
+    const int x = X0 + t;
+    const bool xout = t < nout && x < W;
+    const int px = r101(X0 + a0 + t, W);             // REFLECT_101 on the product image, then again on the source
+    int cx[KT];
+#pragma unroll
+    for (int j = 0; j < KT; j++) cx[j] = r101(px + j - R, W);
+    long long vs0 = 0, vs1 = 0, vs2 = 0;
+    const int nrows = min(ERS, H - Y0) + bs - 1;
+    int slot = 0;
+    for (int k = 0; k < nrows; k++) {
+        const int py = r101(Y0 + a0 + k, H);
+        int sx = 0, sy = 0;
+#pragma unroll
+        for (int i = 0; i < KT; i++) {
+            const uint8_t *row = img + (int64_t)r101(py + i - R, H) * pitch;
+            int hd = 0, hs = 0;
+#pragma unroll
+            for (int j = 0; j < KT; j++) { const int v = row[cx[j]]; hd += ap_d(G, j) * v; hs += ap_s(G, j) * v; }
+            sx += ap_s(G, i) * hd; sy += ap_d(G, i) * hs;
+        }
+        long long *pb = prod + (k & 1) * 3 * EW;
+        pb[t] = (long long)sx * sx; pb[EW + t] = (long long)sx * sy; pb[2 * EW + t] = (long long)sy * sy;
+        __syncthreads();
+        if (t < nout) {
+            long long h0 = 0, h1 = 0, h2 = 0;
+            for (int j = 0; j < bs; j++) { h0 += pb[t + j]; h1 += pb[EW + t + j]; h2 += pb[2 * EW + t + j]; }
+            long long *rg = ring + slot * 3 * EW;
+            if (k >= bs) { vs0 -= rg[t]; vs1 -= rg[EW + t]; vs2 -= rg[2 * EW + t]; }
+            vs0 += h0; vs1 += h1; vs2 += h2;
+            rg[t] = h0; rg[EW + t] = h1; rg[2 * EW + t] = h2;
+            if (k >= bs - 1 && xout) {
+                const int y = Y0 + k - (bs - 1);
+                float e;
+                if (harris) {                                   // cv2.cornerHarris: (a*c - b*b) - k*((a + c)*(a + c)), float, unfused
+                    const float a = (float)((double)vs0 * s2), b = (float)((double)vs1 * s2), c = (float)((double)vs2 * s2);
+                    const float tr = __fadd_rn(a, c);
+                    e = __fsub_rn(__fsub_rn(__fmul_rn(a, c), __fmul_rn(b, b)), __fmul_rn(harris_k, __fmul_rn(tr, tr)));
+                } else {
+                    const float a = __fmul_rn((float)((double)vs0 * s2), 0.5f), b = (float)((double)vs1 * s2);
+                    const float c = __fmul_rn((float)((double)vs2 * s2), 0.5f);
+                    const float d = __fsub_rn(a, c);
+                    e = __fsub_rn(__fadd_rn(a, c), __fsqrt_rn(__fadd_rn(__fmul_rn(d, d), __fmul_rn(b, b))));
+                }
+                eig[(int64_t)y * eig_pitch_f + x] = e;
+            }
+        }
+        slot = slot + 1 == bs ? 0 : slot + 1;
+    }
+}
+
+static size_t eig_ap_smem_bytes(int bs) { return (size_t)(2 + bs) * 3 * EW * sizeof(long long); }
+
+template <int G>
+static int launch_eig_ap_g(const uint8_t *gray, int H, int W, int64_t pitch, int bs, int harris, double k, float *eig,
+                           int64_t eig_pitch_bytes, cudaStream_t st)
+{
+    if (eig_ap_smem_bytes(bs) > 48 * 1024)
+        IBT_CUDA_TRY(cudaFuncSetAttribute(eig_ap_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)eig_ap_smem_bytes(MAX_BLOCK)));
+    const float scale = ap_scale(G, bs);
+    const double s2 = (double)scale * (double)scale;
+    const int nout = EW - bs + 1;
+    dim3 grid((W + nout - 1) / nout, (H + ERS - 1) / ERS);
+    eig_ap_kernel<G><<<grid, EW, eig_ap_smem_bytes(bs), st>>>(gray, H, W, pitch, bs, s2, harris ? 1 : 0, (float)k, eig, eig_pitch_bytes / 4);
+    return check_launch("eig_ap_kernel");
+}
+
+// the map hooks: aperture 3 keeps eig_kernel
+static int launch_eig_ksize(const uint8_t *gray, int H, int W, int64_t pitch, int bs, int ksize, int harris, double k, float *eig,
+                            int64_t eig_pitch_bytes, cudaStream_t st)
+{
+    if (!ap_supported(ksize)) return IBT_E_INVALID;
+    if (ksize == 3) return launch_eig(gray, H, W, pitch, bs, harris, k, eig, eig_pitch_bytes, nullptr, 0, nullptr, st);
+    if (!gray || !eig || H <= 0 || W <= 0 || bs < 1 || bs > MAX_BLOCK || pitch < W || eig_pitch_bytes % 4 != 0 ||
+        eig_pitch_bytes < (int64_t)W * 4)
+        return IBT_E_INVALID;
+    switch (ksize) {
+    case -1: return launch_eig_ap_g<-1>(gray, H, W, pitch, bs, harris, k, eig, eig_pitch_bytes, st);
+    case 1: return launch_eig_ap_g<1>(gray, H, W, pitch, bs, harris, k, eig, eig_pitch_bytes, st);
+    case 5: return launch_eig_ap_g<5>(gray, H, W, pitch, bs, harris, k, eig, eig_pitch_bytes, st);
+    default: return launch_eig_ap_g<7>(gray, H, W, pitch, bs, harris, k, eig, eig_pitch_bytes, st);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // K2a/K2b fused: response + raw 3x3 maxima, one warp per (column strip, row chunk)
 enum : uint8_t { ST_UNDECIDED = 0, ST_ACCEPTED = 1, ST_REJECTED = 2 };
 
@@ -171,6 +305,7 @@ constexpr int EN_CB = 192;                // per-warp candidate buffer (flushed 
 constexpr int EN_PAD = 32;                // generic blockSize: padding of the shared row buffer on both sides
 constexpr int EN_MIN_CTAS = 5;            // CTAs of 4 warps per SM the register budget is compiled for
 constexpr int EN_BORDER_SPLIT = 4;        // border strips (byte gathers, ~4x slower per row) get 4x shorter jobs
+constexpr int EN_AP_MIN_CTAS = 3;         // eig_nms_ap_kernel: the tap rows and 64-bit sums need more registers
 
 struct EigNmsArgs {
     const uint8_t *img; int H, W; int64_t pitch;
@@ -476,21 +611,282 @@ static int launch_eig_nms_bs(const EigNmsArgs &a, cudaStream_t st)
     return check_launch("eig_nms_kernel");
 }
 
-static int launch_eig_nms(const uint8_t *gray, int H, int W, int64_t pitch, int bs, int harris, double harris_k,
+// ---- K2a for the apertures other than 3 (table at eig_ap_kernel).  eig_nms_job's structure: one warp per (strip, row chunk),
+// four adjacent columns per lane, rows top to bottom, word loads on the inner strips and byte gathers on the border strips;
+// what changes is the front end.  The horizontal taps of an image row reach KT / 2 columns (bytes of the neighbour lanes'
+// words, or gathers), the vertical taps combine the last KT rows of horizontal taps (held in registers), the ring keeps
+// (sx, sy) as two int32 (|sx| reaches 163 200 at aperture 7) and the vertical and horizontal window sums are int64.
+template <int G>
+__device__ __forceinline__ void ap_taps_word(uint32_t w, int *hd, int *hs)
+{
+    constexpr int KT = ap_taps(G), R = KT / 2;
+    const uint32_t L = __shfl_up_sync(0xffffffffu, w, 1), Rt = __shfl_down_sync(0xffffffffu, w, 1);
+    int b[4 + 2 * R];                                             // bytes of columns c0 - R .. c0 + 3 + R
+#pragma unroll
+    for (int i = 0; i < 4 + 2 * R; i++) {
+        const int rel = i - R;
+        b[i] = (int)(((rel < 0 ? L : rel < 4 ? w : Rt) >> (((rel + 4) & 3) * 8)) & 0xffu);
+    }
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        int d = 0, s = 0;
+#pragma unroll
+        for (int j = 0; j < KT; j++) { d += ap_d(G, j) * b[k + j]; s += ap_s(G, j) * b[k + j]; }
+        hd[k] = d; hs[k] = s;
+    }
+}
+
+// hbox_smem on int64 sums
+__device__ __forceinline__ void hbox_smem64(const long long *v, long long *out, long long *rowbuf, int bs, int lane)
+{
+    const int a0 = -(bs / 2);
+    __syncwarp();
+    reinterpret_cast<longlong2 *>(rowbuf + EN_PAD + 4 * lane)[0] = make_longlong2(v[0], v[1]);
+    reinterpret_cast<longlong2 *>(rowbuf + EN_PAD + 4 * lane)[1] = make_longlong2(v[2], v[3]);
+    __syncwarp();
+    const long long *p = rowbuf + EN_PAD + 4 * lane + a0;
+    long long s = 0;
+    for (int j = 0; j < bs; j++) s += p[j];
+    out[0] = s;
+#pragma unroll
+    for (int k = 1; k < 4; k++) { s += p[k - 1 + bs] - p[k - 1]; out[k] = s; }
+}
+
+template <int G, bool MASK, bool BORDER, bool HARRIS>
+__device__ __forceinline__ void eig_nms_ap_job(const EigNmsArgs &a, int strip, int Y0, int Y1, int *wsm, int lane)
+{
+    constexpr int KT = ap_taps(G), R = KT / 2;
+    const int bs = a.bs;
+    const int a0 = -(bs / 2);
+    const int H = a.H, W = a.W;
+    const int ox0 = strip * a.outw;                       // first output column of the strip
+    const int c0 = ox0 - a.left + 4 * lane;               // support column of this lane's pixel 0 (multiple of 4)
+    const int ey0 = max(0, Y0 - 1), ey1 = min(H - 1, Y1);         // response rows needed (NMS halo rows included)
+    int *ring = wsm;                                              // [bs][128][2]: (sx, sy) of the last bs product rows
+    unsigned long long *cbuf = reinterpret_cast<unsigned long long *>(wsm + bs * 2 * EN_COLS);
+    int *scount = reinterpret_cast<int *>(cbuf + EN_CB);          // entries in cbuf (may run past EN_CB: those went straight to global)
+    long long *rowbuf = reinterpret_cast<long long *>(scount + 4);  // [EN_PAD + 128 + EN_PAD]
+    unsigned outmask = 0, candmask = 0;                           // pixels this lane owns / may emit
+    int cx[4][KT];                                                // border strips: source columns of the lane's horizontal taps
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const int c = c0 + k;
+        const bool own = c >= ox0 && c < ox0 + a.outw && c < W;
+        if (own) outmask |= 1u << k;
+        if (own && c >= 1 && c <= W - 2) candmask |= 1u << k;
+        const int pc = r101(c, W);                                // REFLECT_101 on the product image ...
+#pragma unroll
+        for (int j = 0; j < KT; j++) cx[k][j] = BORDER ? r101(pc + j - R, W) : 0;   // ... whose Sobel reflects the source again
+    }
+    if (lane == 0) *scount = 0;
+    __syncwarp();
+    long long vxx[4] = {0, 0, 0, 0}, vxy[4] = {0, 0, 0, 0}, vyy[4] = {0, 0, 0, 0};
+    float m3a[4], m3b[4], eprev[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) { m3a[k] = m3b[k] = -FLT_MAX; eprev[k] = 0.f; }
+    unsigned mprev = 0;                                           // mask bits of the previous response row
+    float lmax = -FLT_MAX;
+    bool have_max = false;
+    float thr_lb = 0.f;
+    {
+        const uint32_t mb = *reinterpret_cast<volatile const uint32_t *>(&a.cnt->maxbits);
+        if (mb) thr_lb = fmaxf(0.f, (float)((double)dec_f32(mb) * a.quality));
+    }
+    auto flush = [&]() {
+        __syncwarp();
+        const int ncb = min(*reinterpret_cast<volatile int *>(scount), EN_CB);
+        unsigned base = 0;
+        if (lane == 0 && ncb) base = atomicAdd(&a.cnt->ncand, (unsigned)ncb);
+        base = __shfl_sync(0xffffffffu, base, 0);
+        for (int i = lane; i < ncb; i += 32)
+            if (base + i < a.cap) a.keys[base + i] = cbuf[i];
+        __syncwarp();
+        if (lane == 0) *scount = 0;
+        __syncwarp();
+    };
+    auto row_taps = [&](const uint8_t *row, int *hd, int *hs) {
+        if (BORDER) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                int d = 0, s = 0;
+#pragma unroll
+                for (int j = 0; j < KT; j++) { const int v = __ldg(row + cx[k][j]); d += ap_d(G, j) * v; s += ap_s(G, j) * v; }
+                hd[k] = d; hs[k] = s;
+            }
+        } else {
+            ap_taps_word<G>(__ldg(reinterpret_cast<const uint32_t *>(row + c0)), hd, hs);
+        }
+    };
+    const int p_first = ey0 + a0, p_last = ey1 + a0 + bs - 1;
+    int slot = 0;
+    int hd[KT][4], hs[KT][4];                             // horizontal taps of the KT image rows under product row p, top to bottom
+    bool have = false;                                    // they hold the unreflected rows p-1-R .. p-1+R
+    for (int p = p_first; p <= p_last; p++) {
+        if (have && p + R <= H - 1) {                     // only row p+R is new
+#pragma unroll
+            for (int i = 0; i + 1 < KT; i++)
+#pragma unroll
+                for (int k = 0; k < 4; k++) { hd[i][k] = hd[i + 1][k]; hs[i][k] = hs[i + 1][k]; }
+            row_taps(a.img + (int64_t)(p + R) * a.pitch, hd[KT - 1], hs[KT - 1]);
+        } else {
+            const int rp = r101(p, H);
+#pragma unroll
+            for (int i = 0; i < KT; i++) row_taps(a.img + (int64_t)r101(rp + i - R, H) * a.pitch, hd[i], hs[i]);
+        }
+        have = p - R >= 0 && p + R <= H - 1;
+        // ---- vertical sliding sums of the products; the ring keeps (sx, sy) of the last bs rows -------------------------
+        int4 *rg = reinterpret_cast<int4 *>(ring + slot * 2 * EN_COLS) + 2 * lane;
+        if (p - p_first >= bs) {
+            const int4 o0 = rg[0], o1 = rg[1];
+            const int ox[4] = {o0.x, o0.z, o1.x, o1.z}, oy[4] = {o0.y, o0.w, o1.y, o1.w};
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                vxx[k] -= (long long)ox[k] * ox[k]; vxy[k] -= (long long)ox[k] * oy[k]; vyy[k] -= (long long)oy[k] * oy[k];
+            }
+        }
+        int sx[4], sy[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            int x = 0, y = 0;
+#pragma unroll
+            for (int i = 0; i < KT; i++) { x += ap_s(G, i) * hd[i][k]; y += ap_d(G, i) * hs[i][k]; }
+            sx[k] = x; sy[k] = y;
+            vxx[k] += (long long)x * x; vxy[k] += (long long)x * y; vyy[k] += (long long)y * y;
+        }
+        rg[0] = make_int4(sx[0], sy[0], sx[1], sy[1]);
+        rg[1] = make_int4(sx[2], sy[2], sx[3], sy[3]);
+        slot = slot + 1 == bs ? 0 : slot + 1;
+        const int y = p - a0 - bs + 1;                    // response row completed by this product row
+        if (y < ey0) continue;
+        // ---- horizontal window sums, response ----------------------------------------------------------------------------
+        long long bxx[4], bxy[4], byy[4];
+        hbox_smem64(vxx, bxx, rowbuf, bs, lane); hbox_smem64(vxy, bxy, rowbuf, bs, lane); hbox_smem64(vyy, byy, rowbuf, bs, lane);
+        float e[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            if (HARRIS) {                                 // cv2.cornerHarris: (a*c - b*b) - k*((a + c)*(a + c)), float, unfused
+                const float fa = (float)((double)bxx[k] * a.s2), fb = (float)((double)bxy[k] * a.s2);
+                const float fc = (float)((double)byy[k] * a.s2);
+                const float tr = __fadd_rn(fa, fc);
+                e[k] = __fsub_rn(__fsub_rn(__fmul_rn(fa, fc), __fmul_rn(fb, fb)), __fmul_rn(a.harris_k, __fmul_rn(tr, tr)));
+            } else {
+                const float fa = (float)((double)bxx[k] * a.s2h), fb = (float)((double)bxy[k] * a.s2);
+                const float fc = (float)((double)byy[k] * a.s2h);
+                const float d = __fsub_rn(fa, fc);
+                e[k] = __fsub_rn(__fadd_rn(fa, fc), __fsqrt_rn(__fadd_rn(__fmul_rn(d, d), __fmul_rn(fb, fb))));
+            }
+        }
+        // ---- masked maximum, 3x3 raw maxima of the previous row, candidate buffer: as eig_nms_job ----------------------------
+        unsigned mcur = 0xfu;
+        if (MASK) {
+            mcur = 0;
+#pragma unroll
+            for (int k = 0; k < 4; k++)
+                if ((outmask >> k) & 1u) mcur |= (a.mask[(int64_t)y * a.mask_pitch + c0 + k] ? 1u : 0u) << k;
+        }
+        if (y >= Y0 && y < Y1) {
+#pragma unroll
+            for (int k = 0; k < 4; k++)
+                if (((outmask & mcur) >> k) & 1u) { lmax = fmaxf(lmax, e[k]); have_max = true; }
+        }
+        const float el = __shfl_up_sync(0xffffffffu, e[3], 1), er = __shfl_down_sync(0xffffffffu, e[0], 1);
+        float m3c[4];
+        m3c[0] = fmaxf(fmaxf(el, e[0]), e[1]); m3c[1] = fmaxf(fmaxf(e[0], e[1]), e[2]);
+        m3c[2] = fmaxf(fmaxf(e[1], e[2]), e[3]); m3c[3] = fmaxf(fmaxf(e[2], e[3]), er);
+        const int yc = y - 1;
+        if (yc >= max(Y0, 1) && yc < Y1 && yc <= H - 2) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                const float v = eprev[k];
+                if ((((candmask & mprev) >> k) & 1u) && v > thr_lb && v == fmaxf(fmaxf(m3a[k], m3b[k]), m3c[k])) {
+                    const unsigned long long key = ((unsigned long long)enc_f32(v) << 32) | (uint32_t)(yc * W + c0 + k);
+                    const int pos = atomicAdd(scount, 1);
+                    if (pos < EN_CB) cbuf[pos] = key;
+                    else {
+                        const unsigned g = atomicAdd(&a.cnt->ncand, 1u);
+                        if (g < a.cap) a.keys[g] = key;
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) { m3a[k] = m3b[k]; m3b[k] = m3c[k]; eprev[k] = e[k]; }
+        mprev = mcur;
+        if ((y & 7) == 7) {
+            __syncwarp();
+            if (*reinterpret_cast<volatile int *>(scount) >= EN_CB / 2) flush();
+            if ((y & 31) == 31) {
+                float wm = lmax;
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) wm = fmaxf(wm, __shfl_xor_sync(0xffffffffu, wm, o));
+                if (wm > 0.f) thr_lb = fmaxf(thr_lb, (float)((double)wm * a.quality));
+            }
+        }
+    }
+    flush();
+    uint32_t lbits = have_max ? enc_f32(lmax) : 0u;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lbits = max(lbits, __shfl_xor_sync(0xffffffffu, lbits, o));
+    if (lane == 0 && lbits) atomicMax(&a.cnt->maxbits, lbits);
+}
+
+template <int G, bool MASK, bool HARRIS>
+__global__ void __launch_bounds__(EN_WARPS * 32, EN_AP_MIN_CTAS)
+eig_nms_ap_kernel(const __grid_constant__ EigNmsArgs a)
+{
+    extern __shared__ __align__(16) int en_smem[];
+    pdl_launch_dependents();
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int job = blockIdx.x * EN_WARPS + wib;
+    if (job >= a.njobs) return;
+    int *wsm = en_smem + (size_t)wib * a.warp_smem_ints;
+    const int nbj = a.nborder * a.chunks_border;                  // job split of eig_nms_kernel
+    if (job < nbj) {
+        const int sb = job % a.nborder, chunk = job / a.nborder;
+        const int strip = a.nborder == a.nstrips ? sb : (sb == 0 ? 0 : a.first_right + sb - 1);
+        const int Y0 = chunk * a.rows_border;
+        eig_nms_ap_job<G, MASK, true, HARRIS>(a, strip, Y0, min(a.H, Y0 + a.rows_border), wsm, lane);
+    } else {
+        const int j = job - nbj, nfast = a.nstrips - a.nborder;
+        const int strip = 1 + j % nfast, chunk = j / nfast;
+        const int Y0 = chunk * a.rows_fast;
+        eig_nms_ap_job<G, MASK, false, HARRIS>(a, strip, Y0, min(a.H, Y0 + a.rows_fast), wsm, lane);
+    }
+}
+
+template <int G, bool MASK, bool HARRIS>
+static int launch_eig_nms_ap_kernel(const EigNmsArgs &a, size_t smem, int blocks, cudaStream_t st)
+{
+    if (smem > 48 * 1024) IBT_CUDA_TRY(cudaFuncSetAttribute(eig_nms_ap_kernel<G, MASK, HARRIS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    eig_nms_ap_kernel<G, MASK, HARRIS><<<blocks, EN_WARPS * 32, smem, st>>>(a);
+    return check_launch("eig_nms_ap_kernel");
+}
+
+template <int G>
+static int launch_eig_nms_ap(const EigNmsArgs &a, int harris, cudaStream_t st)
+{
+    const size_t smem = (size_t)a.warp_smem_ints * 4 * EN_WARPS;
+    const int blocks = (a.njobs + EN_WARPS - 1) / EN_WARPS;
+    if (a.mask) return harris ? launch_eig_nms_ap_kernel<G, true, true>(a, smem, blocks, st) : launch_eig_nms_ap_kernel<G, true, false>(a, smem, blocks, st);
+    return harris ? launch_eig_nms_ap_kernel<G, false, true>(a, smem, blocks, st) : launch_eig_nms_ap_kernel<G, false, false>(a, smem, blocks, st);
+}
+
+static int launch_eig_nms(const uint8_t *gray, int H, int W, int64_t pitch, int bs, int ksize, int harris, double harris_k,
                           const uint8_t *mask, int64_t mask_pitch, double quality, GfttCounters *cnt, unsigned long long *keys, uint32_t cap, cudaStream_t st)
 {
-    if (bs < 1 || bs > MAX_BLOCK) return IBT_E_INVALID;
+    if (bs < 1 || bs > MAX_BLOCK || !ap_supported(ksize)) return IBT_E_INVALID;
     EigNmsArgs a;
     a.img = gray; a.H = H; a.W = W; a.pitch = pitch; a.mask = mask; a.mask_pitch = mask_pitch; a.bs = bs;
-    const float scale = (float)(1.0 / (4.0 * bs * 255.0));       // OpenCV's Sobel scale for ksize 3 (SURVEY A.6 step 1)
+    const float scale = ap_scale(ksize, bs);                      // OpenCV's Sobel scale (SURVEY A.6 step 1)
     a.s2 = (double)scale * (double)scale; a.s2h = a.s2 * 0.5;     // the halving of a and c folded in (exact: power of two)
     a.quality = quality; a.cnt = cnt; a.keys = keys; a.cap = cap;
     a.harris_k = (float)harris_k;
-    // strip geometry: lane 0's first column is `left` columns before the strip (Sobel edge + window reach + NMS halo, rounded
+    // strip geometry: lane 0's first column is `left` columns before the strip (Sobel radius + window reach + NMS halo, rounded
     // to words); a warp owns `outw` of its 128 support columns
     const int half = bs / 2;                                      // window offsets [-half, bs - 1 - half]
-    a.left = (2 + half + 3) & ~3;
-    a.outw = (126 - a.left - (bs - 1 - half)) & ~3;
+    const int srad = ap_taps(ksize) / 2;                          // Sobel radius
+    a.left = (srad + 1 + half + 3) & ~3;
+    a.outw = (128 - srad - 1 - a.left - (bs - 1 - half)) & ~3;
     a.nstrips = (W + a.outw - 1) / a.outw;
     a.word_ok = (reinterpret_cast<uintptr_t>(gray) % 4 == 0) && (pitch % 4 == 0);
     // strips whose 128 support columns are all real pixels take the word-load path: 1 <= strip < first_right
@@ -499,11 +895,14 @@ static int launch_eig_nms(const uint8_t *gray, int H, int W, int64_t pitch, int 
     if (!a.word_ok || first_right <= 1) { a.nborder = a.nstrips; first_right = a.nstrips; }
     else a.nborder = 1 + (a.nstrips - first_right);
     a.first_right = first_right;
-    a.warp_smem_ints = bs * EN_COLS + EN_CB * 2 + 4 + (EN_PAD + EN_COLS + EN_PAD);
+    // eig_nms_ap_kernel: (sx, sy) as two ints per ring entry, int64 row buffer
+    a.warp_smem_ints = ksize == 3 ? bs * EN_COLS + EN_CB * 2 + 4 + (EN_PAD + EN_COLS + EN_PAD)
+                                  : bs * 2 * EN_COLS + EN_CB * 2 + 4 + 2 * (EN_PAD + EN_COLS + EN_PAD);
     // rows per job: one wave of warps over the GPU (warm-up costs bs + 2 rows per job), at least 32 rows (8 for border strips)
     int wps = (int)((227 * 1024) / ((size_t)a.warp_smem_ints * 4 * EN_WARPS + 1024)) * EN_WARPS;       // resident warps per SM
     if (wps < 1) wps = 1;
-    if (wps > EN_MIN_CTAS * EN_WARPS) wps = EN_MIN_CTAS * EN_WARPS;   // register budget (launch bounds)
+    const int min_ctas = ksize == 3 ? EN_MIN_CTAS : EN_AP_MIN_CTAS;
+    if (wps > min_ctas * EN_WARPS) wps = min_ctas * EN_WARPS;     // register budget (launch bounds)
     const int nfast = a.nstrips - a.nborder;
     const int weight = nfast + EN_BORDER_SPLIT * a.nborder;       // jobs per row chunk, border strips count EN_BORDER_SPLIT times
     int chunks = (kNumSMs * wps) / weight;
@@ -517,6 +916,13 @@ static int launch_eig_nms(const uint8_t *gray, int H, int W, int64_t pitch, int 
     a.njobs = a.nborder * a.chunks_border + nfast * ((H + rows - 1) / rows);
     // cv2's useHarrisDetector=True (never set by the reference): the response formula changes, nothing else; it takes the
     // runtime-blockSize instantiation whatever the block size
+    switch (ksize) {
+    case -1: return launch_eig_nms_ap<-1>(a, harris, st);
+    case 1: return launch_eig_nms_ap<1>(a, harris, st);
+    case 5: return launch_eig_nms_ap<5>(a, harris, st);
+    case 7: return launch_eig_nms_ap<7>(a, harris, st);
+    default: break;
+    }
     if (harris) return launch_eig_nms_bs<0, true>(a, st);
     if (bs == 10) return launch_eig_nms_bs<10>(a, st);
     if (bs == 3) return launch_eig_nms_bs<3>(a, st);
@@ -1016,12 +1422,12 @@ static GfttLayout gftt_layout(int H, int W)
 
 // Both launches of goodFeaturesToTrack on `st`; nothing is read back.  count_dev (device int) receives the corner count.
 static int gftt_enqueue(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
-                        int maxCorners, double qualityLevel, double minDistance, int blockSize, int useHarris, double harris_k,
+                        int maxCorners, double qualityLevel, double minDistance, int blockSize, int ksize, int useHarris, double harris_k,
                         void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *count_dev, cudaStream_t st)
 {
     if (!gray || !workspace || H < 3 || W < 3 || H > 65535 || W > 65535 || (int64_t)H * W > 0x7fffffffLL ||
         cap < 0 || (cap > 0 && !out_xy) || (mask && mask_pitch < W) || qualityLevel < 0 || minDistance < 0 || minDistance > 1024 ||
-        pitch < W || !(harris_k == harris_k))
+        pitch < W || !(harris_k == harris_k) || !ap_supported(ksize))
         return IBT_E_INVALID;
     const GfttLayout L = gftt_layout(H, W);
     if (workspace_bytes < L.total) return IBT_E_WORKSPACE;
@@ -1029,7 +1435,7 @@ static int gftt_enqueue(const uint8_t *gray, int64_t pitch, const uint8_t *mask,
     GfttCounters *cnt = reinterpret_cast<GfttCounters *>(ws + L.off_cnt);
     IBT_CUDA_TRY(cudaMemsetAsync(cnt, 0, sizeof(GfttCounters), st));
     unsigned long long *keys0 = reinterpret_cast<unsigned long long *>(ws + L.off_keys0);
-    int rc = launch_eig_nms(gray, H, W, pitch, blockSize, useHarris, harris_k, mask, mask_pitch, qualityLevel, cnt, keys0, L.cap, st);
+    int rc = launch_eig_nms(gray, H, W, pitch, blockSize, ksize, useHarris, harris_k, mask, mask_pitch, qualityLevel, cnt, keys0, L.cap, st);
     if (rc) return rc;
     SelArgs a;
     a.cnt = cnt; a.keys0 = keys0;
@@ -1081,11 +1487,24 @@ IBT_API int ibt_min_eigen_f32(const uint8_t *gray, int H, int W, int64_t pitch, 
     return ibt::launch_eig(gray, H, W, pitch, blockSize, 0, 0.0, eig, eig_pitch, nullptr, 0, nullptr, static_cast<cudaStream_t>(stream));
 }
 
+IBT_API int ibt_min_eigen_ksize_f32(const uint8_t *gray, int H, int W, int64_t pitch, int blockSize, int ksize, float *eig,
+                                    int64_t eig_pitch, void *stream)
+{
+    return ibt::launch_eig_ksize(gray, H, W, pitch, blockSize, ksize, 0, 0.0, eig, eig_pitch, static_cast<cudaStream_t>(stream));
+}
+
 IBT_API int ibt_corner_harris_f32(const uint8_t *gray, int H, int W, int64_t pitch, int blockSize, double k, float *dst,
                                   int64_t dst_pitch, void *stream)
 {
     if (!(k == k)) return IBT_E_INVALID;
     return ibt::launch_eig(gray, H, W, pitch, blockSize, 1, k, dst, dst_pitch, nullptr, 0, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+IBT_API int ibt_corner_harris_ksize_f32(const uint8_t *gray, int H, int W, int64_t pitch, int blockSize, int ksize, double k,
+                                        float *dst, int64_t dst_pitch, void *stream)
+{
+    if (!(k == k)) return IBT_E_INVALID;
+    return ibt::launch_eig_ksize(gray, H, W, pitch, blockSize, ksize, 1, k, dst, dst_pitch, static_cast<cudaStream_t>(stream));
 }
 
 IBT_API size_t ibt_gftt_workspace_bytes(int H, int W)
@@ -1094,26 +1513,36 @@ IBT_API size_t ibt_gftt_workspace_bytes(int H, int W)
     return ibt::gftt_layout(H, W).total;
 }
 
+IBT_API int ibt_gftt_async_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
+                                 int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                                 int useHarrisDetector, double k, void *workspace, size_t workspace_bytes, float *out_xy, int cap,
+                                 int *count_dev, void *stream)
+{
+    if (!count_dev) return IBT_E_INVALID;
+    return ibt::gftt_enqueue(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, gradientSize,
+                             useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, count_dev,
+                             static_cast<cudaStream_t>(stream));
+}
+
 IBT_API int ibt_gftt_async(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
                            int maxCorners, double qualityLevel, double minDistance, int blockSize, int useHarrisDetector,
                            double k, void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *count_dev,
                            void *stream)
 {
-    if (!count_dev) return IBT_E_INVALID;
-    return ibt::gftt_enqueue(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize,
-                             useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, count_dev,
-                             static_cast<cudaStream_t>(stream));
+    return ibt_gftt_async_ksize(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, 3,
+                                useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, count_dev, stream);
 }
 
-IBT_API int ibt_gftt(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
-                     int maxCorners, double qualityLevel, double minDistance, int blockSize, int useHarrisDetector, double k,
-                     void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *out_count, void *stream)
+IBT_API int ibt_gftt_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
+                           int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                           int useHarrisDetector, double k, void *workspace, size_t workspace_bytes, float *out_xy, int cap,
+                           int *out_count, void *stream)
 {
     using namespace ibt;
     if (!out_count) return IBT_E_INVALID;
     *out_count = 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int rc = gftt_enqueue(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize,
+    int rc = gftt_enqueue(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, gradientSize,
                           useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, nullptr, st);
     if (rc) return rc;
     // the one host round trip of the synchronous form: the corner count decides the shapes the caller allocates next
@@ -1124,4 +1553,12 @@ IBT_API int ibt_gftt(const uint8_t *gray, int64_t pitch, const uint8_t *mask, in
     IBT_CUDA_TRY(cudaStreamSynchronize(st));
     *out_count = (int)hc->nout;
     return hc->error ? hc->error : IBT_OK;
+}
+
+IBT_API int ibt_gftt(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
+                     int maxCorners, double qualityLevel, double minDistance, int blockSize, int useHarrisDetector, double k,
+                     void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *out_count, void *stream)
+{
+    return ibt_gftt_ksize(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, 3,
+                          useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, out_count, stream);
 }

@@ -392,34 +392,44 @@ def lk_fb_into(prev, next, p0, lk_params, p1, fbdist, alive=None, iter_total=Non
 
 
 # ---------------------------------------------------------------------------------------------------
+APERTURES = (-1, 1, 3, 5, 7)      # cv2's Sobel apertures of the corner detector: -1 = Scharr
+
+
+def _aperture(ksize, what, name):
+    """cv2's ksize / gradientSize -> int; cv2 also takes odd values up to 31 but documents only these"""
+    if isinstance(ksize, bool) or int(ksize) != ksize or int(ksize) not in APERTURES:
+        raise error("%s: %s must be one of -1 (Scharr), 1, 3, 5, 7 (got %r)" % (what, name, ksize))
+    return int(ksize)
+
+
 def cornerMinEigenVal(src, blockSize, dst=None, ksize=3):
     """cv2.cornerMinEigenVal(src, blockSize[, dst[, ksize]]): u8 (H,W) -> (H,W) f32 (SURVEY A.6 steps 1-3); dst is cv2's output
-    placeholder (the map is returned)."""
-    if ksize != 3:
-        raise error("cornerMinEigenVal: only ksize=3 is implemented (the value goodFeaturesToTrack uses)")
+    placeholder (the map is returned).  ksize: Sobel aperture -1 (Scharr), 1, 3, 5 or 7."""
+    ksize = _aperture(ksize, "cornerMinEigenVal", "ksize")
     as_np = _is_np(src)
     s = _to_dev(src, np.uint8, "cornerMinEigenVal src")
     if s.ndim != 2:
         raise error("cornerMinEigenVal: expected a single-channel (H,W) u8 image")
     H, W = s.shape
     eig = torch.empty((H, W), dtype=torch.float32, device=s.device)
-    N.check(N.lib().ibt_min_eigen_f32(_ptr(s), H, W, W, int(blockSize), _ptr(eig), W * 4, _stream()), "ibt_min_eigen_f32")
+    N.check(N.lib().ibt_min_eigen_ksize_f32(_ptr(s), H, W, W, int(blockSize), ksize, _ptr(eig), W * 4, _stream()),
+            "ibt_min_eigen_ksize_f32")
     return _out(eig, as_np)
 
 
 def cornerHarris(src, blockSize, ksize=3, k=0.04):
-    """cv2.cornerHarris(u8 (H,W), blockSize, 3, k) -> (H,W) f32: the response goodFeaturesToTrack(useHarrisDetector=True)
-    ranks.  The reference leaves useHarrisDetector at False (s1:240-243); cv2's signature carries it (SURVEY 8b)."""
-    if ksize != 3:
-        raise error("cornerHarris: only ksize=3 is implemented (the value goodFeaturesToTrack uses)")
+    """cv2.cornerHarris(u8 (H,W), blockSize, ksize, k) -> (H,W) f32: the response goodFeaturesToTrack(useHarrisDetector=True)
+    ranks.  The reference leaves useHarrisDetector at False (s1:240-243); cv2's signature carries it (SURVEY 8b).
+    ksize: Sobel aperture -1 (Scharr), 1, 3, 5 or 7."""
+    ksize = _aperture(ksize, "cornerHarris", "ksize")
     as_np = _is_np(src)
     s = _to_dev(src, np.uint8, "cornerHarris src")
     if s.ndim != 2:
         raise error("cornerHarris: expected a single-channel (H,W) u8 image")
     H, W = s.shape
     dst = torch.empty((H, W), dtype=torch.float32, device=s.device)
-    N.check(N.lib().ibt_corner_harris_f32(_ptr(s), H, W, W, int(blockSize), float(k), _ptr(dst), W * 4, _stream()),
-            "ibt_corner_harris_f32")
+    N.check(N.lib().ibt_corner_harris_ksize_f32(_ptr(s), H, W, W, int(blockSize), ksize, float(k), _ptr(dst), W * 4,
+                                                _stream()), "ibt_corner_harris_ksize_f32")
     return _out(dst, as_np)
 
 
@@ -445,14 +455,14 @@ def goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, corners=No
                         useHarrisDetector=False, k=0.04, gradientSize=3):
     """cv2.goodFeaturesToTrack(frame_gray, mask=mask, **feature_params) (s1:437; SURVEY A.6), positional order of cv2's
     goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance[, corners[, mask[, blockSize[, useHarrisDetector[, k]]]]])
-    (corners is cv2's output placeholder; gradientSize, of cv2's second overload, must be 3 = the Sobel aperture of the first).
+    (corners is cv2's output placeholder; gradientSize, of cv2's second overload, is the Sobel aperture: -1 (Scharr), 1, 3 (the
+    first overload's and the reference's), 5 or 7).
     Returns (K,1,2) float32 integer-valued (x, y) ordered by response, or None when there is no corner
-    (callers test `if p is not None`, s1:445).  useHarrisDetector=True ranks cv2.cornerHarris(image, blockSize, 3, k)
+    (callers test `if p is not None`, s1:445).  useHarrisDetector=True ranks cv2.cornerHarris(image, blockSize, gradientSize, k)
     instead of the minimal eigenvalue (the reference never sets it)."""
     if not (qualityLevel > 0) or minDistance < 0:
         raise error("goodFeaturesToTrack: qualityLevel must be > 0 and minDistance >= 0")
-    if gradientSize != 3:
-        raise error("goodFeaturesToTrack: only gradientSize=3 is implemented (cv2's default; the reference never sets it)")
+    gradientSize = _aperture(gradientSize, "goodFeaturesToTrack", "gradientSize")
     as_np = _is_np(image)
     img = _to_dev(image, np.uint8, "goodFeaturesToTrack image")
     if img.ndim != 2:
@@ -467,10 +477,10 @@ def goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, corners=No
         return None
     ws, out = _gftt_workspace(img.device, H, W)
     cnt = C.c_int(0)
-    rc = N.lib().ibt_gftt(_ptr(img), W, _ptr(m), W, H, W, int(maxCorners), float(qualityLevel), float(minDistance),
-                          int(blockSize), 1 if useHarrisDetector else 0, float(k), _ptr(ws), ws.numel(), _ptr(out), out.shape[0],
-                          C.byref(cnt), _stream())
-    N.check(rc, "ibt_gftt")
+    rc = N.lib().ibt_gftt_ksize(_ptr(img), W, _ptr(m), W, H, W, int(maxCorners), float(qualityLevel), float(minDistance),
+                                int(blockSize), gradientSize, 1 if useHarrisDetector else 0, float(k), _ptr(ws), ws.numel(),
+                                _ptr(out), out.shape[0], C.byref(cnt), _stream())
+    N.check(rc, "ibt_gftt_ksize")
     if cnt.value == 0:
         return None
     return _out(out[:cnt.value].reshape(-1, 1, 2).clone(), as_np)

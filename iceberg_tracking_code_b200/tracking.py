@@ -266,6 +266,7 @@ class SequenceTracker:
         q, md, bs = float(fp["qualityLevel"]), float(fp["minDistance"]), int(fp.get("blockSize", 3))
         if not (q > 0) or md < 0:
             raise cv.error("goodFeaturesToTrack: qualityLevel must be > 0 and minDistance >= 0")
+        gsize = cv._aperture(fp.get("gradientSize", 3), "goodFeaturesToTrack", "gradientSize")
         img = pyr.levels[0]
         H, W = img.shape
         if H < 3 or W < 3:
@@ -285,9 +286,9 @@ class SequenceTracker:
         out = torch.empty((cap, 2), dtype=torch.float32, device=self.device)
         cnt = torch.zeros((1,), dtype=torch.int32, device=self.device)
         p = cv._ptr
-        N.check(N.lib().ibt_gftt_async(p(img), img.stride(0), p(m), W, H, W, maxc, q, md, bs, harris, hk, p(self._ws),
-                                       self._ws.numel(),
-                                       p(out), cap, p(cnt), cv._stream()), "ibt_gftt_async")
+        N.check(N.lib().ibt_gftt_async_ksize(p(img), img.stride(0), p(m), W, H, W, maxc, q, md, bs, gsize, harris, hk,
+                                             p(self._ws), self._ws.numel(), p(out), cap, p(cnt), cv._stream()),
+                "ibt_gftt_async_ksize")
         # (nout, error) of the workspace counters (GfttCounters: maxbits, ncand, nsel, nacc, nout, error): a capacity overflow
         # raised on the device must not pass as "no corners"
         h = self._pin((2,), torch.int32)
@@ -304,7 +305,7 @@ class SequenceTracker:
             ev.synchronize()                              # (issued a frame ago: normally long finished)
             n, err = int(h[0]), int(h[1])
             self._unpin(h)
-            N.check(err, "ibt_gftt_async")
+            N.check(err, "ibt_gftt_async_ksize")
             torch.cuda.current_stream().wait_event(ev)
             out.record_stream(torch.cuda.current_stream())
             p = out[:n] if n else None

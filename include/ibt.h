@@ -134,6 +134,22 @@ int ibt_min_eigen_f32(const uint8_t *gray, int H, int W, int64_t pitch, int bloc
                       float *eig, int64_t eig_pitch, void *stream);
 int ibt_corner_harris_f32(const uint8_t *gray, int H, int W, int64_t pitch, int blockSize, double k,
                           float *dst, int64_t dst_pitch, void *stream);
+/* The same maps for cv2's other Sobel apertures: ksize (cv2's ksize / gradientSize) is -1 (Scharr), 1, 3, 5 or 7; anything else
+ * returns IBT_E_INVALID before any CUDA call.  ksize 3 is exactly ibt_min_eigen_f32 / ibt_corner_harris_f32.  As in OpenCV's
+ * cornerEigenValsVecs, dx correlates the derivative taps d along x and the smoothing taps s along y (dy the transpose), and
+ * the derivatives are scaled by 1 / (sden * blockSize * 255):
+ *     ksize   d                   s                   sden   max |dx| before scaling, u8 input
+ *       1     -1 0 1              1                     1      255
+ *       3     -1 0 1              1 2 1                 4      1 020
+ *      -1     -1 0 1              3 10 3 (Scharr)       8      4 080
+ *       5     -1 -2 0 2 1         1 4 6 4 1            16      12 240
+ *       7     -1 -4 -5 0 5 4 1    1 6 15 20 15 6 1     64      163 200
+ * The window sums of the exact integer products reach 1.6e10 (Scharr), 1.4e11 (5) and 2.6e13 (7) at blockSize 31, beyond
+ * int32: apertures other than 3 sum them in int64, exact (every sum is below 2^53). */
+int ibt_min_eigen_ksize_f32(const uint8_t *gray, int H, int W, int64_t pitch, int blockSize, int ksize,
+                            float *eig, int64_t eig_pitch, void *stream);
+int ibt_corner_harris_ksize_f32(const uint8_t *gray, int H, int W, int64_t pitch, int blockSize, int ksize, double k,
+                                float *dst, int64_t dst_pitch, void *stream);
 
 size_t ibt_gftt_workspace_bytes(int H, int W);
 /* mask may be NULL (all allowed).  out_xy (cap,2) f32 receives integer-valued x,y ordered by
@@ -157,6 +173,18 @@ int ibt_gftt_async(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int6
                    int useHarrisDetector, double k,
                    void *workspace, size_t workspace_bytes,
                    float *out_xy, int cap, int *count_dev, void *stream);
+/* ibt_gftt / ibt_gftt_async with cv2's gradientSize: the Sobel aperture of the response (-1, 1, 3, 5 or 7, as
+ * ibt_min_eigen_ksize_f32; anything else returns IBT_E_INVALID before any CUDA call).  The plain forms are gradientSize 3. */
+int ibt_gftt_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch,
+                   int H, int W, int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                   int useHarrisDetector, double k,
+                   void *workspace, size_t workspace_bytes,
+                   float *out_xy, int cap, int *out_count, void *stream);
+int ibt_gftt_async_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch,
+                         int H, int W, int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                         int useHarrisDetector, double k,
+                         void *workspace, size_t workspace_bytes,
+                         float *out_xy, int cap, int *count_dev, void *stream);
 
 /* ---- track bookkeeping at a group boundary (s1:362-395): stable compaction of the live
  * tracks.  tracks_tm (T+1, N, 2) f32 time-major, quality_tm (T, N) f32, alive (N) u8 ->

@@ -1,14 +1,47 @@
-"""Profiling helper: one 24 MP goodFeaturesToTrack call (config-2 parameters) after a warm-up call."""
+"""Profiling helper: one 24 MP goodFeaturesToTrack call (config-2 parameters) after a warm-up call.
+
+    python tools/prof_gftt.py [maxCorners] [--ksize G ...]
+
+With --ksize, times the call for each Sobel aperture G (cv2's gradientSize: -1 = Scharr, 1, 3, 5, 7) with CUDA events after
+warm-up and prints the card name and power limit beside the times."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from iceberg_tracking_code_b200 import cv, synthetic as syn
 
+args = sys.argv[1:]
+ksizes = []
+if "--ksize" in args:
+    i = args.index("--ksize")
+    ksizes = [int(v) for v in args[i + 1:]]
+    args = args[:i]
 H, W = 4000, 6000
 base = syn.base_texture(H, W, 7, device="cuda")
 g = syn.frame_gray(base, 0)
 del base
-maxc = int(sys.argv[1]) if len(sys.argv) > 1 else 20000
+maxc = int(args[0]) if args else 20000
+
+if ksizes:
+    import subprocess
+    try:
+        card = subprocess.check_output(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], text=True)
+        print("card:", card.strip().splitlines()[torch.cuda.current_device()])
+    except Exception as e:                                  # noqa: BLE001
+        print("card:", torch.cuda.get_device_name(), "(power limit unreadable: %s)" % e)
+    for ks in ksizes:
+        gp = dict(maxCorners=maxc, qualityLevel=0.007, minDistance=10, blockSize=10, gradientSize=ks)
+        for _ in range(3):
+            cv.goodFeaturesToTrack(g, **gp)
+        reps, ts = 20, []
+        for _ in range(reps):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record(); p = cv.goodFeaturesToTrack(g, **gp); e1.record(); e1.synchronize()
+            ts.append(e0.elapsed_time(e1))
+        ts.sort()
+        print("gradientSize %2d: median %.3f ms  min %.3f ms  (%d calls)  corners %s" % (ks, ts[reps // 2], ts[0], reps,
+                                                                                       None if p is None else p.shape[0]))
+    sys.exit(0)
+
 for it in range(3):
     torch.cuda.synchronize(); t0 = time.perf_counter()
     p = cv.goodFeaturesToTrack(g, maxCorners=maxc, qualityLevel=0.007, minDistance=10, blockSize=10)
@@ -24,5 +57,3 @@ prev = ts[0]
 for i in range(1, 11):
     if ts[i] >= ts[0] and ts[i] > 0:
         print("  %-10s +%6.1f us (at %6.1f)" % (names[i], (ts[i] - prev) / 1e3, (ts[i] - ts[0]) / 1e3)); prev = ts[i]
-
-
