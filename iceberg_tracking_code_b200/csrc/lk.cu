@@ -10,15 +10,16 @@
 //      2*MARGIN px).  Intensity patches that overhang the image are mirrored (REFLECT_101) inside shared memory after the
 //      zero-filling copy; cp.async / gather paths remain for far-out windows and images that are not 16-byte aligned;
 //  (b) builds the template: lane = window column, rows walked top to bottom.  Per window pixel the slab keeps only the
-//      packed int16 pair (Ix, Iy) -- 4 bytes -- and the pass accumulates, exactly, the structure tensor and the two
-//      constants C1 = sum(Iw*Ix), C2 = sum(Iw*Iy).  The template rows overwrite the Scharr patch rows already consumed;
+//      int16 pair (Ix, Iy) -- 4 bytes, Ix and Iy of 4 columns grouped (tmpl_store) -- and the pass accumulates, exactly,
+//      the structure tensor and the two constants C1 = sum(Iw*Ix), C2 = sum(Iw*Iy).  The template rows overwrite the
+//      Scharr patch rows already consumed;
 //  (c) runs the Newton iterations out of shared memory with a different lane mapping: lane = (row group, column quad),
 //      4 adjacent columns x RG consecutive rows.  Per row a lane loads the two aligned words that hold its 5 J bytes,
 //      two PRMTs (warp-uniform selectors) turn them into the byte windows (b0..b3), (b1..b4), and dp2a.lo / dp2a.hi on
 //      those against OpenCV's packed 14-bit weights give the four bilinear samples; one 16-byte load brings the four
-//      template entries.  The mismatch vector is  b = sum(Jw*Ix) - C1  (sum(Jw*Iy) - C2): identical, as an exact
-//      integer, to OpenCV's sum((Jw - Iw)*Ix), and it halves the template.  Template entries outside the window are
-//      zero, so the iteration loop carries no masks.
+//      template entries, and the products with them run on dp2a as well (samples split into bytes).  The mismatch vector
+//      is  b = sum(Jw*Ix) - C1  (sum(Jw*Iy) - C2): identical, as an exact integer, to OpenCV's sum((Jw - Iw)*Ix), and it
+//      halves the template.  Template entries outside the window are zero, so the iteration loop carries no masks.
 // Multi-channel frames (cv2 takes 3- and 4-channel images) run the same solver with every window sum taken over the channel
 // planes as well, on the runtime-window kernel without tensor maps.
 // All sums are exact integers (int32 per lane, REDUX across the warp, int64 totals) rounded to float once; OpenCV
@@ -286,8 +287,19 @@ __device__ __forceinline__ void stage_deriv(const LKLevel &L, const LKArgs &a, i
 }
 
 // ---- template --------------------------------------------------------------------------------------------
-// lane = template column (strips of <= 32 columns), rows top to bottom.  Writes tmpl[row][col] = (Ix << 16) | (Iy & 0xffff)
-// for the TROWS x TCOLS template (zero outside the window) and returns the exact sums
+// Template layout: a row is TCOLS int16 pairs (4 * TCOLS bytes), in quads of 4 columns.  A quad's 16 bytes hold
+// Ix0 Ix1 Ix2 Ix3 Iy0 Iy1 Iy2 Iy3 (int16), so the Newton lane's one 16-byte load gives dp2a-ready pairs: x = (Ix0, Ix1),
+// y = (Ix2, Ix3), z = (Iy0, Iy1), w = (Iy2, Iy3).  Column c keeps Ix at halfword (c >> 2) * 8 + (c & 3) of its row, Iy 4
+// halfwords later.
+__device__ __forceinline__ void tmpl_store(uint32_t *tmpl, int row, int tc, int c, int Ix, int Iy)
+{
+    int16_t *h = reinterpret_cast<int16_t *>(tmpl) + 2 * row * tc + (c >> 2) * 8 + (c & 3);
+    h[0] = (int16_t)Ix;
+    h[4] = (int16_t)Iy;
+}
+
+// lane = template column (strips of <= 32 columns), rows top to bottom.  Writes column col of row r (tmpl_store) for the
+// TROWS x TCOLS template (zero outside the window) and returns the exact sums
 //   A11 = sum Ix^2, A12 = sum Ix*Iy, A22 = sum Iy^2, C1 = sum Iw*Ix, C2 = sum Iw*Iy.
 // The template row r overwrites Scharr patch bytes below row r+1 only (TCOLS <= DPITCH), which every lane has consumed
 // by then (one __syncwarp per row keeps the lanes within a row of each other).
@@ -351,7 +363,7 @@ __device__ __forceinline__ void build_template_split(const uint8_t *ip0, const u
         const int Iw = (int)(v >> 9);
         const int Ix = (d00x * iw00 + d01x * iw01 + d10x * iw10 + d11x * iw11 + 8192) >> 14;
         const int Iy = (d00y * iw00 + d01y * iw01 + d10y * iw10 + d11y * iw11 + 8192) >> 14;
-        tmpl[r * TC + lane] = ((uint32_t)Ix << 16) | ((uint32_t)Iy & 0xffffu);
+        tmpl_store(tmpl, r, TC, lane, Ix, Iy);
         a11 += Ix * Ix; a12 += Ix * Iy; a22 += Iy * Iy;
         c1 += Iw * Ix; c2 += Iw * Iy;
         ipair = cpair; d00x = d10x; d00y = d10y; d01x = d11x; d01y = d11y;
@@ -361,7 +373,7 @@ __device__ __forceinline__ void build_template_split(const uint8_t *ip0, const u
 #pragma unroll
     for (int i = 0; i < NR; i++) {
         const int r = ph + PH * i;
-        if (lane1 && r < WH) tmpl[r * TC + xc] = tv[i];
+        if (lane1 && r < WH) tmpl_store(tmpl, r, TC, xc, (int)tv[i] >> 16, (int)(short)(tv[i] & 0xffffu));
     }
     for (int i = WH * TC + lane; i < TR * TC; i += 32) tmpl[i] = 0u;
     sA11 = warp_sum_wide(a11) + warp_sum_wide(e11); sA12 = warp_sum_wide(a12) + warp_sum_wide(e12);
@@ -427,7 +439,7 @@ __device__ __forceinline__ void build_template(const LKArgs &a, const uint8_t *i
                 const int Iy = (d00y[s] * m00[s] + d01y[s] * m01[s] + d10y * m10[s] + d11y * m11[s] + 8192) >> 14;
                 // (compile-time window sizes fold these guards away where every lane owns a template column)
                 if ((SC >= 32 || lane < SC) && (NS * SC <= TC || col < TC))
-                    tmpl[r * TC + col] = ((uint32_t)Ix << 16) | ((uint32_t)Iy & 0xffffu);
+                    tmpl_store(tmpl, r, TC, col, Ix, Iy);
                 a11[s] += Ix * Ix; a12[s] += Ix * Iy; a22[s] += Iy * Iy;
                 c1[s] += Iw * Ix; c2[s] += Iw * Iy;
                 ipair[s] = cpair; d00x[s] = d10x; d00y[s] = d10y; d01x[s] = d11x; d01y[s] = d11y;
@@ -450,7 +462,12 @@ __device__ __forceinline__ void build_template(const LKArgs &a, const uint8_t *i
 // ---- Newton pass ---------------------------------------------------------------------------------------------
 // Lane = (row group, column quad): rows [rowbase, rowbase + RG), template columns [4*cq, 4*cq + 4).
 // S1 = sum Jw * Ix, S2 = sum Jw * Iy over the window, Jw = DESCALE(bilinear J at byte offset (ox, oy) inside the patch, 9).
-// Partial sums are flushed to int64 every 16 rows (64 pixels * 8160 * 4080 < 2^31).
+// The products run on dp2a too: the four samples j0..j3 (0 <= j <= 255 * 32 = 8160) are split into bytes, jb01 = (lo0, lo1,
+// hi0, hi1), jb23 likewise, and dp2a.lo / dp2a.hi against the template pairs give sum lo * Ix and sum hi * Ix separately;
+// S1 = sum(lo * Ix) + 256 * sum(hi * Ix), the same integer as sum j * Ix.
+// Headroom: |Ix|, |Iy| <= 16 * 255 = 4080 (Scharr of u8, bilinear weights summing to 2^14), lo <= 255, hi <= 31.  A lane
+// flushes every 16 rows of its 4 columns, at most 64 pixels whatever the window, so a lo sum is within 64 * 4080 * 255 =
+// 66 585 600 and the 32-lane total within 2 130 739 200 < 2^31: one plain REDUX per sum.
 template <int WW, int WH>
 __device__ __forceinline__ void newton_sums(const LKArgs &a, const uint8_t *__restrict__ patch, int ox, int oy, uint32_t wtop,
                                             uint32_t wbot, const uint32_t *__restrict__ tmpl, int rowbase, int cq, bool lane_on,
@@ -470,25 +487,27 @@ __device__ __forceinline__ void newton_sums(const LKArgs &a, const uint8_t *__re
     S1 = 0; S2 = 0;
     for (int r0 = 0; r0 < RG; r0 += 16) {
         const int r1 = (WW && WH) ? ((RG < r0 + 16) ? RG : r0 + 16) : min(RG, r0 + 16);
-        int b1 = 0, b2 = 0;
+        uint32_t b1lo = 0, b1hi = 0, b2lo = 0, b2hi = 0;
 #pragma unroll((WW && WH) ? 16 : 2)
         for (int r = r0; r < r1; r++) {
             jp += JP >> 2;
             const uint32_t w0 = jp[0], w1 = jp[1];
             const uint32_t c0 = __byte_perm(w0, w1, sel0), c1 = __byte_perm(w0, w1, sel1);
             const uint4 t = tp[r * (TC >> 2)];
-            const int j0 = (int)(dp2a_lo(wbot, c0, dp2a_lo(wtop, p0, 256u)) >> 9);
-            const int j1 = (int)(dp2a_lo(wbot, c1, dp2a_lo(wtop, p1, 256u)) >> 9);
-            const int j2 = (int)(dp2a_hi(wbot, c0, dp2a_hi(wtop, p0, 256u)) >> 9);
-            const int j3 = (int)(dp2a_hi(wbot, c1, dp2a_hi(wtop, p1, 256u)) >> 9);
-            b1 += j0 * ((int)t.x >> 16); b2 += j0 * (int)(short)(t.x & 0xffffu);
-            b1 += j1 * ((int)t.y >> 16); b2 += j1 * (int)(short)(t.y & 0xffffu);
-            b1 += j2 * ((int)t.z >> 16); b2 += j2 * (int)(short)(t.z & 0xffffu);
-            b1 += j3 * ((int)t.w >> 16); b2 += j3 * (int)(short)(t.w & 0xffffu);
+            const uint32_t j0 = dp2a_lo(wbot, c0, dp2a_lo(wtop, p0, 256u)) >> 9;
+            const uint32_t j1 = dp2a_lo(wbot, c1, dp2a_lo(wtop, p1, 256u)) >> 9;
+            const uint32_t j2 = dp2a_hi(wbot, c0, dp2a_hi(wtop, p0, 256u)) >> 9;
+            const uint32_t j3 = dp2a_hi(wbot, c1, dp2a_hi(wtop, p1, 256u)) >> 9;
+            const uint32_t jb01 = __byte_perm(j0, j1, 0x5140u), jb23 = __byte_perm(j2, j3, 0x5140u);
+            b1lo = dp2a_lo(t.y, jb23, dp2a_lo(t.x, jb01, b1lo));
+            b1hi = dp2a_hi(t.y, jb23, dp2a_hi(t.x, jb01, b1hi));
+            b2lo = dp2a_lo(t.w, jb23, dp2a_lo(t.z, jb01, b2lo));
+            b2hi = dp2a_hi(t.w, jb23, dp2a_hi(t.z, jb01, b2hi));
             p0 = c0; p1 = c1;
         }
-        if (!lane_on) { b1 = 0; b2 = 0; }                       // lanes beyond the last row group
-        S1 += warp_sum_wide(b1); S2 += warp_sum_wide(b2);
+        if (!lane_on) { b1lo = b1hi = b2lo = b2hi = 0; }        // lanes beyond the last row group
+        S1 += (long long)__reduce_add_sync(0xffffffffu, (int)b1lo) + ((long long)__reduce_add_sync(0xffffffffu, (int)b1hi) << 8);
+        S2 += (long long)__reduce_add_sync(0xffffffffu, (int)b2lo) + ((long long)__reduce_add_sync(0xffffffffu, (int)b2hi) << 8);
     }
 }
 
