@@ -57,10 +57,13 @@ SIGNATURES = {
     "ibt_pyramid_levels": (_i, [_i, _i, _i, _i, _i, C.POINTER(C.c_int)]),
     "ibt_pyr_level_u8": (_i, [_vp, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp]),
     "ibt_pyramid_build": (_i, [_PYR, _i, _vp]),
+    "ibt_pyramid_build_multichannel": (_i, [_vp, _i64, _i, C.POINTER(_PYR), _i, _vp]),
     "ibt_lk": (_i, [_PYR, _PYR, _vp, _vp, _i, _i, _i, _i, _d, _d, _i, _vp, _vp, _vp, _vp]),
     "ibt_lk_multichannel": (_i, [C.POINTER(_PYR), C.POINTER(_PYR), _i, _vp, _vp, _i, _i, _i, _i, _d, _d, _i, _vp, _vp, _vp, _vp]),
     "ibt_lk_fb": (_i, [_PYR, _PYR, _vp, _i, _i, _i, _i, _d, _d, _f, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                        _vp, _vp]),
+    "ibt_lk_fb_multichannel": (_i, [C.POINTER(_PYR), C.POINTER(_PYR), _i, _vp, _i, _i, _i, _i, _d, _d, _f, _vp, _vp, _vp, _vp,
+                                    _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ibt_min_eigen_f32": (_i, [_vp, _i, _i, _i64, _i, _vp, _i64, _vp]),
     "ibt_gftt_workspace_bytes": (_sz, [_i, _i]),
     "ibt_corner_harris_f32": (_i, [_vp, _i, _i, _i64, _i, _d, _vp, _i64, _vp]),

@@ -795,7 +795,7 @@ lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKFrames<CN>
         const LKPyr *PI = a.pyr + pass, *PJ = a.pyr + (pass ^ 1);
         const CUtensorMap *mapI = nullptr, *mapJ = nullptr, *mapD = nullptr;
         if constexpr (CN == 1) { mapI = fr.imgI[pass]; mapJ = fr.imgJ[pass ^ 1]; mapD = fr.der[pass]; }
-        else { PI = fr.I; PJ = fr.J; }
+        else { PI = pass ? fr.J : fr.I; PJ = pass ? fr.I : fr.J; }
         lk_point<WW, WH, CN>(PI, PJ, cn, a, ptx, pty, use_init, want_status, want_err, ox, oy, status, err, iters,
                              slab, rowbase, cq, lane_on, lane, mapI, mapJ, mapD, lk_bars[wib], phases);
         if (pass == 0) it_f = iters; else it_b = iters;
@@ -882,7 +882,7 @@ static int lk_queue_for(int dev, cudaStream_t st, unsigned int **out)
 
 // The one launcher of every LK entry point.  A and B are host arrays of cn pyramids, one per channel plane.  planes == false
 // (ibt_lk, ibt_lk_fb; cn == 1): gray frames in a.pyr, with tensor maps, on the window-specialised kernels.  planes == true
-// (ibt_lk_multichannel): the channel pyramids travel as LKMcPyr to the runtime-cn kernel.
+// (ibt_lk_multichannel, ibt_lk_fb_multichannel): the channel pyramids travel as LKMcPyr to the runtime-cn kernel.
 static int launch_lk(LKArgs &a, const ibt_pyramid_t *const *A, const ibt_pyramid_t *const *B, int cn, bool planes, int winW,
                      int winH, int max_count, double epsilon, double min_eig, cudaStream_t st)
 {
@@ -1041,5 +1041,21 @@ IBT_API int ibt_lk_multichannel(const ibt_pyramid_t *const *pyrI, const ibt_pyra
     a.p0 = pts; a.n = N; a.flags = flags; a.fb = 0;
     a.p1 = next_pts; a.st1 = status; a.err1 = err; a.iters = iters;
     return ibt::launch_lk(a, pyrI, pyrJ, cn, true, winW, winH, max_count, epsilon, min_eig_threshold,
+                          static_cast<cudaStream_t>(stream));
+}
+
+IBT_API int ibt_lk_fb_multichannel(const ibt_pyramid_t *const *prev, const ibt_pyramid_t *const *next, int cn, const float *p0,
+                                   int N, int winW, int winH, int max_count, double epsilon, double min_eig_threshold,
+                                   float fb_threshold, float *p1, uint8_t *st1, float *err1, float *p0r, uint8_t *st0,
+                                   float *err0, float *fbdist, uint8_t *alive, int32_t *iters, unsigned long long *iter_total,
+                                   void *stream)
+{
+    if (cn < 2 || cn > ibt::LK_MC_MAX) return IBT_E_INVALID;
+    ibt::LKArgs a;
+    memset(&a, 0, sizeof(a));
+    a.p0 = p0; a.n = N; a.flags = 0; a.fb = 1; a.fb_thresh = fb_threshold;
+    a.p1 = p1; a.st1 = st1; a.err1 = err1; a.p0r = p0r; a.st0 = st0; a.err0 = err0;
+    a.fbdist = fbdist; a.alive = alive; a.iters = iters; a.iter_total = iter_total;
+    return ibt::launch_lk(a, prev, next, cn, true, winW, winH, max_count, epsilon, min_eig_threshold,
                           static_cast<cudaStream_t>(stream));
 }

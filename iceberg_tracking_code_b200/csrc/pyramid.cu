@@ -294,6 +294,236 @@ pyr_level_tma_kernel(const __grid_constant__ PyrArgs a, const __grid_constant__ 
     }
 }
 
+// ---- multi-channel frames (ibt_pyramid_build_multichannel) ------------------------------------------------------------
+// A level >= 1 of a cn-channel frame is cn single-channel planes of one geometry, filtered in ONE launch: the tile index also
+// selects the channel (tile t = channel t / ntiles, that plane's tile t % ntiles), each plane brings its own PyrArgs and tensor
+// map.  Same tiles, helpers and pipelines as pyr_level_kernel / pyr_level_tma_kernel, whose loops are repeated here rather
+// than shared: routing the gray kernels through a common body changes their register allocation.
+constexpr int PYR_MAX_CN = 4;
+struct PyrLevelSet {
+    PyrArgs ch[PYR_MAX_CN];
+    int cn;
+};
+struct PyrMapSet { CUtensorMap m[PYR_MAX_CN]; };
+
+__device__ __forceinline__ const PyrArgs &set_tile(const PyrLevelSet &s, int t, int &tc, int &c)
+{
+    c = t / s.ch[0].ntiles;
+    tc = t - c * s.ch[0].ntiles;
+    return s.ch[c];
+}
+
+template <bool DERIV, bool DOWN, int NW, int RPW>
+__global__ void __launch_bounds__(NW * 32, pyr_ctas_per_sm(NW))
+pyr_level_set_kernel(const __grid_constant__ PyrLevelSet s)
+{
+    constexpr int TH = NW * RPW, SROWS = TH + 3;
+    __shared__ __align__(16) uint8_t tiles[2][SROWS * SPITCH];
+    const int tid = threadIdx.x, ntiles = s.cn * s.ch[0].ntiles;
+    pdl_launch_dependents();
+    pdl_wait();                                           // the source level is the previous launch's output
+    int t = blockIdx.x, buf = 0, tc, c;
+    if (t < ntiles) { const PyrArgs &a = set_tile(s, t, tc, c); stage_tile<NW, RPW>(a, tc, tiles[0], tid); }
+    asm volatile("cp.async.commit_group;" ::: "memory");
+    for (; t < ntiles; t += gridDim.x) {
+        const int tn = t + gridDim.x;
+        if (tn < ntiles) { const PyrArgs &an = set_tile(s, tn, tc, c); stage_tile<NW, RPW>(an, tc, tiles[buf ^ 1], tid); }
+        asm volatile("cp.async.commit_group;" ::: "memory");
+        asm volatile("cp.async.wait_group 1;" ::: "memory");                  // tile t has landed
+        __syncthreads();
+        const PyrArgs &a = set_tile(s, t, tc, c);
+        if (reflect_tile<NW, RPW>(a, tc, tiles[buf], tid)) __syncthreads();
+        const int ty = tc / a.ntx, tx = tc - ty * a.ntx;
+        if ((tx + 1) * TW <= a.w && (ty + 1) * TH <= a.h) filter_tile<DERIV, DOWN, NW, RPW, true>(a, tc, tiles[buf], tid);
+        else filter_tile<DERIV, DOWN, NW, RPW, false>(a, tc, tiles[buf], tid);
+        __syncthreads();                                                      // buffer may be refilled next round
+        buf ^= 1;
+    }
+}
+
+template <bool DERIV, bool DOWN, int NW, int RPW>
+__global__ void __launch_bounds__(NW * 32, pyr_ctas_per_sm(NW))
+pyr_level_set_tma_kernel(const __grid_constant__ PyrLevelSet s, const __grid_constant__ PyrMapSet maps)
+{
+    constexpr int TH = NW * RPW, SROWS = TH + 3;
+    constexpr unsigned TILE_BYTES = SROWS * SPITCH;
+    constexpr unsigned TILE_ALLOC = (TILE_BYTES + 127) & ~127u;
+    __shared__ __align__(128) uint8_t tiles[2][TILE_ALLOC];
+    __shared__ __align__(8) uint64_t full[2];
+    const int tid = threadIdx.x, ntiles = s.cn * s.ch[0].ntiles;
+    pdl_launch_dependents();
+    if (tid == 0) {
+        for (int c = 0; c < s.cn; c++) tma_prefetch_map(&maps.m[c]);     // the descriptors do not depend on the previous launch
+        mbar_init(&full[0], 1); mbar_init(&full[1], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    pdl_wait();                                           // the source level is the previous launch's output
+    auto issue = [&](int t, int b) {                      // one thread: arm the barrier, launch the bulk tensor copy
+        if (tid == 0) {
+            int tc, c;
+            const PyrArgs &a = set_tile(s, t, tc, c);
+            const int ty = tc / a.ntx, tx = tc - ty * a.ntx;
+            fence_proxy_async();                                              // our generic-proxy patches precede the async write
+            mbar_expect_tx(&full[b], TILE_BYTES);
+            tma_load_2d(tiles[b], &maps.m[c], tx * TW - HXB, ty * TH - 2, &full[b]);
+        }
+    };
+    unsigned phases = 0u;                                 // bit b = parity to wait for on full[b]
+    int t = blockIdx.x, buf = 0;
+    if (t < ntiles) issue(t, 0);
+    for (; t < ntiles; t += gridDim.x) {
+        const int tn = t + gridDim.x;
+        if (tn < ntiles) issue(tn, buf ^ 1);                                  // prefetch the next tile of this CTA
+        mbar_wait(&full[buf], (phases >> buf) & 1u);                          // tile t has landed
+        phases ^= 1u << buf;
+        int tc, c;
+        const PyrArgs &a = set_tile(s, t, tc, c);
+        if (reflect_rows<NW, RPW>(a, tc, tiles[buf], tid)) __syncthreads();
+        if (reflect_tile<NW, RPW>(a, tc, tiles[buf], tid)) __syncthreads();
+        const int ty = tc / a.ntx, tx = tc - ty * a.ntx;
+        if ((tx + 1) * TW <= a.w && (ty + 1) * TH <= a.h) filter_tile<DERIV, DOWN, NW, RPW, true>(a, tc, tiles[buf], tid);
+        else filter_tile<DERIV, DOWN, NW, RPW, false>(a, tc, tiles[buf], tid);
+        __syncthreads();                                                      // buffer may be refilled next round
+        buf ^= 1;
+    }
+}
+
+// Level 0 of a cn-channel frame: the interleaved (H,W,cn) u8 frame is read once, at any pitch and alignment, and every channel
+// gets its level-0 plane, its Scharr planes and its level-1 plane.  Tiles of 128 x 32 pixels (4 warps x 8 rows; a 128 x 64
+// tile of 4 channels would not leave room for two CTAs per SM).  16-byte aligned frames (base and pitch) stage the interleaved
+// halo tile by cp.async, zero-filling past the end of the row, and de-interleave it once into the cn single-channel tiles that
+// filter_tile reads; the REFLECT_101 columns are then patched per channel by reflect_tile.  Any other frame takes the byte
+// path, which gathers the pixels channel by channel with REFLECT_101 resolved on load (as pyr_level_kernel does).  The
+// interleaved buffer is refilled with the next tile while the channels of this one are filtered.
+constexpr int F_NW = 4, F_RPW = 8, F_TH = F_NW * F_RPW, F_SROWS = F_TH + 3;
+struct PyrFrameArgs {
+    PyrArgs ch[PYR_MAX_CN];         // per channel: its level-0 plane (h, w, pitch), Scharr planes, level-1 plane
+    uint8_t *plane[PYR_MAX_CN];     // = ch[c].src, written here
+    const uint8_t *frame; int64_t fpitch;
+    int frame_vec_ok;               // 16-byte aligned base and pitch: cp.async staging
+    int plane_vec_ok;               // every plane has a 4-byte aligned base and pitch: word stores
+};
+
+template <int CN>
+__device__ __forceinline__ void stage_frame(const PyrFrameArgs &f, int t, uint8_t *stage, int tid)
+{
+    constexpr int FP = SPITCH * CN, CH = FP / 16, RSTEP = F_NW * 32 / CH;
+    const PyrArgs &a = f.ch[0];
+    const int ty = t / a.ntx, tx = t - ty * a.ntx;
+    const int r0 = tid / CH, c = tid - r0 * CH;
+    const int64_t gx = (int64_t)(tx * TW - HXB) * CN + 16 * c, rowb = (int64_t)a.w * CN;
+    if (r0 >= RSTEP || gx < 0 || gx >= rowb) return;
+    const unsigned n = gx + 16 <= rowb ? 16u : (unsigned)(rowb - gx);       // the rest of the chunk is zero-filled
+    const unsigned sdst = (unsigned)__cvta_generic_to_shared(stage) + 16 * c;
+    const uint8_t *g0 = f.frame + gx;
+    for (int r = r0; r < F_SROWS; r += RSTEP) {
+        const uint8_t *g = g0 + (int64_t)r101(ty * F_TH - 2 + r, a.h) * f.fpitch;
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(sdst + r * FP), "l"(g), "r"(n) : "memory");
+    }
+}
+
+// interleaved staged rows -> CN tiles of the single-channel layout, four pixels (CN words in, one word per channel out) a step
+template <int CN>
+__device__ __forceinline__ void deinterleave(const uint8_t *stage, uint8_t (*tiles)[F_SROWS * SPITCH], int tid)
+{
+    constexpr int Q = SPITCH / 4;
+    for (int i = tid; i < F_SROWS * Q; i += F_NW * 32) {
+        const int r = i / Q, q = i - r * Q;
+        const uint32_t *src = reinterpret_cast<const uint32_t *>(stage + r * SPITCH * CN) + q * CN;
+        uint32_t w[CN];
+#pragma unroll
+        for (int k = 0; k < CN; k++) w[k] = src[k];
+#pragma unroll
+        for (int c = 0; c < CN; c++) {
+            uint32_t o = 0;
+#pragma unroll
+            for (int p = 0; p < 4; p++) {
+                const int b = p * CN + c;
+                o |= ((w[b >> 2] >> (8 * (b & 3))) & 0xffu) << (8 * p);
+            }
+            reinterpret_cast<uint32_t *>(tiles[c] + r * SPITCH)[q] = o;
+        }
+    }
+}
+
+// byte path: pixel columns x0-4 .. x0+TW+3 of every channel, REFLECT_101 resolved here
+template <int CN>
+__device__ __forceinline__ void gather_frame(const PyrFrameArgs &f, int t, uint8_t (*tiles)[F_SROWS * SPITCH], int tid)
+{
+    const PyrArgs &a = f.ch[0];
+    const int ty = t / a.ntx, tx = t - ty * a.ntx;
+    for (int idx = tid; idx < F_SROWS * (TW + 8); idx += F_NW * 32) {
+        const int r = idx / (TW + 8), c = idx - r * (TW + 8);
+        const uint8_t *g = f.frame + (int64_t)r101(ty * F_TH - 2 + r, a.h) * f.fpitch + (int64_t)r101(tx * TW - 4 + c, a.w) * CN;
+#pragma unroll
+        for (int k = 0; k < CN; k++) tiles[k][r * SPITCH + (HXB - 4) + c] = g[k];
+    }
+}
+
+// this warp's rows of the level-0 plane, straight from the channel tile
+__device__ __forceinline__ void store_plane(const PyrArgs &a, uint8_t *plane, bool vec, int t, const uint8_t *tile, int tid)
+{
+    const int ty = t / a.ntx, tx = t - ty * a.ntx;
+    const int lane = tid & 31, wy = tid >> 5;
+    const int x = tx * TW + 4 * lane, y0 = ty * F_TH + F_RPW * wy;
+    if (x >= a.w) return;
+    const uint8_t *s = tile + (F_RPW * wy + 2) * SPITCH + HXB + 4 * lane;
+    uint8_t *p = plane + (int64_t)y0 * a.pitch + x;
+    for (int j = 0; j < F_RPW && y0 + j < a.h; j++, s += SPITCH, p += a.pitch) {
+        if (vec && x + 3 < a.w) {
+            *reinterpret_cast<uint32_t *>(p) = *reinterpret_cast<const uint32_t *>(s);
+        } else {
+            for (int i = 0; i < 4 && x + i < a.w; i++) p[i] = s[i];
+        }
+    }
+}
+
+template <int CN, bool DERIV, bool DOWN>
+__global__ void __launch_bounds__(F_NW * 32)
+pyr_frame_kernel(const __grid_constant__ PyrFrameArgs f)
+{
+    __shared__ __align__(16) uint8_t stage[F_SROWS * SPITCH * CN];           // interleaved rows of the next tile
+    __shared__ __align__(16) uint8_t tiles[CN][F_SROWS * SPITCH];
+    const int tid = threadIdx.x, ntiles = f.ch[0].ntiles;
+    const bool vec = f.frame_vec_ok != 0;
+    pdl_launch_dependents();
+    pdl_wait();                                           // the frame may be the previous launch's output
+    int t = blockIdx.x;
+    if (vec && t < ntiles) stage_frame<CN>(f, t, stage, tid);
+    asm volatile("cp.async.commit_group;" ::: "memory");
+    for (; t < ntiles; t += gridDim.x) {
+        if (vec) {
+            asm volatile("cp.async.wait_group 0;" ::: "memory");
+            __syncthreads();                              // tile t has landed; the channel tiles of t - grid are consumed
+            deinterleave<CN>(stage, tiles, tid);
+            __syncthreads();                              // the interleaved buffer is free again
+            if (t + gridDim.x < ntiles) stage_frame<CN>(f, t + gridDim.x, stage, tid);
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            bool patched = false;
+#pragma unroll
+            for (int c = 0; c < CN; c++) patched |= reflect_tile<F_NW, F_RPW>(f.ch[c], t, tiles[c], tid);
+            if (patched) __syncthreads();
+        } else {
+            __syncthreads();                              // the channel tiles of t - grid are consumed
+            gather_frame<CN>(f, t, tiles, tid);
+            __syncthreads();
+        }
+        const PyrArgs &a0 = f.ch[0];
+        const int ty = t / a0.ntx, tx = t - ty * a0.ntx;
+        const bool full = (tx + 1) * TW <= a0.w && (ty + 1) * F_TH <= a0.h;
+#pragma unroll
+        for (int c = 0; c < CN; c++) {
+            store_plane(f.ch[c], f.plane[c], f.plane_vec_ok != 0, t, tiles[c], tid);
+            if (DERIV || DOWN) {
+                if (full) filter_tile<DERIV, DOWN, F_NW, F_RPW, true>(f.ch[c], t, tiles[c], tid);
+                else filter_tile<DERIV, DOWN, F_NW, F_RPW, false>(f.ch[c], t, tiles[c], tid);
+            }
+        }
+    }
+    asm volatile("cp.async.wait_group 0;" ::: "memory");
+}
+
 static bool make_tile_map(CUtensorMap *m, const uint8_t *src, int h, int w, int64_t pitch, int srows)
 {
     return make_map_2d(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, src, w, h, pitch, SPITCH, srows);
@@ -320,15 +550,14 @@ static void launch_variant(const PyrArgs &a0, cudaStream_t st)
     (void)launch_pdl(pyr_level_kernel<DERIV, DOWN, NW, RPW>, dim3(blocks), dim3(NW * 32), 0, st, a);
 }
 
-static int launch_level(const uint8_t *src, int h, int w, int64_t pitch, int16_t *deriv, int64_t dpitch,
-                        uint8_t *down, int64_t downpitch, cudaStream_t st)
+// checks one level step's arguments and fills its PyrArgs (ntx / ntiles are set by the launcher)
+static int level_args(const uint8_t *src, int h, int w, int64_t pitch, int16_t *deriv, int64_t dpitch, uint8_t *down,
+                      int64_t downpitch, PyrArgs &a)
 {
     if (!src || h <= 0 || w <= 0 || pitch < w) return IBT_E_INVALID;
-    if (!deriv && !down) return IBT_OK;
     if (deriv && (dpitch < (int64_t)w * 4 || dpitch % 4 != 0 || reinterpret_cast<uintptr_t>(deriv) % 4 != 0))
         return IBT_E_INVALID;
     if (down && downpitch < (w + 1) / 2) return IBT_E_INVALID;
-    PyrArgs a;
     a.src = src; a.h = h; a.w = w; a.pitch = pitch;
     a.deriv = reinterpret_cast<uint8_t *>(deriv); a.dpitch = dpitch;
     a.down = down; a.downpitch = downpitch;
@@ -336,6 +565,17 @@ static int launch_level(const uint8_t *src, int h, int w, int64_t pitch, int16_t
     a.deriv_vec_ok = deriv && (reinterpret_cast<uintptr_t>(deriv) % 16 == 0) && (dpitch % 16 == 0);
     a.down_vec_ok = down && (reinterpret_cast<uintptr_t>(down) % 2 == 0) && (downpitch % 2 == 0);
     a.ntx = a.ntiles = 0;
+    return IBT_OK;
+}
+
+static int launch_level(const uint8_t *src, int h, int w, int64_t pitch, int16_t *deriv, int64_t dpitch,
+                        uint8_t *down, int64_t downpitch, cudaStream_t st)
+{
+    if (!src || h <= 0 || w <= 0 || pitch < w) return IBT_E_INVALID;
+    if (!deriv && !down) return IBT_OK;
+    PyrArgs a;
+    const int rc = level_args(src, h, w, pitch, deriv, dpitch, down, downpitch, a);
+    if (rc != IBT_OK) return rc;
     // big levels: 128 x 64 tiles (4 warps x 16 rows).  Smaller levels are latency-bound -- a launch lasts as long as one warp
     // needs for its rows -- so they take 1-warp tiles of 4 rows: every SM gets work and no warp walks more than 7 rows
     const bool big = (int64_t)((w + TW - 1) / TW) * ((h + 63) / 64) >= 2 * kNumSMs;
@@ -343,6 +583,119 @@ static int launch_level(const uint8_t *src, int h, int w, int64_t pitch, int16_t
     else if (deriv)    { if (big) launch_variant<true, false, 4, 16>(a, st); else launch_variant<true, false, 1, 4>(a, st); }
     else               { if (big) launch_variant<false, true, 4, 16>(a, st); else launch_variant<false, true, 1, 4>(a, st); }
     return check_launch("ibt_pyr_level_u8");
+}
+
+// one level of all cn channel planes in one launch (the tile choice of launch_level, counted over the channels)
+template <bool DERIV, bool DOWN, int NW, int RPW>
+static void launch_set_variant(PyrLevelSet &s, cudaStream_t st)
+{
+    constexpr int TH = NW * RPW;
+    bool tma = getenv("IBT_NO_TMA") == nullptr;
+    static thread_local PyrMapSet maps;
+    for (int c = 0; c < s.cn; c++) {
+        PyrArgs &a = s.ch[c];
+        a.ntx = (a.w + TW - 1) / TW;
+        a.ntiles = a.ntx * ((a.h + TH - 1) / TH);
+        tma = tma && a.src_vec_ok && a.h >= 8 && a.w >= 16 && make_tile_map(&maps.m[c], a.src, a.h, a.w, a.pitch, TH + 3);
+    }
+    const int ntiles = s.cn * s.ch[0].ntiles;
+    const int resident = kNumSMs * pyr_ctas_per_sm(NW);
+    const int per_cta = (ntiles + resident - 1) / resident;
+    const int blocks = (ntiles + per_cta - 1) / per_cta;
+    if (tma) (void)launch_pdl(pyr_level_set_tma_kernel<DERIV, DOWN, NW, RPW>, dim3(blocks), dim3(NW * 32), 0, st, s, maps);
+    else (void)launch_pdl(pyr_level_set_kernel<DERIV, DOWN, NW, RPW>, dim3(blocks), dim3(NW * 32), 0, st, s);
+}
+
+static void launch_level_set(PyrLevelSet &s, cudaStream_t st)
+{
+    const PyrArgs &a = s.ch[0];
+    const bool deriv = a.deriv != nullptr, down = a.down != nullptr;
+    const bool big = (int64_t)((a.w + TW - 1) / TW) * ((a.h + 63) / 64) * s.cn >= 2 * kNumSMs;
+    if (deriv && down) { if (big) launch_set_variant<true, true, 4, 16>(s, st); else launch_set_variant<true, true, 1, 4>(s, st); }
+    else if (deriv)    { if (big) launch_set_variant<true, false, 4, 16>(s, st); else launch_set_variant<true, false, 1, 4>(s, st); }
+    else               { if (big) launch_set_variant<false, true, 4, 16>(s, st); else launch_set_variant<false, true, 1, 4>(s, st); }
+}
+
+template <int CN, bool DERIV, bool DOWN>
+static void launch_frame_variant(const PyrFrameArgs &f, int ntiles, cudaStream_t st)
+{
+    static int per_sm[64] = {0};                          // resident CTAs per SM, per device (shared memory grows with CN)
+    int dev = 0;
+    (void)cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64) dev = 0;
+    if (per_sm[dev] == 0) {
+        int n = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, pyr_frame_kernel<CN, DERIV, DOWN>, F_NW * 32, 0) != cudaSuccess || n < 1)
+            n = 1;
+        per_sm[dev] = n;
+    }
+    const int resident = kNumSMs * per_sm[dev];
+    const int per_cta = (ntiles + resident - 1) / resident;
+    const int blocks = (ntiles + per_cta - 1) / per_cta;
+    (void)launch_pdl(pyr_frame_kernel<CN, DERIV, DOWN>, dim3(blocks), dim3(F_NW * 32), 0, st, f);
+}
+
+template <int CN>
+static void launch_frame(const PyrFrameArgs &f, int ntiles, cudaStream_t st)
+{
+    const bool deriv = f.ch[0].deriv != nullptr, down = f.ch[0].down != nullptr;
+    if (deriv && down) launch_frame_variant<CN, true, true>(f, ntiles, st);
+    else if (deriv)    launch_frame_variant<CN, true, false>(f, ntiles, st);
+    else if (down)     launch_frame_variant<CN, false, true>(f, ntiles, st);
+    else               launch_frame_variant<CN, false, false>(f, ntiles, st);
+}
+
+static int build_multichannel(const uint8_t *frame, int64_t fpitch, int cn, const ibt_pyramid_t *const *pyr, int with_derivs,
+                              cudaStream_t st)
+{
+    if (!frame || cn < 2 || cn > PYR_MAX_CN || !pyr) return IBT_E_INVALID;
+    for (int c = 0; c < cn; c++)
+        if (!pyr[c]) return IBT_E_INVALID;
+    const ibt_pyramid_t &p0 = *pyr[0];
+    const int L = p0.nlevels;
+    if (L < 1 || L > IBT_MAX_LEVELS || p0.rows[0] <= 0 || p0.cols[0] <= 0 || fpitch < (int64_t)p0.cols[0] * cn)
+        return IBT_E_INVALID;
+    for (int c = 0; c < cn; c++) {
+        const ibt_pyramid_t &p = *pyr[c];
+        if (p.nlevels != L) return IBT_E_INVALID;
+        for (int l = 0; l < L; l++) {
+            if (p.rows[l] != p0.rows[l] || p.cols[l] != p0.cols[l] || !p.img[l]) return IBT_E_INVALID;
+            if (l + 1 < L && (p.rows[l + 1] != (p.rows[l] + 1) / 2 || p.cols[l + 1] != (p.cols[l] + 1) / 2)) return IBT_E_INVALID;
+            if (with_derivs && !p.deriv[l]) return IBT_E_INVALID;
+        }
+    }
+    // every level's arguments are checked before the first launch
+    PyrFrameArgs f;
+    static thread_local PyrLevelSet sets[IBT_MAX_LEVELS];
+    f.frame = frame; f.fpitch = fpitch;
+    f.frame_vec_ok = (reinterpret_cast<uintptr_t>(frame) % 16 == 0) && (fpitch % 16 == 0);
+    f.plane_vec_ok = 1;
+    for (int l = 0; l < L; l++) {
+        sets[l].cn = cn;
+        for (int c = 0; c < cn; c++) {
+            const ibt_pyramid_t &p = *pyr[c];
+            const bool last = l + 1 == L;
+            PyrArgs &a = l == 0 ? f.ch[c] : sets[l].ch[c];
+            const int rc = level_args(p.img[l], p.rows[l], p.cols[l], p.img_pitch[l],
+                                      with_derivs ? const_cast<int16_t *>(p.deriv[l]) : nullptr, with_derivs ? p.deriv_pitch[l] : 0,
+                                      last ? nullptr : const_cast<uint8_t *>(p.img[l + 1]), last ? 0 : p.img_pitch[l + 1], a);
+            if (rc != IBT_OK) return rc;
+        }
+    }
+    const int ntx = (p0.cols[0] + TW - 1) / TW, ntiles = ntx * ((p0.rows[0] + F_TH - 1) / F_TH);
+    for (int c = 0; c < cn; c++) {
+        PyrArgs &a = f.ch[c];
+        f.plane[c] = const_cast<uint8_t *>(a.src);
+        f.plane_vec_ok &= (reinterpret_cast<uintptr_t>(a.src) % 4 == 0) && (a.pitch % 4 == 0);
+        a.src_vec_ok = f.frame_vec_ok;                    // reflect_tile: REFLECT_101 columns are patched in the tile
+        a.ntx = ntx; a.ntiles = ntiles;
+    }
+    if (cn == 2) launch_frame<2>(f, ntiles, st);
+    else if (cn == 3) launch_frame<3>(f, ntiles, st);
+    else launch_frame<4>(f, ntiles, st);
+    for (int l = 1; l < L; l++)
+        if (with_derivs || l + 1 < L) launch_level_set(sets[l], st);
+    return check_launch("ibt_pyramid_build_multichannel");
 }
 
 } // namespace ibt
@@ -384,4 +737,10 @@ IBT_API int ibt_pyramid_build(const ibt_pyramid_t *pyr, int with_derivs, void *s
         if (rc != IBT_OK) return rc;
     }
     return IBT_OK;
+}
+
+IBT_API int ibt_pyramid_build_multichannel(const uint8_t *frame, int64_t frame_pitch, int cn, const ibt_pyramid_t *const *pyr,
+                                           int with_derivs, void *stream)
+{
+    return ibt::build_multichannel(frame, frame_pitch, cn, pyr, with_derivs, static_cast<cudaStream_t>(stream));
 }

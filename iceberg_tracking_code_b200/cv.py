@@ -114,27 +114,46 @@ def _round_up(v, m):
     return (v + m - 1) // m * m
 
 
+def _frame_dev(img, what):
+    """(H,W,C) u8 frame -> CUDA tensor whose pixels are interleaved (strides (pitch, C, 1)); a device view with a row pitch (a
+    crop) is used as it is, anything else is made contiguous."""
+    f = img if isinstance(img, torch.Tensor) and img.is_cuda and img.dtype == torch.uint8 else _to_dev(img, np.uint8, what)
+    if f.ndim == 3 and f.shape[0] > 0 and not (f.stride(2) == 1 and f.stride(1) == f.shape[2]
+                                               and f.stride(0) >= f.shape[1] * f.shape[2]):
+        f = f.contiguous()
+    return f
+
+
 class FramePyramid:
     """Device-resident Gaussian pyramid (+ Scharr derivative planes) of one frame, as the LK solver consumes it.
     Built ONCE per frame and reused as `next` of pair t-1, `prev` of pair t and by both FB directions (the reference
     rebuilds it four times per pair inside cv2.calcOpticalFlowPyrLK; SURVEY Appendix C).  Accepted by
-    calcOpticalFlowPyrLK in place of an image, like cv2 accepts buildOpticalFlowPyramid's output."""
+    calcOpticalFlowPyrLK in place of an image, like cv2 accepts buildOpticalFlowPyramid's output.
+    A gray (H,W) frame gives levels[l] (h,w) u8 and derivs[l] (h,w,2) int16.  An (H,W,C) frame, C = 2..4, gives one pyramid
+    per channel plane (what cv2 builds for it): levels[l] (C,h,w) u8 and derivs[l] (C,h,w,2) int16, planar; `cn` is C."""
 
     def __init__(self, gray, winSize=(21, 21), maxLevel=3, withDerivatives=True):
-        g = _to_dev(gray, np.uint8, "FramePyramid gray")
-        if g.ndim != 2 or g.shape[0] < 1 or g.shape[1] < 1:
-            raise error("FramePyramid: expected a single-channel (H,W) u8 image")
+        colour = hasattr(gray, "ndim") and gray.ndim == 3
+        if colour and not (2 <= gray.shape[2] <= 4):
+            raise error("FramePyramid: a multi-channel frame is (H,W,C) u8 with C = 2..4, got %s" % (tuple(gray.shape),))
+        g = _frame_dev(gray, "FramePyramid frame") if colour else _to_dev(gray, np.uint8, "FramePyramid gray")
+        if g.ndim not in (2, 3) or g.shape[0] < 1 or g.shape[1] < 1:
+            raise error("FramePyramid: expected a single-channel (H,W) or an (H,W,C) u8 image")
         if not (0 <= int(maxLevel) < N.IBT_MAX_LEVELS):
             raise error("FramePyramid: maxLevel must be in [0, %d]" % (N.IBT_MAX_LEVELS - 1))
         self.winSize = (int(winSize[0]), int(winSize[1]))
         self.with_derivs = bool(withDerivatives)
-        H, W = g.shape
+        self.cn = int(g.shape[2]) if colour else 1
+        H, W = g.shape[:2]
         sizes = (C.c_int * (2 * N.IBT_MAX_LEVELS))()
         ml = N.lib().ibt_pyramid_levels(H, W, self.winSize[0], self.winSize[1], int(maxLevel), sizes)
         if ml < 0:
             N.check(ml, "ibt_pyramid_levels")
         self.maxLevel = ml
         self.sizes = [(sizes[2 * l], sizes[2 * l + 1]) for l in range(ml + 1)]
+        if colour:
+            self._init_planes(g)
+            return
         dev = g.device
         g = self._level0(g)
         self._img_buf = [g]
@@ -163,6 +182,55 @@ class FramePyramid:
                 st.deriv_pitch[l] = dpitch
         self.c = st
         self._build(None)
+
+    def _init_planes(self, frame):
+        """one ibt_pyramid_t per channel plane; every level of every channel (level 0 too: it is de-interleaved from the frame)
+        in buffers of 128-byte row pitch"""
+        cn, dev = self.cn, frame.device
+        self._img_buf, self._deriv_buf, self.levels, self.derivs = [], [], [], []
+        self.chans = [N.ibt_pyramid_t() for _ in range(cn)]
+        for st in self.chans:
+            st.nlevels = self.maxLevel + 1
+        for l, (h, w) in enumerate(self.sizes):
+            pitch = _round_up(w, 128)
+            buf = torch.empty((cn, h, pitch), dtype=torch.uint8, device=dev)
+            self._img_buf.append(buf)
+            self.levels.append(buf[:, :, :w])
+            if self.with_derivs:
+                dpitch = _round_up(w * 4, 128)
+                dbuf = torch.empty((cn, h, dpitch // 2), dtype=torch.int16, device=dev)
+                self._deriv_buf.append(dbuf)
+                self.derivs.append(dbuf[:, :, :2 * w].unflatten(2, (w, 2)))
+            for c, st in enumerate(self.chans):
+                st.rows[l], st.cols[l] = h, w
+                st.img[l] = buf[c].data_ptr()
+                st.img_pitch[l] = pitch
+                if self.with_derivs:
+                    st.deriv[l] = self._deriv_buf[l][c].data_ptr()
+                    st.deriv_pitch[l] = dpitch
+        self.c = None
+        self.chan_ptrs = (C.POINTER(N.ibt_pyramid_t) * cn)(*[C.pointer(st) for st in self.chans])
+        self._build_planes(frame, None)
+
+    def _build_planes(self, frame, probe):
+        if probe is not None:
+            probe[0].record()
+        N.check(N.lib().ibt_pyramid_build_multichannel(_ptr(frame), frame.stride(0), self.cn, self.chan_ptrs,
+                                                       1 if self.with_derivs else 0, _stream()), "ibt_pyramid_build_multichannel")
+        if probe is not None:
+            probe[1].record()
+
+    def level(self, l):
+        """level l in cv2's layout: (h,w) u8, or (h,w,C) u8 for a multi-channel frame"""
+        return self.levels[l] if self.cn == 1 else self.levels[l].permute(1, 2, 0)
+
+    def deriv(self, l):
+        """Scharr planes of level l in cv2's layout: (h,w,2) int16 (dx, dy), or (h,w,2C) int16 with channel c's (dx, dy) at
+        [2c, 2c+1]"""
+        if self.cn == 1:
+            return self.derivs[l]
+        d = self.derivs[l]
+        return d.permute(1, 2, 0, 3).reshape(d.shape[1], d.shape[2], 2 * self.cn)
 
     def _level0(self, g):
         """Level 0 is the caller's gray image itself when its rows are 16-byte aligned (the TMA staging paths need that);
@@ -196,7 +264,14 @@ class FramePyramid:
 
     def rebuild(self, gray, probe=None):
         """Recompute this pyramid in place for another frame of the same size (no allocation: steady-state loop).
-        probe = (start_event, end_event) records CUDA events around the level-0 launch."""
+        probe = (start_event, end_event) records CUDA events around the level-0 launch (multi-channel frames: around the
+        whole build, which is one call)."""
+        if self.cn > 1:
+            f = _frame_dev(gray, "FramePyramid frame")
+            if tuple(f.shape) != tuple(self.sizes[0]) + (self.cn,):
+                raise error("FramePyramid.rebuild: frame size or channel count changed")
+            self._build_planes(f, probe)
+            return self
         g = _to_dev(gray, np.uint8, "FramePyramid gray")
         if tuple(g.shape) != tuple(self.sizes[0]):
             raise error("FramePyramid.rebuild: frame size changed")
@@ -218,14 +293,15 @@ class FramePyramid:
 
 def buildOpticalFlowPyramid(img, winSize, maxLevel, withDerivatives=True):
     """cv2.buildOpticalFlowPyramid -> (maxLevelOut, [L0, D0, L1, D1, ...]) (SURVEY A.3): levels (h,w) u8,
-    derivatives (h,w,2) int16 (dx, dy).  cv2 returns views into padded buffers; these are plain arrays."""
+    derivatives (h,w,2) int16 (dx, dy); an (H,W,C) frame, C = 2..4, gives cv2's (h,w,C) u8 levels and (h,w,2C) int16
+    derivatives (channel c's dx, dy at 2c, 2c+1).  cv2 returns views into padded buffers; these are plain arrays."""
     as_np = _is_np(img)
     p = FramePyramid(img, winSize, maxLevel, withDerivatives)
     out = []
     for l in range(p.maxLevel + 1):
-        out.append(_out(p.levels[l].contiguous(), as_np))
+        out.append(_out(p.level(l).contiguous(), as_np))
         if withDerivatives:
-            out.append(_out(p.derivs[l].contiguous(), as_np))
+            out.append(_out(p.deriv(l).contiguous(), as_np))
     return p.maxLevel, out
 
 
@@ -253,8 +329,10 @@ def _as_pyramid(img, winSize, maxLevel, need_derivs, what):
 
 
 def _channels(img):
-    """1 for a FramePyramid or an (H,W) / (H,W,1) image, C for an (H,W,C) image"""
-    if isinstance(img, FramePyramid) or not hasattr(img, "ndim") or img.ndim != 3:
+    """a FramePyramid's cn; 1 for an (H,W) / (H,W,1) image, C for an (H,W,C) image"""
+    if isinstance(img, FramePyramid):
+        return img.cn
+    if not hasattr(img, "ndim") or img.ndim != 3:
         return 1
     return int(img.shape[2])
 
@@ -268,6 +346,11 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
     Returns (nextPts, status (N,1) u8, err (N,1) f32); nextPts has prevPts' shape; N == 0 -> (None, None, None).
     err is 0 where status == 0 (cv2 leaves uninitialised memory there).  prevImg / nextImg may be FramePyramid
     objects.  return_iters=True appends the (N,) int32 count of inner iterations executed per point."""
+    cn = _channels(prevImg)
+    if cn != _channels(nextImg):
+        raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in the number of channels")
+    if cn > 4:
+        raise error("calcOpticalFlowPyrLK: at most 4 channels")
     as_np = _is_np(prevPts)
     if as_np and prevPts.dtype != np.float32:
         raise error("calcOpticalFlowPyrLK: prevPts must be float32 (cv2 asserts the same)")
@@ -285,27 +368,14 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
     if maxLevel < 0:
         raise error("calcOpticalFlowPyrLK: maxLevel must be >= 0")
     cnt, eps = _criteria(criteria)
-    cn = _channels(prevImg)
-    if cn != _channels(nextImg):
-        raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in the number of channels")
-    if cn == 1:
-        pI = _as_pyramid(prevImg, w, maxLevel, True, "calcOpticalFlowPyrLK prevImg")
-        pJ = _as_pyramid(nextImg, w, maxLevel, False, "calcOpticalFlowPyrLK nextImg")
-        if pI.sizes[0] != pJ.sizes[0]:
-            raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
-        if pI.maxLevel != pJ.maxLevel:
-            raise error("calcOpticalFlowPyrLK: pyramids differ in depth")
-    else:
-        # (H,W,C) u8 frames, C = 2..4 (cv2 takes 3-channel frames; the reference converts to gray first, s1:311): one
-        # single-channel pyramid per channel plane, window sums taken over pixels and channels
-        if cn > 4:
-            raise error("calcOpticalFlowPyrLK: at most 4 channels")
-        a = _to_dev(prevImg, np.uint8, "calcOpticalFlowPyrLK prevImg")
-        b = _to_dev(nextImg, np.uint8, "calcOpticalFlowPyrLK nextImg")
-        if tuple(a.shape) != tuple(b.shape):
-            raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
-        pI = [FramePyramid(a[..., c].contiguous(), w, maxLevel, True) for c in range(cn)]
-        pJ = [FramePyramid(b[..., c].contiguous(), w, maxLevel, False) for c in range(cn)]
+    # (H,W,C) u8 frames, C = 2..4 (cv2 takes 3-channel frames; the reference converts to gray first, s1:311): one pyramid per
+    # channel plane, window sums taken over pixels and channels
+    pI = _as_pyramid(prevImg, w, maxLevel, True, "calcOpticalFlowPyrLK prevImg")
+    pJ = _as_pyramid(nextImg, w, maxLevel, False, "calcOpticalFlowPyrLK nextImg")
+    if pI.sizes[0] != pJ.sizes[0]:
+        raise error("calcOpticalFlowPyrLK: prevImg and nextImg differ in size")
+    if pI.maxLevel != pJ.maxLevel:
+        raise error("calcOpticalFlowPyrLK: pyramids differ in depth")
     flags = int(flags)
     if flags & OPTFLOW_USE_INITIAL_FLOW:
         if nextPts is None:
@@ -322,10 +392,7 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
         N.check(N.lib().ibt_lk(C.byref(pI.c), C.byref(pJ.c), _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps,
                                float(minEigThreshold), flags, _ptr(st), _ptr(err), _ptr(iters), _stream()), "ibt_lk")
     else:
-        PP = C.POINTER(N.ibt_pyramid_t)
-        arrI = (PP * cn)(*[C.pointer(p.c) for p in pI])
-        arrJ = (PP * cn)(*[C.pointer(p.c) for p in pJ])
-        N.check(N.lib().ibt_lk_multichannel(arrI, arrJ, cn, _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps, float(minEigThreshold),
+        N.check(N.lib().ibt_lk_multichannel(pI.chan_ptrs, pJ.chan_ptrs, cn, _ptr(pts), _ptr(nxt), n, w[0], w[1], cnt, eps, float(minEigThreshold),
                                             flags, _ptr(st), _ptr(err), _ptr(iters), _stream()), "ibt_lk_multichannel")
     res = (_out(nxt.reshape(shp), as_np), _out(st.reshape(n, 1), as_np), _out(err.reshape(n, 1), as_np))
     return res + ((_out(iters, as_np),) if return_iters else ())
@@ -334,7 +401,7 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
 def calcOpticalFlowPyrLK_FB(prev, next, p0, winSize=(21, 21), maxLevel=3,
                             criteria=(TERM_CRITERIA_COUNT | TERM_CRITERIA_EPS, 30, 0.01), minEigThreshold=1e-4,
                             fb_threshold=1.0, alive=None, iter_total=None, return_iters=False):
-    """The reference's whole per-pair block in one launch (s1:323-333):
+    """The reference's whole per-pair block in one launch (s1:323-333), on gray or (H,W,C) frames (C = 2..4) or FramePyramids:
         p1, st, err  = calcOpticalFlowPyrLK(prev, next, p0, None, **lk_params)
         p0r, st, err = calcOpticalFlowPyrLK(next, prev, p1, None, **lk_params)
         dist = hypot(|p0 - p0r|); valid = dist < 1
@@ -352,6 +419,8 @@ def calcOpticalFlowPyrLK_FB(prev, next, p0, winSize=(21, 21), maxLevel=3,
     pB = _as_pyramid(next, w, maxLevel, True, "calcOpticalFlowPyrLK_FB next")
     if pA.sizes != pB.sizes:
         raise error("calcOpticalFlowPyrLK_FB: prev and next differ in size")
+    if pA.cn != pB.cn:
+        raise error("calcOpticalFlowPyrLK_FB: prev and next differ in the number of channels")
     cnt, eps = _criteria(criteria)
     dev = pts.device
     f32 = lambda *s: torch.empty(s, dtype=torch.float32, device=dev)
@@ -362,9 +431,12 @@ def calcOpticalFlowPyrLK_FB(prev, next, p0, winSize=(21, 21), maxLevel=3,
     if own_alive:
         alive = torch.ones((n,), dtype=torch.uint8, device=dev)
     iters = torch.zeros((n, 2), dtype=torch.int32, device=dev) if return_iters else None
-    N.check(N.lib().ibt_lk_fb(C.byref(pA.c), C.byref(pB.c), _ptr(pts), n, w[0], w[1], cnt, eps, float(minEigThreshold),
-                              float(fb_threshold), _ptr(p1), _ptr(st1), _ptr(err1), _ptr(p0r), _ptr(st0), _ptr(err0),
-                              _ptr(dist), _ptr(alive), _ptr(iters), _ptr(iter_total), _stream()), "ibt_lk_fb")
+    tail = (_ptr(pts), n, w[0], w[1], cnt, eps, float(minEigThreshold), float(fb_threshold), _ptr(p1), _ptr(st1), _ptr(err1),
+            _ptr(p0r), _ptr(st0), _ptr(err0), _ptr(dist), _ptr(alive), _ptr(iters), _ptr(iter_total), _stream())
+    if pA.cn == 1:
+        N.check(N.lib().ibt_lk_fb(C.byref(pA.c), C.byref(pB.c), *tail), "ibt_lk_fb")
+    else:
+        N.check(N.lib().ibt_lk_fb_multichannel(pA.chan_ptrs, pB.chan_ptrs, pA.cn, *tail), "ibt_lk_fb_multichannel")
     r = dict(p1=_out(p1.reshape(shp), as_np), st1=_out(st1.reshape(n, 1), as_np), err1=_out(err1.reshape(n, 1), as_np),
              p0r=_out(p0r.reshape(shp), as_np), st0=_out(st0.reshape(n, 1), as_np), err0=_out(err0.reshape(n, 1), as_np),
              dist=_out(dist, as_np), valid=_out(alive.bool(), as_np))

@@ -84,6 +84,20 @@ typedef struct ibt_pyramid {
  * the Scharr planes. */
 int ibt_pyramid_build(const ibt_pyramid_t *pyr, int with_derivs, void *stream);
 
+/* Whole pyramids of one multi-channel frame (cv2.buildOpticalFlowPyramid / calcOpticalFlowPyrLK on an (H,W,cn) u8 frame):
+ * frame (H,W,cn) u8 interleaved, row pitch frame_pitch >= W*cn bytes, any pitch and any alignment; cn 2..4.  pyr is a HOST
+ * array of cn pyramid pointers, one per channel plane, all with the same nlevels, rows and cols.  Unlike ibt_pyramid_build,
+ * pyr[c]->img[0] is an OUTPUT: channel c's level-0 plane, de-interleaved from the frame; pyr[c]->img[1..] and
+ * pyr[c]->deriv[0..] are caller-allocated outputs as there.  For every channel the result is ibt_pyramid_build of that
+ * channel's plane, which is what OpenCV builds for a multi-channel frame (level l of channel c = the gray pyramid of plane c;
+ * OpenCV's derivative channels 2c, 2c+1 = its Scharr (dx, dy)).  One launch reads the frame once and writes every channel's
+ * level 0, Scharr planes and level 1; each further level of all channels is one launch.  16-byte aligned frames (base and
+ * pitch) are staged by 16-byte copies, any other frame (e.g. a crop view) by a byte gather; the planes take the vector paths
+ * of ibt_pyramid_build with 16-byte aligned rows (the LK solver's staging wants 128-byte pitches).  Invalid arguments (cn,
+ * null pointers, geometry that differs between channels or levels, a bad pitch) return IBT_E_INVALID before any CUDA call. */
+int ibt_pyramid_build_multichannel(const uint8_t *frame, int64_t frame_pitch, int cn, const ibt_pyramid_t *const *pyr,
+                                   int with_derivs, void *stream);
+
 /* ---- K3: cv2.calcOpticalFlowPyrLK(img0, img1, p0, None, **lk_params)  s1:323 (forward),
  *      s1:326 (backward); s0_1:92,95.  One pass, I = pyrI (needs deriv), J = pyrJ.
  *      pts (N,2) f32; next_pts (N,2) f32 out (in/out with IBT_LK_USE_INITIAL_FLOW);
@@ -122,6 +136,17 @@ int ibt_lk_multichannel(const ibt_pyramid_t *const *pyrI, const ibt_pyramid_t *c
                         const float *pts, float *next_pts, int N,
                         int winW, int winH, int max_count, double epsilon, double min_eig_threshold, int flags,
                         uint8_t *status, float *err, int32_t *iters, void *stream);
+/* ibt_lk_fb on multi-channel frames: prev / next are HOST arrays of cn (2..4) channel pyramids as in ibt_lk_multichannel, and
+ * BOTH need Scharr planes (the backward pass tracks next -> prev).  Forward, backward and the forward-backward check run in one
+ * launch with ibt_lk_fb's arguments and outputs; each pass equals ibt_lk_multichannel in that direction. */
+int ibt_lk_fb_multichannel(const ibt_pyramid_t *const *prev, const ibt_pyramid_t *const *next, int cn,
+                           const float *p0, int N,
+                           int winW, int winH, int max_count, double epsilon, double min_eig_threshold,
+                           float fb_threshold,
+                           float *p1, uint8_t *st1, float *err1,
+                           float *p0r, uint8_t *st0, float *err0,
+                           float *fbdist, uint8_t *alive, int32_t *iters, unsigned long long *iter_total,
+                           void *stream);
 /* Process-wide occupancy cap of the persistent LK launches: at most `ctas` resident CTAs (of 8 warps) per SM, 0 = fill the SM
  * (default, 3 for the usual window sizes).  With 2 the launch leaves a third of every SM's shared memory and registers to
  * kernels of other streams -- e.g. the JPEG decode of the next frame (measured: LK 7 % slower, decode fully overlapped). */
