@@ -117,6 +117,12 @@ __device__ __forceinline__ long long warp_sum_wide(int v)
 }
 
 __device__ __forceinline__ int cv_floor(float v) { return __float2int_rd(v); }
+// OpenCV's cvFloor gives INT_MIN for NaN on x86, so cv2 finds the window of a NaN point or guess out of bounds at every level
+// (status 0, err 0, nextPts = the propagated input).  PTX converts NaN to 0, which would put that window at the origin.  The
+// coordinates that can be NaN -- the point and the guess at each level, the final position -- pass through no_nan before they
+// are floored (-inf floors to INT_MIN); the Newton iterates of a finite guess stay finite, so the iteration loop needs no test.
+// +-inf and |v| >= 2^31 saturate to INT_MIN / INT_MAX (INT_MIN on x86): out of bounds either way.
+__device__ __forceinline__ float no_nan(float v) { return v == v ? v : __int_as_float(0xff800000); }
 
 // d = c + a.lo16 * b.byte0 + a.hi16 * b.byte1 (.lo) / b.byte2, b.byte3 (.hi) with SIGNED 16-bit weights (iw11 = 2^14 - iw00 -
 // iw01 - iw10 can be -1 after rounding) and UNSIGNED pixel bytes.
@@ -603,12 +609,12 @@ __device__ __forceinline__ void lk_point(const LKPyr *PI, const LKPyr *PJ, int c
         ox = nx; oy = ny;
 
         ppx = __fsub_rn(ppx, halfx); ppy = __fsub_rn(ppy, halfy);
-        const int ipx = cv_floor(ppx), ipy = cv_floor(ppy);
+        const int ipx = cv_floor(no_nan(ppx)), ipy = cv_floor(no_nan(ppy));
         if (window_oob(ipx, ipy, winW, winH, rows, cols)) {
             if (level == 0) { status = 0; err = 0.f; }
             continue;
         }
-        nx = __fsub_rn(nx, halfx); ny = __fsub_rn(ny, halfy);
+        nx = no_nan(__fsub_rn(nx, halfx)); ny = no_nan(__fsub_rn(ny, halfy));      // (ox, oy) keep a NaN guess
 
         // ---- one burst of async copies: I window + its Scharr planes (barrier / group 0), J search patch (1) -------------
         // TMA where the level has tensor maps and the patch needs no reflection (bulk tensor copies zero-fill outside the
@@ -727,7 +733,7 @@ __device__ __forceinline__ void lk_point(const LKPyr *PI, const LKPyr *PJ, int c
         // The reference never reads status or err (s1:323-333): callers that pass no status / err buffers skip the stage.
         if (status && level == 0 && !(a.flags & IBT_LK_GET_MIN_EIGENVALS) && (want_status || want_err)) {
             const float qx = __fsub_rn(ox, halfx), qy = __fsub_rn(oy, halfy);
-            const int iqx = cv_floor(qx), iqy = cv_floor(qy);
+            const int iqx = cv_floor(no_nan(qx)), iqy = cv_floor(no_nan(qy));
             if (window_oob(iqx, iqy, winW, winH, rows, cols)) { status = 0; err = 0.f; continue; }
             if (!want_err) continue;
             if (!staged || (unsigned)(iqx - vx0) > 2u * LK_MARGIN || (unsigned)(iqy - py0) > 2u * LK_MARGIN) {

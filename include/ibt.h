@@ -104,7 +104,11 @@ int ibt_pyramid_build_multichannel(const uint8_t *frame, int64_t frame_pitch, in
  *      status (N) u8; err (N) f32 (0 where status == 0; cv2 leaves garbage there);
  *      iters (N) i32 or NULL: inner Newton iterations executed, summed over levels.
  *      max_count/epsilon are the TERM_CRITERIA values after cv2's defaults were applied
- *      (clamped here to [0,100] / [0,10] like cv2). */
+ *      (clamped here to [0,100] / [0,10] like cv2).
+ *      Non-finite points (NaN or +-inf in x or y) and points beyond +-2^31 px put the window out of bounds at every
+ *      level, as cv2 does on x86: status 0, err 0, no iterations, and next_pts = the input (or the initial flow)
+ *      scaled to the top level and back.  A NaN initial flow gives status 0 with no iterations (err = the level-0
+ *      minimum eigenvalue with IBT_LK_GET_MIN_EIGENVALS, else 0).  ibt_lk_fb reports such points as not valid. */
 int ibt_lk(const ibt_pyramid_t *pyrI, const ibt_pyramid_t *pyrJ,
            const float *pts, float *next_pts, int N,
            int winW, int winH, int max_count, double epsilon, double min_eig_threshold, int flags,

@@ -43,6 +43,62 @@ def assert_lk_parity(p_a, st_a, p_b, st_b, what=""):
     return agree, frac, mx
 
 
+def _f32_same(a, b):
+    """element-wise: same float32 bytes, or NaN on both sides (the GPU returns the canonical NaN, x86 keeps the payload)"""
+    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
+    return (a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))
+
+
+def _lk_n(ref):
+    return np.asarray(ref["st"]).size if "st" in ref else np.asarray(ref["p1"]).size // 2
+
+
+def lk_exact_mismatch(gpu, ref):
+    """gpu / ref: dicts with any of p1 (N,2) f32, st (N,) u8, err (N,) f32, iters (N,) or per level (N, L) int.  -> bool (N,),
+    True where the two differ in any of the keys both hold.  The CUDA solver and the oracle sum the same exact integers and
+    round the same float steps, so there is no tolerance: p1 and err by bytes, status and the iteration counts equal."""
+    n = _lk_n(ref)
+    bad = np.zeros(n, bool)
+    for k in ("p1", "st", "err", "iters"):
+        if k not in gpu or k not in ref:
+            continue
+        g, r = np.asarray(gpu[k]), np.asarray(ref[k])
+        if k == "p1":
+            bad |= ~_f32_same(g.reshape(n, 2), r.reshape(n, 2)).all(1)
+        elif k == "err":
+            bad |= ~_f32_same(g.reshape(n), r.reshape(n))
+        elif k == "iters":
+            bad |= g.reshape(n, -1).sum(1) != r.reshape(n, -1).sum(1)
+        else:
+            bad |= g.reshape(n) != r.reshape(n)
+    return bad
+
+
+def assert_lk_exact(gpu, ref, what="", pts=None, guess=None, show=6):
+    """Exact agreement of a CUDA LK result with the oracle's (lk_exact_mismatch).  A failure lists the first `show`
+    mismatching points with their input, initial guess and both sides' outputs; `what` names the case (sizes, parameters)."""
+    bad = np.flatnonzero(lk_exact_mismatch(gpu, ref))
+    if not len(bad):
+        return
+    lines = []
+    for i in bad[:show]:
+        s = "  #%d" % i
+        if pts is not None:
+            s += " pt %r" % (np.asarray(pts, np.float32).reshape(-1, 2)[i].tolist(),)
+        if guess is not None:
+            s += " guess %r" % (np.asarray(guess, np.float32).reshape(-1, 2)[i].tolist(),)
+        for k in ("p1", "st", "err", "iters"):
+            if k in gpu and k in ref:
+                r = np.asarray(ref[k])
+                g, r = np.asarray(gpu[k]).reshape(r.shape[0], -1)[i], r.reshape(r.shape[0], -1)[i]
+                if k == "iters":
+                    g, r = g.sum(), r.sum()
+                s += " | %s gpu %r oracle %r" % (k, np.asarray(g).tolist(), np.asarray(r).tolist())
+        lines.append(s)
+    n = _lk_n(ref)
+    raise AssertionError("%s: %d of %d points differ from the oracle\n%s" % (what, len(bad), n, "\n".join(lines)))
+
+
 def corner_overlap(a, b):
     """|A n B| / max(|A|, |B|) over integer (x, y) corner sets; None counts as empty."""
     sa = set() if a is None else set(map(tuple, np.asarray(a).reshape(-1, 2).astype(np.int64).tolist()))

@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 import torch
 
-from parity import CORNER_OVERLAP, as_corners, assert_lk_parity, corner_overlap
+from parity import CORNER_OVERLAP, as_corners, assert_lk_exact, assert_lk_parity, corner_overlap
 
 pytestmark = pytest.mark.gpu
 
@@ -358,17 +358,15 @@ def test_lk_layout_invariance(ibt, oracle, lk_scene, win):
         lv = [S["planes"][c] for c in range(LK_CN)]
         crit = dict(winSize=win, maxLevel=maxLevel, criteria=(3, 30, 0.01))
         for flags in (0, INIT, MINEIG):
-            g = canon["lk", flags]
-            po, so, eo = oracle.calcOpticalFlowPyrLK(lv[0][0], lv[0][1], S["pts"], S["guess"], flags=flags, **crit)
-            assert_lk_parity(g["p1"], g["st"], po, so, "%s ml %d flags %d" % (win, maxLevel, flags))
-            if flags == MINEIG:
-                ok = (g["st"] == 1) & (so.ravel() == 1)
-                assert np.abs(g["err"][ok] - eo.ravel()[ok]).max(initial=0) <= 1e-5 * max(1.0, np.abs(eo).max())
+            po, so, eo, io = oracle.calcOpticalFlowPyrLK(lv[0][0], lv[0][1], S["pts"], S["guess"], flags=flags, return_iters=True,
+                                                        **crit)
+            assert_lk_exact(canon["lk", flags], dict(p1=po, st=so, err=eo, iters=io), "%s ml %d flags %d" % (win, maxLevel, flags),
+                            S["pts"], S["guess"] if flags & INIT else None)
         fb = canon["fb"]
         assert _same(fb["p1"], canon["lk", 0]["p1"]) and _same(fb["st1"], canon["lk", 0]["st"])
         stack = lambda k: np.stack([lv[c][k] for c in range(2)], -1)
-        po, so, _ = oracle.calcOpticalFlowPyrLK(stack(0), stack(1), S["pts"], None, **crit)
-        assert_lk_parity(canon["mc2"]["p1"], canon["mc2"]["st"], po, so, "%s ml %d cn 2" % (win, maxLevel))
+        po, so, eo, io = oracle.calcOpticalFlowPyrLK(stack(0), stack(1), S["pts"], None, return_iters=True, **crit)
+        assert_lk_exact(canon["mc2"], dict(p1=po, st=so, err=eo, iters=io), "%s ml %d cn 2" % (win, maxLevel), S["pts"])
         st = canon["lk", 0]["st"]
         assert 0 < st.sum() < len(st), (win, maxLevel)          # both outcomes occur: the border cases are exercised
 
@@ -672,18 +670,20 @@ def test_lk_int32_headroom(ibt, oracle):
         pts = _hr_points(win)
         for maxLevel in (0, 2):
             lp = dict(winSize=win, maxLevel=maxLevel, criteria=(3, 30, 0.01))
-            p1, st, err = ibt.calcOpticalFlowPyrLK(I, J, pts, None, **lp)
-            po, so, eo = oracle.calcOpticalFlowPyrLK(I, J, pts, None, **lp)
-            assert_lk_parity(p1, st, po, so, "headroom %s ml %d" % (win, maxLevel))
+            p1, st, err, it = ibt.calcOpticalFlowPyrLK(I, J, pts, None, return_iters=True, **lp)
+            po, so, eo, io = oracle.calcOpticalFlowPyrLK(I, J, pts, None, return_iters=True, **lp)
+            assert_lk_exact(dict(p1=p1, st=st, err=err, iters=it), dict(p1=po, st=so, err=eo, iters=io),
+                            "headroom %s ml %d" % (win, maxLevel), pts)
             assert st.all(), (win, maxLevel)
             if cv2 is not None:
                 pc, sc, _ = cv2.calcOpticalFlowPyrLK(I, J, pts.reshape(-1, 1, 2), None, **lp)
                 assert_lk_parity(p1, st, pc, sc, "headroom vs cv2 %s ml %d" % (win, maxLevel))
             # the same scene as 4 identical channel planes
             I4, J4 = np.repeat(I[..., None], 4, -1), np.repeat(J[..., None], 4, -1)
-            q1, qs, _ = ibt.calcOpticalFlowPyrLK(I4, J4, pts, None, **lp)
-            qo, qso, _ = oracle.calcOpticalFlowPyrLK(I4, J4, pts, None, **lp)
-            assert_lk_parity(q1, qs, qo, qso, "headroom 4 channels %s ml %d" % (win, maxLevel))
+            q1, qs, qe, qi = ibt.calcOpticalFlowPyrLK(I4, J4, pts, None, return_iters=True, **lp)
+            qo, qso, qeo, qio = oracle.calcOpticalFlowPyrLK(I4, J4, pts, None, return_iters=True, **lp)
+            assert_lk_exact(dict(p1=q1, st=qs, err=qe, iters=qi), dict(p1=qo, st=qso, err=qeo, iters=qio),
+                            "headroom 4 channels %s ml %d" % (win, maxLevel), pts)
         # min eigenvalue at level 0: err with GET_MIN_EIGENVALS, against the int64 restatement
         _, _, err = ibt.calcOpticalFlowPyrLK(I, J, pts, None, winSize=win, maxLevel=0, flags=MINEIG)
         for k, pt in enumerate(pts):

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from parity import (GFTT_SETS, LK_SETS, ERR_TOL, CORNER_OVERLAP, assert_lk_parity, as_corners, corner_overlap)
+from parity import (GFTT_SETS, LK_SETS, ERR_TOL, CORNER_OVERLAP, assert_lk_exact, assert_lk_parity, as_corners, corner_overlap)
 
 pytestmark = pytest.mark.gpu
 SCENES = ["kat_texture.npz", "kat_iceberg.npz"]
@@ -179,11 +179,12 @@ def test_config1_vs_oracle(ibt, oracle):
     assert pts is not None and len(pts) == 2000
     p1, st, err, it = ibt.calcOpticalFlowPyrLK(f0, f1, pts, None, return_iters=True, **lp)
     p1_o, st_o, err_o, it_o = oracle.calcOpticalFlowPyrLK(f0, f1, pts, None, return_iters=True, **lp)
-    agree, frac, mx = assert_lk_parity(p1, st, p1_o, st_o, "config 1 fwd")
-    assert np.mean(it == it_o.sum(1)) >= 0.99          # the BASELINE unit (feature-pair-iterations) counts the same
-    p0r, st0, _ = ibt.calcOpticalFlowPyrLK(f1, f0, p1, None, **lp)
-    p0r_o, st0_o, _ = oracle.calcOpticalFlowPyrLK(f1, f0, p1, None, **lp)
-    assert_lk_parity(p0r, st0, p0r_o, st0_o, "config 1 bwd")
+    # exact, iterations too: the BASELINE unit (feature-pair-iterations) counts the same on every point
+    assert_lk_exact(dict(p1=p1, st=st, err=err, iters=it), dict(p1=p1_o, st=st_o, err=err_o, iters=it_o), "config 1 fwd", pts)
+    p0r, st0, err0, it0 = ibt.calcOpticalFlowPyrLK(f1, f0, p1, None, return_iters=True, **lp)
+    p0r_o, st0_o, err0_o, it0_o = oracle.calcOpticalFlowPyrLK(f1, f0, p1, None, return_iters=True, **lp)
+    assert_lk_exact(dict(p1=p0r, st=st0, err=err0, iters=it0), dict(p1=p0r_o, st=st0_o, err=err0_o, iters=it0_o),
+                    "config 1 bwd", p1)
     # the synthetic shift is known: tracked displacement == (-VX, -VY) content motion seen from the camera
     d = (p1 - pts).reshape(-1, 2)[st.reshape(-1) == 1]
     assert np.abs(np.median(d, 0) - [-syn.VX, -syn.VY]).max() < 0.05
