@@ -124,6 +124,17 @@ __device__ __forceinline__ int cv_floor(float v) { return __float2int_rd(v); }
 // +-inf and |v| >= 2^31 saturate to INT_MIN / INT_MAX (INT_MIN on x86): out of bounds either way.
 __device__ __forceinline__ float no_nan(float v) { return v == v ? v : __int_as_float(0xff800000); }
 
+// The FB distance as numpy's float32 hypot computes it (s1:330): glibc's hypotf, the double square root of the exact double
+// sum of squares rounded to float, and +inf if either input is infinite even when the other is NaN (the sum alone would
+// give NaN there; a NaN otherwise propagates).  CUDA's hypotf differs in the last bit, and dist < fb_thresh and the
+// trackquality files rest on these bits.
+__device__ __forceinline__ float glibc_hypotf(float x, float y)
+{
+    if (isinf(x) || isinf(y)) return __int_as_float(0x7f800000);
+    const double a = x, b = y;
+    return __double2float_rn(__dsqrt_rn(__dadd_rn(__dmul_rn(a, a), __dmul_rn(b, b))));
+}
+
 // d = c + a.lo16 * b.byte0 + a.hi16 * b.byte1 (.lo) / b.byte2, b.byte3 (.hi) with SIGNED 16-bit weights (iw11 = 2^14 - iw00 -
 // iw01 - iw10 can be -1 after rounding) and UNSIGNED pixel bytes.
 __device__ __forceinline__ uint32_t dp2a_lo(uint32_t a, uint32_t b, uint32_t c)
@@ -814,7 +825,7 @@ lk_kernel(const __grid_constant__ LKArgs a, const __grid_constant__ LKFrames<CN>
                 if (a.p0r) { a.p0r[2 * k] = ox; a.p0r[2 * k + 1] = oy; }
                 if (a.st0) a.st0[k] = (uint8_t)status;
                 if (a.err0) a.err0[k] = err;
-                const float d = hypotf(fabsf(__fsub_rn(p0x, ox)), fabsf(__fsub_rn(p0y, oy)));
+                const float d = glibc_hypotf(fabsf(__fsub_rn(p0x, ox)), fabsf(__fsub_rn(p0y, oy)));
                 if (a.fbdist) a.fbdist[k] = d;
                 if (a.alive) a.alive[k] = (d < a.fb_thresh) ? 1 : 0;
             }

@@ -49,6 +49,45 @@ __device__ __forceinline__ double2 project(const UtmCam &c, float2 p)
                         c.Hc * (c.sX1 + xi * c.U1 + yi * c.V1) / den + c.N0);
 }
 
+// numpy's float64 hypot (s2:286, 328) as glibc >= 2.35 computes it without FMA: Borges, "An Improved Algorithm for
+// hypot(a, b)" (arXiv:1904.09481), restated operation for operation (tests/test_libm_restatements.py pins it on the host's
+// libm).  It is not correctly rounded, and CUDA's hypot rounds differently, so the speeds written to the hourly files and
+// compared with min_speed, max_speed and speed_threshold would differ from numpy's in the last bit.
+__device__ __forceinline__ double glibc_hypot_kernel(double ax, double ay)         // ax >= ay >= 0, squares in range
+{
+    double h = __dsqrt_rn(__dadd_rn(__dmul_rn(ax, ax), __dmul_rn(ay, ay)));
+    double t1, t2;
+    if (h <= __dmul_rn(2.0, ay)) {
+        const double d = __dsub_rn(h, ay);
+        t1 = __dmul_rn(ax, __dsub_rn(__dmul_rn(2.0, d), ax));
+        t2 = __dmul_rn(__dsub_rn(d, __dmul_rn(2.0, __dsub_rn(ax, ay))), d);
+    } else {
+        const double d = __dsub_rn(h, ax);
+        t1 = __dmul_rn(__dmul_rn(2.0, d), __dsub_rn(ax, __dmul_rn(2.0, ay)));
+        t2 = __dadd_rn(__dmul_rn(__dsub_rn(__dmul_rn(4.0, d), ay), ay), __dmul_rn(d, d));
+    }
+    return __dsub_rn(h, __ddiv_rn(__dadd_rn(t1, t2), __dmul_rn(2.0, h)));
+}
+
+__device__ double glibc_hypot(double x, double y)
+{
+    constexpr double kScale = 0x1p-600, kLarge = 0x1p+511, kTiny = 0x1p-459, kEps = 0x1p-54;
+    if (isinf(x) || isinf(y)) return __longlong_as_double(0x7ff0000000000000ll);
+    if (isnan(x) || isnan(y)) return __dadd_rn(x, y);
+    x = fabs(x); y = fabs(y);
+    const double ax = x < y ? y : x, ay = x < y ? x : y;
+    if (ax > kLarge) {                                   // scale down: the squares would overflow
+        if (ay <= __dmul_rn(ax, kEps)) return __dadd_rn(ax, ay);
+        return __ddiv_rn(glibc_hypot_kernel(__dmul_rn(ax, kScale), __dmul_rn(ay, kScale)), kScale);
+    }
+    if (ay < kTiny) {                                    // scale up: the correction terms would underflow
+        if (ax >= __ddiv_rn(ay, kEps)) return __dadd_rn(ax, ay);
+        return __dmul_rn(glibc_hypot_kernel(__ddiv_rn(ax, kScale), __ddiv_rn(ay, kScale)), kScale);
+    }
+    if (ay <= __dmul_rn(ax, kEps)) return __dadd_rn(ax, ay);
+    return glibc_hypot_kernel(ax, ay);
+}
+
 // np.mean(speedsublist) (s2:310) sums with numpy's pairwise scheme (loops_utils.h.src @TYPE@_pairwise_sum): sequential below 8
 // elements, 8 accumulators up to 128, recursive halving above.  A borderline mean < min_speed decision follows numpy's bits.
 __device__ double np_sum_block(const double *v, int n)
@@ -95,7 +134,7 @@ track_velocities_kernel(const __grid_constant__ VelArgs a)
         const double2 cur = project(a.cam, tr[i]);
         en[i] = cur;
         const double u = (cur.x - prev.x) / a.interval, v = (cur.y - prev.y) / a.interval;     // s2:284-285
-        const double s = hypot(u, v);                                                           // s2:286
+        const double s = glibc_hypot(u, v);                                                     // s2:286
         uv[i - 1] = make_double2(u, v);
         sp[i - 1] = s;
         if (i == 1 || s > smax) smax = s;
@@ -108,7 +147,7 @@ track_velocities_kernel(const __grid_constant__ VelArgs a)
         for (int c1 = 0; c1 + 1 < T; c1++) {
             const double2 a1 = uv[c1], a2 = uv[c1 + 1];
             const double dot = a1.x * a2.x + a1.y * a2.y;
-            const double mag1 = hypot(a1.x, a1.y), mag2 = hypot(a2.x, a2.y);
+            const double mag1 = glibc_hypot(a1.x, a1.y), mag2 = glibc_hypot(a2.x, a2.y);
             const double ang = fabs(acos(dot / (mag1 * mag2)) * (180.0 / 3.14159265358979323846));   // s2:327-329
             const double s1 = sp[c1], s2 = sp[c1 + 1];
             const double hi = (s2 > s1) ? s2 : s1;                    // max([s1, s2])
