@@ -74,6 +74,10 @@ SIGNATURES = {
     "ibt_gftt_ksize": (_i, [_vp, _i64, _vp, _i64, _i, _i, _i, _d, _d, _i, _i, _i, _d, _vp, _sz, _vp, _i, C.POINTER(C.c_int),
                             _vp]),
     "ibt_gftt_async_ksize": (_i, [_vp, _i64, _vp, _i64, _i, _i, _i, _d, _d, _i, _i, _i, _d, _vp, _sz, _vp, _i, _vp, _vp]),
+    "ibt_gftt_f32src": (_i, [_vp, _i64, _vp, _i64, _i, _i, _i, _d, _d, _i, _i, _i, _d, _vp, _sz, _vp, _i, C.POINTER(C.c_int),
+                             _vp]),
+    "ibt_min_eigen_f32src": (_i, [_vp, _i, _i, _i64, _i, _i, _vp, _i64, _vp]),
+    "ibt_corner_harris_f32src": (_i, [_vp, _i, _i, _i64, _i, _i, _d, _vp, _i64, _vp]),
     "ibt_tracks_compact": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, C.POINTER(C.c_int), _vp]),
     "ibt_tracks_compact_async": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "ibt_photo_to_utm": (_i, [_vp, _i64, C.POINTER(C.c_double), _vp, _vp]),

@@ -14,7 +14,7 @@ void set_last_error(cudaError_t e, const char *where)
 
 } // namespace ibt
 
-IBT_API int ibt_version(void) { return 103; }     /* major * 100 + minor */
+IBT_API int ibt_version(void) { return 104; }     /* major * 100 + minor */
 
 IBT_API const char *ibt_error_string(int code)
 {

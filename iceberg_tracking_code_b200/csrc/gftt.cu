@@ -25,6 +25,7 @@
 //   ibt_min_eigen_f32    (cornerMinEigenVal test hook) keeps the map-writing eig_kernel.
 //   cv2's other Sobel apertures (gradientSize / ksize = -1, 1, 5, 7) take eig_nms_ap_kernel / eig_ap_kernel in place of K2a /
 //   eig_kernel (table and int64 bound at eig_ap_kernel); K2b is the same.
+//   float32 images take eig_f32_kernel (every aperture; the fused K2a and the map hooks); K2b is the same.
 #include "common.cuh"
 #include <atomic>
 #include <float.h>
@@ -930,6 +931,372 @@ static int launch_eig_nms(const uint8_t *gray, int H, int W, int64_t pitch, int 
 }
 
 // ---------------------------------------------------------------------------------------------
+// float32 images (cv2 takes CV_8UC1 and CV_32FC1): eig_f32_kernel, one body for every aperture, both responses, the fused
+// K2a (raw 3x3 maxima as keys for K2b) and the map hooks (MAP: the response map is written instead).  eig_nms_ap_job's warp /
+// strip structure, with OpenCV's CV_32F front end: Sobel / Scharr in float with the scale 1 / (sden * blockSize) (no 255) on
+// the smoothing taps (cv2's Sobel scales the smoothing kernel; taps rounded to float as its float kernels are), the
+// derivative taps of a row first, then the column taps; float products; window sums in double; the float response.
+//   - Inner strips load four floats per lane (16 bytes: image pointer and pitch multiples of 16), border strips (and every
+//     strip of a less aligned image) gather.  Zero taps are skipped, so a NaN / inf pixel reaches the pixels cv2's does.
+//   - The window sums are not cv2's running sums: each pixel adds its bs x bs products in a fixed order (rows of a column
+//     first, then the columns), so its value depends on its window only -- the map hooks and goodFeaturesToTrack compute the
+//     same bits, whatever the job split.  cv2's running double sums differ from these by rounding (bound in tests/f32_cases.py).
+//   - A non-finite response (a NaN / inf pixel, or products beyond float range) sets GfttCounters.error to IBT_E_UNSUPPORTED:
+//     goodFeaturesToTrack refuses the image rather than return corners derived from it.  The map hooks write NaN / inf.
+struct EigF32Args {
+    EigNmsArgs n;             // geometry, mask, counters and keys of the fused kernel (n.img unused)
+    const float *img; int64_t pitch_f;
+    float ss[7];              // smoothing taps * scale, rounded to float (the taps of the Sobel's smoothing direction)
+    float *map; int64_t map_pitch_f;     // MAP instantiations
+};
+
+template <int G>
+__device__ __forceinline__ void f32_taps_vec(float4 w4, const float *ss, float *hd, float *hs)
+{
+    constexpr int KT = ap_taps(G), R = KT / 2;
+    const float w[4] = {w4.x, w4.y, w4.z, w4.w};
+    float b[4 + 2 * R];                                            // columns c0 - R .. c0 + 3 + R (neighbour lanes' floats)
+#pragma unroll
+    for (int i = 0; i < 4 + 2 * R; i++) {
+        const int rel = i - R;
+        const float v = w[(rel + 4) & 3];
+        b[i] = rel < 0 ? __shfl_up_sync(0xffffffffu, v, 1) : rel < 4 ? v : __shfl_down_sync(0xffffffffu, v, 1);
+    }
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        float d = 0.f, s = 0.f;
+#pragma unroll
+        for (int j = 0; j < KT; j++) {
+            if (ap_d(G, j) != 0) d = __fadd_rn(d, __fmul_rn((float)ap_d(G, j), b[k + j]));
+            if (ap_s(G, j) != 0) s = __fadd_rn(s, __fmul_rn(ss[j], b[k + j]));
+        }
+        hd[k] = d; hs[k] = s;
+    }
+}
+
+template <int G, bool MASK, bool BORDER, bool HARRIS, bool MAP>
+__device__ __forceinline__ void eig_f32_job(const EigF32Args &f, int strip, int Y0, int Y1, int *wsm, int lane)
+{
+    constexpr int KT = ap_taps(G), R = KT / 2;
+    const EigNmsArgs &a = f.n;
+    const int bs = a.bs;
+    const int a0 = -(bs / 2);
+    const int H = a.H, W = a.W;
+    const int ox0 = strip * a.outw;
+    const int c0 = ox0 - a.left + 4 * lane;
+    const int ey0 = max(0, Y0 - 1), ey1 = min(H - 1, Y1);
+    float *ring = reinterpret_cast<float *>(wsm);                 // [bs][128][2]: (dx, dy) of the last bs product rows
+    unsigned long long *cbuf = reinterpret_cast<unsigned long long *>(wsm + bs * 2 * EN_COLS);
+    int *scount = reinterpret_cast<int *>(cbuf + EN_CB);
+    double *rowbuf = reinterpret_cast<double *>(scount + 4);      // [EN_PAD + 128 + EN_PAD]
+    float ss[KT];
+#pragma unroll
+    for (int j = 0; j < KT; j++) ss[j] = f.ss[j];
+    unsigned outmask = 0, candmask = 0;
+    int cx[4][KT];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const int c = c0 + k;
+        const bool own = c >= ox0 && c < ox0 + a.outw && c < W;
+        if (own) outmask |= 1u << k;
+        if (own && c >= 1 && c <= W - 2) candmask |= 1u << k;
+        const int pc = r101(c, W);
+#pragma unroll
+        for (int j = 0; j < KT; j++) cx[k][j] = BORDER ? r101(pc + j - R, W) : 0;
+    }
+    if (!MAP && lane == 0) *scount = 0;
+    __syncwarp();
+    float m3a[4], m3b[4], eprev[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) { m3a[k] = m3b[k] = -FLT_MAX; eprev[k] = 0.f; }
+    unsigned mprev = 0;
+    float lmax = -FLT_MAX;
+    bool have_max = false, finite = true;
+    float thr_lb = 0.f;
+    if (!MAP) {
+        const uint32_t mb = *reinterpret_cast<volatile const uint32_t *>(&a.cnt->maxbits);
+        if (mb) thr_lb = fmaxf(0.f, (float)((double)dec_f32(mb) * a.quality));
+    }
+    auto flush = [&]() {
+        __syncwarp();
+        const int ncb = min(*reinterpret_cast<volatile int *>(scount), EN_CB);
+        unsigned base = 0;
+        if (lane == 0 && ncb) base = atomicAdd(&a.cnt->ncand, (unsigned)ncb);
+        base = __shfl_sync(0xffffffffu, base, 0);
+        for (int i = lane; i < ncb; i += 32)
+            if (base + i < a.cap) a.keys[base + i] = cbuf[i];
+        __syncwarp();
+        if (lane == 0) *scount = 0;
+        __syncwarp();
+    };
+    auto row_taps = [&](const float *row, float *hd, float *hs) {
+        if (BORDER) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                float d = 0.f, s = 0.f;
+#pragma unroll
+                for (int j = 0; j < KT; j++) {
+                    if (ap_d(G, j) == 0 && ap_s(G, j) == 0) continue;
+                    const float v = __ldg(row + cx[k][j]);
+                    if (ap_d(G, j) != 0) d = __fadd_rn(d, __fmul_rn((float)ap_d(G, j), v));
+                    if (ap_s(G, j) != 0) s = __fadd_rn(s, __fmul_rn(ss[j], v));
+                }
+                hd[k] = d; hs[k] = s;
+            }
+        } else {
+            f32_taps_vec<G>(__ldg(reinterpret_cast<const float4 *>(row + c0)), ss, hd, hs);
+        }
+    };
+    // window sum over columns [x + a0, x + a0 + bs) of a double plane held as 4 values per lane, columns in order
+    auto hbox = [&](const double *v, double *out) {
+        __syncwarp();
+        reinterpret_cast<double2 *>(rowbuf + EN_PAD + 4 * lane)[0] = make_double2(v[0], v[1]);
+        reinterpret_cast<double2 *>(rowbuf + EN_PAD + 4 * lane)[1] = make_double2(v[2], v[3]);
+        __syncwarp();
+        const double *p = rowbuf + EN_PAD + 4 * lane + a0;
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            double s = 0.0;
+            for (int j = 0; j < bs; j++) s = __dadd_rn(s, p[k + j]);
+            out[k] = s;
+        }
+    };
+    const int p_first = ey0 + a0, p_last = ey1 + a0 + bs - 1;
+    int slot = 0;
+    float hd[KT][4], hs[KT][4];
+    bool have = false;
+    for (int p = p_first; p <= p_last; p++) {
+        if (have && p + R <= H - 1) {
+#pragma unroll
+            for (int i = 0; i + 1 < KT; i++)
+#pragma unroll
+                for (int k = 0; k < 4; k++) { hd[i][k] = hd[i + 1][k]; hs[i][k] = hs[i + 1][k]; }
+            row_taps(f.img + (int64_t)(p + R) * f.pitch_f, hd[KT - 1], hs[KT - 1]);
+        } else {
+            const int rp = r101(p, H);
+#pragma unroll
+            for (int i = 0; i < KT; i++) row_taps(f.img + (int64_t)r101(rp + i - R, H) * f.pitch_f, hd[i], hs[i]);
+        }
+        have = p - R >= 0 && p + R <= H - 1;
+        float dx[4], dy[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            float x = 0.f, y = 0.f;
+#pragma unroll
+            for (int i = 0; i < KT; i++) {
+                if (ap_s(G, i) != 0) x = __fadd_rn(x, __fmul_rn(ss[i], hd[i][k]));
+                if (ap_d(G, i) != 0) y = __fadd_rn(y, __fmul_rn((float)ap_d(G, i), hs[i][k]));
+            }
+            dx[k] = x; dy[k] = y;
+        }
+        float4 *rg = reinterpret_cast<float4 *>(ring + slot * 2 * EN_COLS) + 2 * lane;
+        rg[0] = make_float4(dx[0], dy[0], dx[1], dy[1]);
+        rg[1] = make_float4(dx[2], dy[2], dx[3], dy[3]);
+        slot = slot + 1 == bs ? 0 : slot + 1;             // now the oldest row of the window
+        const int y = p - a0 - bs + 1;
+        if (y < ey0) continue;
+        // ---- vertical window sums: the bs products of each column, top to bottom, in double ---------------------------
+        double vxx[4] = {0.0, 0.0, 0.0, 0.0}, vxy[4] = {0.0, 0.0, 0.0, 0.0}, vyy[4] = {0.0, 0.0, 0.0, 0.0};
+        int s = slot;
+        for (int i = 0; i < bs; i++) {
+            const float4 *q = reinterpret_cast<const float4 *>(ring + s * 2 * EN_COLS) + 2 * lane;
+            const float4 o0 = q[0], o1 = q[1];
+            const float ox[4] = {o0.x, o0.z, o1.x, o1.z}, oy[4] = {o0.y, o0.w, o1.y, o1.w};
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                vxx[k] = __dadd_rn(vxx[k], (double)__fmul_rn(ox[k], ox[k]));
+                vxy[k] = __dadd_rn(vxy[k], (double)__fmul_rn(ox[k], oy[k]));
+                vyy[k] = __dadd_rn(vyy[k], (double)__fmul_rn(oy[k], oy[k]));
+            }
+            s = s + 1 == bs ? 0 : s + 1;
+        }
+        double bxx[4], bxy[4], byy[4];
+        hbox(vxx, bxx); hbox(vxy, bxy); hbox(vyy, byy);
+        float e[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            if (HARRIS) {                                 // cv2.cornerHarris: (a*c - b*b) - k*((a + c)*(a + c)), float, unfused
+                const float fa = (float)bxx[k], fb = (float)bxy[k], fc = (float)byy[k];
+                const float tr = __fadd_rn(fa, fc);
+                e[k] = __fsub_rn(__fsub_rn(__fmul_rn(fa, fc), __fmul_rn(fb, fb)), __fmul_rn(a.harris_k, __fmul_rn(tr, tr)));
+            } else {
+                const float fa = __fmul_rn((float)bxx[k], 0.5f), fb = (float)bxy[k], fc = __fmul_rn((float)byy[k], 0.5f);
+                const float d = __fsub_rn(fa, fc);
+                e[k] = __fsub_rn(__fadd_rn(fa, fc), __fsqrt_rn(__fadd_rn(__fmul_rn(d, d), __fmul_rn(fb, fb))));
+            }
+        }
+        if (MAP) {
+            if (y >= Y0 && y < Y1) {
+#pragma unroll
+                for (int k = 0; k < 4; k++)
+                    if ((outmask >> k) & 1u) f.map[(int64_t)y * f.map_pitch_f + c0 + k] = e[k];
+            }
+            continue;
+        }
+        // ---- masked maximum, 3x3 raw maxima of the previous row, candidate buffer: as eig_nms_job ----------------------------
+        unsigned mcur = 0xfu;
+        if (MASK) {
+            mcur = 0;
+#pragma unroll
+            for (int k = 0; k < 4; k++)
+                if ((outmask >> k) & 1u) mcur |= (a.mask[(int64_t)y * a.mask_pitch + c0 + k] ? 1u : 0u) << k;
+        }
+        if (y >= Y0 && y < Y1) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                if ((outmask >> k) & 1u) finite = finite && isfinite(e[k]);
+                if (((outmask & mcur) >> k) & 1u) { lmax = fmaxf(lmax, e[k]); have_max = true; }
+            }
+        }
+        const float el = __shfl_up_sync(0xffffffffu, e[3], 1), er = __shfl_down_sync(0xffffffffu, e[0], 1);
+        float m3c[4];
+        m3c[0] = fmaxf(fmaxf(el, e[0]), e[1]); m3c[1] = fmaxf(fmaxf(e[0], e[1]), e[2]);
+        m3c[2] = fmaxf(fmaxf(e[1], e[2]), e[3]); m3c[3] = fmaxf(fmaxf(e[2], e[3]), er);
+        const int yc = y - 1;
+        if (yc >= max(Y0, 1) && yc < Y1 && yc <= H - 2) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                const float v = eprev[k];
+                if ((((candmask & mprev) >> k) & 1u) && v > thr_lb && v == fmaxf(fmaxf(m3a[k], m3b[k]), m3c[k])) {
+                    const unsigned long long key = ((unsigned long long)enc_f32(v) << 32) | (uint32_t)(yc * W + c0 + k);
+                    const int pos = atomicAdd(scount, 1);
+                    if (pos < EN_CB) cbuf[pos] = key;
+                    else {
+                        const unsigned g = atomicAdd(&a.cnt->ncand, 1u);
+                        if (g < a.cap) a.keys[g] = key;
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) { m3a[k] = m3b[k]; m3b[k] = m3c[k]; eprev[k] = e[k]; }
+        mprev = mcur;
+        if ((y & 7) == 7) {
+            __syncwarp();
+            if (*reinterpret_cast<volatile int *>(scount) >= EN_CB / 2) flush();
+            if ((y & 31) == 31) {
+                float wm = lmax;
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) wm = fmaxf(wm, __shfl_xor_sync(0xffffffffu, wm, o));
+                if (wm > 0.f) thr_lb = fmaxf(thr_lb, (float)((double)wm * a.quality));
+            }
+        }
+    }
+    if (MAP) return;
+    flush();
+    uint32_t lbits = have_max ? enc_f32(lmax) : 0u;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lbits = max(lbits, __shfl_xor_sync(0xffffffffu, lbits, o));
+    if (lane == 0 && lbits) atomicMax(&a.cnt->maxbits, lbits);
+    if (!__all_sync(0xffffffffu, finite) && lane == 0) atomicCAS(&a.cnt->error, 0, IBT_E_UNSUPPORTED);
+}
+
+template <int G, bool MASK, bool HARRIS, bool MAP>
+__global__ void __launch_bounds__(EN_WARPS * 32, EN_AP_MIN_CTAS)
+eig_f32_kernel(const __grid_constant__ EigF32Args f)
+{
+    extern __shared__ __align__(16) int en_smem[];
+    if (!MAP) pdl_launch_dependents();
+    const EigNmsArgs &a = f.n;
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int job = blockIdx.x * EN_WARPS + wib;
+    if (job >= a.njobs) return;
+    int *wsm = en_smem + (size_t)wib * a.warp_smem_ints;
+    const int nbj = a.nborder * a.chunks_border;                  // job split of eig_nms_kernel
+    if (job < nbj) {
+        const int sb = job % a.nborder, chunk = job / a.nborder;
+        const int strip = a.nborder == a.nstrips ? sb : (sb == 0 ? 0 : a.first_right + sb - 1);
+        const int Y0 = chunk * a.rows_border;
+        eig_f32_job<G, MASK, true, HARRIS, MAP>(f, strip, Y0, min(a.H, Y0 + a.rows_border), wsm, lane);
+    } else {
+        const int j = job - nbj, nfast = a.nstrips - a.nborder;
+        const int strip = 1 + j % nfast, chunk = j / nfast;
+        const int Y0 = chunk * a.rows_fast;
+        eig_f32_job<G, MASK, false, HARRIS, MAP>(f, strip, Y0, min(a.H, Y0 + a.rows_fast), wsm, lane);
+    }
+}
+
+template <int G, bool MASK, bool HARRIS, bool MAP>
+static int launch_eig_f32_kernel(const EigF32Args &f, cudaStream_t st)
+{
+    const size_t smem = (size_t)f.n.warp_smem_ints * 4 * EN_WARPS;
+    const int blocks = (f.n.njobs + EN_WARPS - 1) / EN_WARPS;
+    if (smem > 48 * 1024) IBT_CUDA_TRY(cudaFuncSetAttribute(eig_f32_kernel<G, MASK, HARRIS, MAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    eig_f32_kernel<G, MASK, HARRIS, MAP><<<blocks, EN_WARPS * 32, smem, st>>>(f);
+    return check_launch("eig_f32_kernel");
+}
+
+template <int G>
+static int launch_eig_f32_g(const EigF32Args &f, int harris, int map, cudaStream_t st)
+{
+    if (map) return harris ? launch_eig_f32_kernel<G, false, true, true>(f, st) : launch_eig_f32_kernel<G, false, false, true>(f, st);
+    if (f.n.mask) return harris ? launch_eig_f32_kernel<G, true, true, false>(f, st) : launch_eig_f32_kernel<G, true, false, false>(f, st);
+    return harris ? launch_eig_f32_kernel<G, false, true, false>(f, st) : launch_eig_f32_kernel<G, false, false, false>(f, st);
+}
+
+static bool f32_image_ok(const float *img, int H, int W, int64_t pitch_bytes)
+{
+    return img && H > 0 && W > 0 && reinterpret_cast<uintptr_t>(img) % 4 == 0 && pitch_bytes % 4 == 0 &&
+           pitch_bytes >= (int64_t)W * 4;
+}
+
+// map hooks (map != nullptr: mask / counters unused) and the fused K2a of goodFeaturesToTrack on a float32 image
+static int launch_eig_f32(const float *img, int H, int W, int64_t pitch_bytes, int bs, int ksize, int harris, double harris_k,
+                          float *map, int64_t map_pitch_bytes, const uint8_t *mask, int64_t mask_pitch, double quality,
+                          GfttCounters *cnt, unsigned long long *keys, uint32_t cap, cudaStream_t st)
+{
+    if (bs < 1 || bs > MAX_BLOCK || !ap_supported(ksize) || !f32_image_ok(img, H, W, pitch_bytes) || !(harris_k == harris_k))
+        return IBT_E_INVALID;
+    if (map && (map_pitch_bytes % 4 != 0 || map_pitch_bytes < (int64_t)W * 4)) return IBT_E_INVALID;
+    EigF32Args f;
+    memset(&f, 0, sizeof(f));
+    EigNmsArgs &a = f.n;
+    a.H = H; a.W = W; a.mask = mask; a.mask_pitch = mask_pitch; a.bs = bs;
+    a.quality = quality; a.cnt = cnt; a.keys = keys; a.cap = cap;
+    a.harris_k = (float)harris_k;
+    f.img = img; f.pitch_f = pitch_bytes / 4;
+    f.map = map; f.map_pitch_f = map_pitch_bytes / 4;
+    const double sden = ksize == -1 ? 8.0 : (double)(1 << ((ksize > 0 ? ksize : 3) - 1));
+    const double scale = 1.0 / (sden * bs);                       // cv2's CV_32F scale: no factor 255
+    for (int j = 0; j < ap_taps(ksize); j++) f.ss[j] = (float)(ap_s(ksize, j) * scale);
+    // strip geometry of launch_eig_nms; 16-byte loads on the inner strips
+    const int half = bs / 2;
+    const int srad = ap_taps(ksize) / 2;
+    a.left = (srad + 1 + half + 3) & ~3;
+    a.outw = (128 - srad - 1 - a.left - (bs - 1 - half)) & ~3;
+    a.nstrips = (W + a.outw - 1) / a.outw;
+    a.word_ok = (reinterpret_cast<uintptr_t>(img) % 16 == 0) && (pitch_bytes % 16 == 0);
+    int first_right = a.nstrips;
+    while (first_right > 1 && (first_right - 1) * a.outw - a.left + EN_COLS > W) first_right--;
+    if (!a.word_ok || first_right <= 1) { a.nborder = a.nstrips; first_right = a.nstrips; }
+    else a.nborder = 1 + (a.nstrips - first_right);
+    a.first_right = first_right;
+    a.warp_smem_ints = bs * 2 * EN_COLS + EN_CB * 2 + 4 + 2 * (EN_PAD + EN_COLS + EN_PAD);
+    int wps = (int)((227 * 1024) / ((size_t)a.warp_smem_ints * 4 * EN_WARPS + 1024)) * EN_WARPS;
+    if (wps < 1) wps = 1;
+    if (wps > EN_AP_MIN_CTAS * EN_WARPS) wps = EN_AP_MIN_CTAS * EN_WARPS;
+    const int nfast = a.nstrips - a.nborder;
+    const int weight = nfast + EN_BORDER_SPLIT * a.nborder;
+    int chunks = (kNumSMs * wps) / weight;
+    if (chunks < 1) chunks = 1;
+    int rows = (H + chunks - 1) / chunks;
+    if (rows < 32) rows = 32;
+    a.rows_fast = rows;
+    a.rows_border = (rows + EN_BORDER_SPLIT - 1) / EN_BORDER_SPLIT;
+    if (a.rows_border < 8) a.rows_border = 8;
+    a.chunks_border = (H + a.rows_border - 1) / a.rows_border;
+    a.njobs = a.nborder * a.chunks_border + nfast * ((H + rows - 1) / rows);
+    const int m = map ? 1 : 0;
+    switch (ksize) {
+    case -1: return launch_eig_f32_g<-1>(f, harris, m, st);
+    case 1: return launch_eig_f32_g<1>(f, harris, m, st);
+    case 3: return launch_eig_f32_g<3>(f, harris, m, st);
+    case 5: return launch_eig_f32_g<5>(f, harris, m, st);
+    default: return launch_eig_f32_g<7>(f, harris, m, st);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // K2b: the whole selection in ONE persistent launch.  sorted[r] = ~key of rank r (rank 0 = strongest).
 constexpr int SEL_THREADS = 256;
 constexpr int SEL_CTAS_PER_SM = 2;                   // 2 x 256 threads x 128 registers fill an SM: the grid is kNumSMs * 2, all resident
@@ -1421,13 +1788,16 @@ static GfttLayout gftt_layout(int H, int W)
 }
 
 // Both launches of goodFeaturesToTrack on `st`; nothing is read back.  count_dev (device int) receives the corner count.
-static int gftt_enqueue(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
+// f32src: `gray` is a float32 image and `pitch` its byte pitch (eig_f32_kernel produces the candidates).
+static int gftt_enqueue(const void *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
                         int maxCorners, double qualityLevel, double minDistance, int blockSize, int ksize, int useHarris, double harris_k,
-                        void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *count_dev, cudaStream_t st)
+                        void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *count_dev, cudaStream_t st,
+                        bool f32src = false)
 {
     if (!gray || !workspace || H < 3 || W < 3 || H > 65535 || W > 65535 || (int64_t)H * W > 0x7fffffffLL ||
         cap < 0 || (cap > 0 && !out_xy) || (mask && mask_pitch < W) || qualityLevel < 0 || minDistance < 0 || minDistance > 1024 ||
-        pitch < W || !(harris_k == harris_k) || !ap_supported(ksize))
+        pitch < W || !(harris_k == harris_k) || !ap_supported(ksize) || blockSize < 1 || blockSize > MAX_BLOCK ||
+        (f32src && !f32_image_ok(static_cast<const float *>(gray), H, W, pitch)))
         return IBT_E_INVALID;
     const GfttLayout L = gftt_layout(H, W);
     if (workspace_bytes < L.total) return IBT_E_WORKSPACE;
@@ -1435,7 +1805,10 @@ static int gftt_enqueue(const uint8_t *gray, int64_t pitch, const uint8_t *mask,
     GfttCounters *cnt = reinterpret_cast<GfttCounters *>(ws + L.off_cnt);
     IBT_CUDA_TRY(cudaMemsetAsync(cnt, 0, sizeof(GfttCounters), st));
     unsigned long long *keys0 = reinterpret_cast<unsigned long long *>(ws + L.off_keys0);
-    int rc = launch_eig_nms(gray, H, W, pitch, blockSize, ksize, useHarris, harris_k, mask, mask_pitch, qualityLevel, cnt, keys0, L.cap, st);
+    int rc = f32src ? launch_eig_f32(static_cast<const float *>(gray), H, W, pitch, blockSize, ksize, useHarris, harris_k, nullptr, 0,
+                                     mask, mask_pitch, qualityLevel, cnt, keys0, L.cap, st)
+                    : launch_eig_nms(static_cast<const uint8_t *>(gray), H, W, pitch, blockSize, ksize, useHarris, harris_k, mask,
+                                     mask_pitch, qualityLevel, cnt, keys0, L.cap, st);
     if (rc) return rc;
     SelArgs a;
     a.cnt = cnt; a.keys0 = keys0;
@@ -1533,19 +1906,19 @@ IBT_API int ibt_gftt_async(const uint8_t *gray, int64_t pitch, const uint8_t *ma
                                 useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, count_dev, stream);
 }
 
-IBT_API int ibt_gftt_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
-                           int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
-                           int useHarrisDetector, double k, void *workspace, size_t workspace_bytes, float *out_xy, int cap,
-                           int *out_count, void *stream)
+// the synchronous form: both launches, then the one host round trip -- the corner count decides the shapes the caller
+// allocates next
+static int gftt_sync(const void *img, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W, int maxCorners,
+                     double qualityLevel, double minDistance, int blockSize, int gradientSize, int useHarrisDetector, double k,
+                     void *workspace, size_t workspace_bytes, float *out_xy, int cap, int *out_count, void *stream, bool f32src)
 {
     using namespace ibt;
     if (!out_count) return IBT_E_INVALID;
     *out_count = 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int rc = gftt_enqueue(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, gradientSize,
-                          useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, nullptr, st);
+    int rc = gftt_enqueue(img, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, gradientSize,
+                          useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, nullptr, st, f32src);
     if (rc) return rc;
-    // the one host round trip of the synchronous form: the corner count decides the shapes the caller allocates next
     struct Head { uint32_t maxbits, ncand, nsel, nacc, nout; int32_t error; };
     static thread_local Head *hc = nullptr;                        // page-locked: the copy is a real asynchronous DMA
     if (!hc) IBT_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void **>(&hc), sizeof(Head), cudaHostAllocDefault));
@@ -1553,6 +1926,40 @@ IBT_API int ibt_gftt_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *ma
     IBT_CUDA_TRY(cudaStreamSynchronize(st));
     *out_count = (int)hc->nout;
     return hc->error ? hc->error : IBT_OK;
+}
+
+IBT_API int ibt_gftt_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
+                           int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                           int useHarrisDetector, double k, void *workspace, size_t workspace_bytes, float *out_xy, int cap,
+                           int *out_count, void *stream)
+{
+    return gftt_sync(gray, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, gradientSize,
+                     useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, out_count, stream, false);
+}
+
+IBT_API int ibt_gftt_f32src(const float *img, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,
+                            int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                            int useHarrisDetector, double k, void *workspace, size_t workspace_bytes, float *out_xy, int cap,
+                            int *out_count, void *stream)
+{
+    return gftt_sync(img, pitch, mask, mask_pitch, H, W, maxCorners, qualityLevel, minDistance, blockSize, gradientSize,
+                     useHarrisDetector, k, workspace, workspace_bytes, out_xy, cap, out_count, stream, true);
+}
+
+IBT_API int ibt_min_eigen_f32src(const float *img, int H, int W, int64_t pitch, int blockSize, int ksize, float *eig,
+                                 int64_t eig_pitch, void *stream)
+{
+    if (!eig) return IBT_E_INVALID;
+    return ibt::launch_eig_f32(img, H, W, pitch, blockSize, ksize, 0, 0.0, eig, eig_pitch, nullptr, 0, 0.0, nullptr, nullptr, 0,
+                               static_cast<cudaStream_t>(stream));
+}
+
+IBT_API int ibt_corner_harris_f32src(const float *img, int H, int W, int64_t pitch, int blockSize, int ksize, double k,
+                                     float *dst, int64_t dst_pitch, void *stream)
+{
+    if (!dst) return IBT_E_INVALID;
+    return ibt::launch_eig_f32(img, H, W, pitch, blockSize, ksize, 1, k, dst, dst_pitch, nullptr, 0, 0.0, nullptr, nullptr, 0,
+                               static_cast<cudaStream_t>(stream));
 }
 
 IBT_API int ibt_gftt(const uint8_t *gray, int64_t pitch, const uint8_t *mask, int64_t mask_pitch, int H, int W,

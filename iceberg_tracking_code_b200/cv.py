@@ -474,16 +474,32 @@ def _aperture(ksize, what, name):
     return int(ksize)
 
 
+def _corner_src(src, what):
+    """the image of the corner family -> (CUDA tensor, is_float): u8 or float32 (cv2: CV_8UC1 || CV_32FC1); any other dtype
+    raises like cv2's assertion in corner.cpp"""
+    dt = src.dtype if isinstance(src, (np.ndarray, torch.Tensor)) else None
+    if dt in (np.float32, torch.float32):
+        return _to_dev(src, np.float32, what), True
+    if dt is None or dt in (np.uint8, torch.uint8):
+        return _to_dev(src, np.uint8, what), False
+    raise error("%s: src.type() == CV_8UC1 || src.type() == CV_32FC1 (got %s)" % (what, dt))
+
+
 def cornerMinEigenVal(src, blockSize, dst=None, ksize=3):
-    """cv2.cornerMinEigenVal(src, blockSize[, dst[, ksize]]): u8 (H,W) -> (H,W) f32 (SURVEY A.6 steps 1-3); dst is cv2's output
-    placeholder (the map is returned).  ksize: Sobel aperture -1 (Scharr), 1, 3, 5 or 7."""
+    """cv2.cornerMinEigenVal(src, blockSize[, dst[, ksize]]): u8 or float32 (H,W) -> (H,W) f32 (SURVEY A.6 steps 1-3); dst is
+    cv2's output placeholder (the map is returned).  ksize: Sobel aperture -1 (Scharr), 1, 3, 5 or 7.  A float32 image takes
+    cv2's CV_32F scale (no factor 255); NaN / inf pixels give NaN / inf responses, as in cv2."""
     ksize = _aperture(ksize, "cornerMinEigenVal", "ksize")
     as_np = _is_np(src)
-    s = _to_dev(src, np.uint8, "cornerMinEigenVal src")
+    s, f32 = _corner_src(src, "cornerMinEigenVal src")
     if s.ndim != 2:
-        raise error("cornerMinEigenVal: expected a single-channel (H,W) u8 image")
+        raise error("cornerMinEigenVal: expected a single-channel (H,W) u8 or float32 image")
     H, W = s.shape
     eig = torch.empty((H, W), dtype=torch.float32, device=s.device)
+    if f32:
+        N.check(N.lib().ibt_min_eigen_f32src(_ptr(s), H, W, W * 4, int(blockSize), ksize, _ptr(eig), W * 4, _stream()),
+                "ibt_min_eigen_f32src")
+        return _out(eig, as_np)
     N.check(N.lib().ibt_min_eigen_ksize_f32(_ptr(s), H, W, W, int(blockSize), ksize, _ptr(eig), W * 4, _stream()),
             "ibt_min_eigen_ksize_f32")
     return _out(eig, as_np)
@@ -492,14 +508,18 @@ def cornerMinEigenVal(src, blockSize, dst=None, ksize=3):
 def cornerHarris(src, blockSize, ksize=3, k=0.04):
     """cv2.cornerHarris(u8 (H,W), blockSize, ksize, k) -> (H,W) f32: the response goodFeaturesToTrack(useHarrisDetector=True)
     ranks.  The reference leaves useHarrisDetector at False (s1:240-243); cv2's signature carries it (SURVEY 8b).
-    ksize: Sobel aperture -1 (Scharr), 1, 3, 5 or 7."""
+    ksize: Sobel aperture -1 (Scharr), 1, 3, 5 or 7.  src may also be float32 (cv2's CV_32F scale, as cornerMinEigenVal)."""
     ksize = _aperture(ksize, "cornerHarris", "ksize")
     as_np = _is_np(src)
-    s = _to_dev(src, np.uint8, "cornerHarris src")
+    s, f32 = _corner_src(src, "cornerHarris src")
     if s.ndim != 2:
-        raise error("cornerHarris: expected a single-channel (H,W) u8 image")
+        raise error("cornerHarris: expected a single-channel (H,W) u8 or float32 image")
     H, W = s.shape
     dst = torch.empty((H, W), dtype=torch.float32, device=s.device)
+    if f32:
+        N.check(N.lib().ibt_corner_harris_f32src(_ptr(s), H, W, W * 4, int(blockSize), ksize, float(k), _ptr(dst), W * 4,
+                                                 _stream()), "ibt_corner_harris_f32src")
+        return _out(dst, as_np)
     N.check(N.lib().ibt_corner_harris_ksize_f32(_ptr(s), H, W, W, int(blockSize), ksize, float(k), _ptr(dst), W * 4,
                                                 _stream()), "ibt_corner_harris_ksize_f32")
     return _out(dst, as_np)
@@ -531,14 +551,16 @@ def goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, corners=No
     first overload's and the reference's), 5 or 7).
     Returns (K,1,2) float32 integer-valued (x, y) ordered by response, or None when there is no corner
     (callers test `if p is not None`, s1:445).  useHarrisDetector=True ranks cv2.cornerHarris(image, blockSize, gradientSize, k)
-    instead of the minimal eigenvalue (the reference never sets it)."""
+    instead of the minimal eigenvalue (the reference never sets it).
+    image may also be float32 (cv2's CV_32F scale): an image whose response is not finite everywhere (a NaN / inf pixel, or
+    derivative products beyond float range) raises cv.error rather than return corners derived from it."""
     if not (qualityLevel > 0) or minDistance < 0:
         raise error("goodFeaturesToTrack: qualityLevel must be > 0 and minDistance >= 0")
     gradientSize = _aperture(gradientSize, "goodFeaturesToTrack", "gradientSize")
     as_np = _is_np(image)
-    img = _to_dev(image, np.uint8, "goodFeaturesToTrack image")
+    img, f32 = _corner_src(image, "goodFeaturesToTrack image")
     if img.ndim != 2:
-        raise error("goodFeaturesToTrack: expected a single-channel (H,W) u8 image")
+        raise error("goodFeaturesToTrack: expected a single-channel (H,W) u8 or float32 image")
     H, W = img.shape
     m = None
     if mask is not None:
@@ -549,6 +571,17 @@ def goodFeaturesToTrack(image, maxCorners, qualityLevel, minDistance, corners=No
         return None
     ws, out = _gftt_workspace(img.device, H, W)
     cnt = C.c_int(0)
+    if f32:
+        rc = N.lib().ibt_gftt_f32src(_ptr(img), W * 4, _ptr(m), W, H, W, int(maxCorners), float(qualityLevel),
+                                     float(minDistance), int(blockSize), gradientSize, 1 if useHarrisDetector else 0, float(k),
+                                     _ptr(ws), ws.numel(), _ptr(out), out.shape[0], C.byref(cnt), _stream())
+        if rc == N.IBT_E_UNSUPPORTED:
+            raise error("goodFeaturesToTrack: the float32 image gives a non-finite corner response (NaN / inf pixels, or "
+                        "derivative products beyond float range)")
+        N.check(rc, "ibt_gftt_f32src")
+        if cnt.value == 0:
+            return None
+        return _out(out[:cnt.value].reshape(-1, 1, 2).clone(), as_np)
     rc = N.lib().ibt_gftt_ksize(_ptr(img), W, _ptr(m), W, H, W, int(maxCorners), float(qualityLevel), float(minDistance),
                                 int(blockSize), gradientSize, 1 if useHarrisDetector else 0, float(k), _ptr(ws), ws.numel(),
                                 _ptr(out), out.shape[0], C.byref(cnt), _stream())

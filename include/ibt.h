@@ -214,6 +214,24 @@ int ibt_gftt_async_ksize(const uint8_t *gray, int64_t pitch, const uint8_t *mask
                          int useHarrisDetector, double k,
                          void *workspace, size_t workspace_bytes,
                          float *out_xy, int cap, int *count_dev, void *stream);
+/* The same three on a float32 image (cv2 takes CV_8UC1 and CV_32FC1): arguments of ibt_gftt_ksize /
+ * ibt_min_eigen_ksize_f32 / ibt_corner_harris_ksize_f32, except that img is float and pitch is in BYTES.  img must be 4-byte
+ * aligned and pitch a multiple of 4 (>= 4 * W); anything else, like any other invalid argument, returns IBT_E_INVALID before
+ * any CUDA call (16-byte alignment of both takes the vector-load path; any 4-byte layout gives the same bytes).  OpenCV's
+ * CV_32F front end: Sobel / Scharr in float with scale 1 / (sden * blockSize) (no 255), float products, double window sums,
+ * the float response.  The window sums are added per pixel in a fixed order, not as OpenCV's running sums: the maps agree
+ * with cv2's to rounding.  The workspace is sized by ibt_gftt_workspace_bytes.  Non-finite values: the map hooks write the
+ * NaN / inf they produce; ibt_gftt_f32src returns IBT_E_UNSUPPORTED when any response is not finite (a NaN / inf pixel, or
+ * derivative products beyond float range) instead of corners derived from it. */
+int ibt_gftt_f32src(const float *img, int64_t pitch, const uint8_t *mask, int64_t mask_pitch,
+                    int H, int W, int maxCorners, double qualityLevel, double minDistance, int blockSize, int gradientSize,
+                    int useHarrisDetector, double k,
+                    void *workspace, size_t workspace_bytes,
+                    float *out_xy, int cap, int *out_count, void *stream);
+int ibt_min_eigen_f32src(const float *img, int H, int W, int64_t pitch, int blockSize, int ksize,
+                         float *eig, int64_t eig_pitch, void *stream);
+int ibt_corner_harris_f32src(const float *img, int H, int W, int64_t pitch, int blockSize, int ksize, double k,
+                             float *dst, int64_t dst_pitch, void *stream);
 
 /* ---- track bookkeeping at a group boundary (s1:362-395): stable compaction of the live
  * tracks.  tracks_tm (T+1, N, 2) f32 time-major, quality_tm (T, N) f32, alive (N) u8 ->

@@ -3,7 +3,8 @@
     python tools/prof_gftt.py [maxCorners] [--ksize G ...]
 
 With --ksize, times the call for each Sobel aperture G (cv2's gradientSize: -1 = Scharr, 1, 3, 5, 7) with CUDA events after
-warm-up and prints the card name and power limit beside the times."""
+warm-up and prints the card name and power limit beside the times: on the u8 frame, then on the same frame as float32
+(I / 255, the float path's front end)."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -28,18 +29,20 @@ if ksizes:
         print("card:", card.strip().splitlines()[torch.cuda.current_device()])
     except Exception as e:                                  # noqa: BLE001
         print("card:", torch.cuda.get_device_name(), "(power limit unreadable: %s)" % e)
-    for ks in ksizes:
-        gp = dict(maxCorners=maxc, qualityLevel=0.007, minDistance=10, blockSize=10, gradientSize=ks)
-        for _ in range(3):
-            cv.goodFeaturesToTrack(g, **gp)
-        reps, ts = 20, []
-        for _ in range(reps):
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record(); p = cv.goodFeaturesToTrack(g, **gp); e1.record(); e1.synchronize()
-            ts.append(e0.elapsed_time(e1))
-        ts.sort()
-        print("gradientSize %2d: median %.3f ms  min %.3f ms  (%d calls)  corners %s" % (ks, ts[reps // 2], ts[0], reps,
-                                                                                       None if p is None else p.shape[0]))
+    gf = g.float() / 255.0
+    for img, kind in ((g, "u8"), (gf, "float32")):
+        for ks in ksizes:
+            gp = dict(maxCorners=maxc, qualityLevel=0.007, minDistance=10, blockSize=10, gradientSize=ks)
+            for _ in range(3):
+                cv.goodFeaturesToTrack(img, **gp)
+            reps, ts = 20, []
+            for _ in range(reps):
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record(); p = cv.goodFeaturesToTrack(img, **gp); e1.record(); e1.synchronize()
+                ts.append(e0.elapsed_time(e1))
+            ts.sort()
+            print("%-7s gradientSize %2d: median %.3f ms  min %.3f ms  (%d calls)  corners %s" % (
+                kind, ks, ts[reps // 2], ts[0], reps, None if p is None else p.shape[0]))
     sys.exit(0)
 
 for it in range(3):
